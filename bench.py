@@ -6,6 +6,7 @@ scene at 1280x720, 64 spp, bokeh DoF + HDRi importance sampling, on 1/2/4/8 B200
   python bench.py --impl reference ...                     (the reference's algorithm on the host CPU)
   python bench.py --config {1..5}                          (the other BASELINE.json configs; default 2 = the metric's)
   python bench.py --gpus N --scaling strong                (ONE fixed frame split over N GPUs by tiles x sample sets)
+  python bench.py ... --dump-outputs DIR                   (the last timed step's accumulation buffer -> DIR/accum.npy)
 
 A "step" = one frame of the workload (config 2: 64 spp of 1280x720 = 58.98 M path samples).
   value : device-resident throughput -- scene already in HBM, CUDA events on the library's launch stream around
@@ -311,6 +312,23 @@ def verify_parity(rank, world, local_rank, comm_ok):
     return ok, "96x64, 8 samples, %d tile(s) x %d sample set(s), accumulation sum bit-exact vs CPU oracle" % (n_tiles, n_sets)
 
 
+DUMP_LIMIT = 64 * 10 ** 6  # bytes written by --dump-outputs, .npy headers included
+
+
+def dump_outputs(out_dir, accum):
+    """--dump-outputs: the (H, W, 4) float32 accumulation buffer the timed render left, as a caller of fspt_read_accum
+    receives it, so that two builds can be compared output for output.  A buffer above 64 MB (config 5) is replaced by
+    a fixed, seeded sample of its pixels, accum.npy (n, 4), with their row-major pixel indices in accum_pixel_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    px = accum.reshape(-1, 4)
+    if accum.nbytes > DUMP_LIMIT:
+        n = (DUMP_LIMIT - 1024) // (px.itemsize * 4 + 8)
+        idx = np.sort(np.random.default_rng(0).choice(px.shape[0], n, replace=False))
+        np.save(os.path.join(out_dir, "accum_pixel_index.npy"), idx.astype(np.float64))
+        accum = px[idx]
+    np.save(os.path.join(out_dir, "accum.npy"), np.ascontiguousarray(accum, np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -328,6 +346,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-verify", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the accumulation buffer of the last one to DIR/accum.npy (float32)")
     args = ap.parse_args()
     cfg = CONFIGS[args.config]
     args.width = args.width or cfg["res"][0]
@@ -450,6 +470,8 @@ def main():
     else:
         dev_ms_max, rays_total = dev_ms, float(rays)
     value = samples_per_step * args.steps / (dev_ms_max * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx.read_accum())  # before the e2e steps below render into the same buffer
 
     # ---- end-to-end through the host API with host buffers ---------------------------------------------------
     e2e = None

@@ -6,10 +6,16 @@ Bars (BASELINE.md section 4 / north star):
     implement the same FSPT-DM2 arithmetic as the oracle, so these are asserted bit-exact as well
     (stated tolerance: 0 ulp; a mismatch-rate report is printed if that ever fails).
 """
+import os
+import sys
+
 import numpy as np
 import pytest
 
 from fspt_b200 import capi, scenes
+
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+import make_reference_outputs as golden  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -226,40 +232,33 @@ def test_node_records_through_the_lsu_path_bit_exact(oracle_mod, monkeypatch, sm
     _full_frame_check(oracle_mod, sa, cam, 160, 96, 2, 19)
 
 
+REF_W, REF_H, REF_N = 128, 72, 4
+REF_POST = dict(exposure=1.2, saturation=0.9, denoise=True, max_sigma=2.0)
+
+
 def test_cuda_against_the_reference_shaders_themselves(small_bunny):
-    """No restatement in between: the CUDA path against /root/reference/shader/*.fs compiled for the CPU
-    (oracle/_ref/libfspt_ref.so, built where the reference tree exists; the built file travels to this box).
-    Camera rays, primary hits (index, t, count), the running-mean accumulator over 4 ticks and the RGBA8 post-pass."""
-    from oracle import reference_shaders as R
-    if not R.available():
-        pytest.skip("oracle/_ref/libfspt_ref.so did not travel and there is no reference tree to build it from")
+    """No restatement in between: the CUDA path against what the reference's own camera.fs, bvh_test.fs, tracer.fs and
+    draw.fs, compiled for the CPU, computed on the same inputs (tests/golden/reference_shaders/outputs.npz, generator
+    tests/golden/make_reference_outputs.py).  Camera rays, primary hits (index, t, count), the running-mean accumulator
+    over 4 ticks and the RGBA8 post-pass."""
     sa, cam = small_bunny
-    W, H, N = 128, 72, 4
-    Rf = R.Reference(sa)
-    lens = np.asarray(scenes.lens_features(cam), np.float32)
+    W, H, N = REF_W, REF_H, REF_N
     rc, rt = scenes.rand_bases(N, 29)
     ctx = capi.Context(W, H)
     try:
         ctx.scene_upload(sa)
         fr = _frame(ctx, cam)
         idx, t, cnt, pos, d = ctx.debug_primary(fr, float(rc[0]))
-        rpos, rdir = R.camera(W, H, cam["eye"], cam["dir"], cam["fov_scale"], lens, rc[0])
-        assert_bit_equal(pos, rpos, "camera.fs position")
-        assert_bit_equal(d, rdir, "camera.fs direction")
-        ri, rt_, rcnt = Rf.bvh_test(rpos, rdir)
-        assert_bit_equal(idx, ri, "bvh_test.fs index")
-        assert_bit_equal(t, rt_, "bvh_test.fs t")
-        assert_bit_equal(cnt, rcnt, "bvh_test.fs count")
+        golden.check("cuda/camera/pos", pos)
+        golden.check("cuda/camera/dir", d)
+        golden.check("cuda/bvh_test/index", idx)
+        golden.check("cuda/bvh_test/t", t)
+        golden.check("cuda/bvh_test/count", cnt)
         ctx.clear()
         ctx.set_param(capi.PARAM_SANITIZE_NAN, 0)  # the reference lets NaN stick (tracer.fs:515-517)
         ctx.render(fr, 0, rc, rt)
-        fb = None
-        for k in range(N):
-            p4, d4 = R.camera(W, H, cam["eye"], cam["dir"], cam["fov_scale"], lens, rc[k])
-            fb = Rf.trace(p4, d4, W, H, k, rt[k], cam["env_theta"], fb_prev=fb)
-        assert_bit_equal(ctx.read_accum()[..., :3], fb[..., :3], "tracer.fs accumulation")
-        post = dict(exposure=1.2, saturation=0.9, denoise=True, max_sigma=2.0)
-        assert_bit_equal(ctx.resolve(**post), R.draw(fb, **post), "draw.fs RGBA8")
+        golden.check("cuda/tracer/accum_rgb", ctx.read_accum()[..., :3])
+        golden.check("cuda/draw/rgba8", ctx.resolve(**REF_POST))
     finally:
         ctx.close()
 
