@@ -156,8 +156,11 @@ inline int scene_prepass(HostPool& pool, int hw, const fspt_scene_desc* s, Scene
     size_t visited = top_visited;
     for (int k = 0; k < n_sub; ++k) { max_depth = std::max(max_depth, sub_depth[k]); visited += sub_visited[k]; }
     if (visited > (size_t)N) return fail(FSPT_E_INVALID, "BVH is not a tree (cycle or shared node)", 0, 0);
-    if (max_depth + 1 > FSPT_STACK)
-      return fail(FSPT_E_LIMIT, "BVH depth %d exceeds the traversal stack (%d, as in tracer.fs:368)", max_depth, FSPT_STACK);
+    // max_depth counts the nodes on the longest root-to-leaf path.  The walk down it defers at most one child per interior
+    // node (max_depth - 1 entries) on top of the sentinel, so a tree of FSPT_STACK levels fills the stack exactly.
+    if (max_depth > FSPT_STACK)
+      return fail(FSPT_E_LIMIT, "BVH of %d levels exceeds the traversal stack (at most %d levels, tracer.fs:368)", max_depth,
+                  FSPT_STACK);
     P.max_depth = max_depth;
   }
   for (int ch = 0; ch < n_nchunks; ++ch) chunk_interiors[ch + 1] += chunk_interiors[ch];

@@ -33,7 +33,7 @@ class OScene(C.Structure):
 
 class OStats(C.Structure):
     _fields_ = [("rays", C.c_uint64), ("node_visits", C.c_uint64), ("leaf_visits", C.c_uint64),
-                ("stack_overflow", C.c_uint64)]
+                ("stack_overflow", C.c_uint64), ("capped", C.c_uint64)]
 
     def as_dict(self):
         return {k: int(getattr(self, k)) for k, _ in self._fields_}

@@ -53,6 +53,7 @@ struct OStats {
   uint64_t node_visits; /* loop iterations V (tracer.fs:373)          */
   uint64_t leaf_visits; /* processLeaf calls L (tracer.fs:380)        */
   uint64_t stack_overflow;
+  uint64_t capped;      /* paths stopped by the refraction safety cap      */
 };
 
 }  // extern "C"
@@ -67,7 +68,7 @@ const float M_TAU = M_PI_F * 2.0f;    /* tracer.fs:13 */
 const float INV_PI = 1.0f / M_PI_F;   /* tracer.fs:14 */
 
 struct Hit { float t; int index; };
-struct Counters { uint64_t rays = 0, nodes = 0, leaves = 0, overflow = 0; };
+struct Counters { uint64_t rays = 0, nodes = 0, leaves = 0, overflow = 0, capped = 0; };
 
 inline int32_t f2i(float f) { int32_t i; memcpy(&i, &f, 4); return i; }
 
@@ -412,7 +413,7 @@ v3 tracePixel(Frag& F, v3 rayOrigin, v3 rayDir, int maxRefractions) {
         rayDir = refract(neg(incident), microNormal, ns.x / ns.y);     /* :486 */
         i--;                                                           /* :488 */
         /* the reference loop is unbounded here; cap documented in DESIGN.md */
-        if (++refractions > maxRefractions) i = NUM_BOUNCES;
+        if (++refractions > maxRefractions) { i = NUM_BOUNCES; F.c.capped++; }
       } else {
         rayDir = F.sampleLambert(macroNormal);                      /* :490 */
         bsdfPdf = lambertPdf(macroNormal, rayDir);                  /* :491 */
@@ -599,11 +600,12 @@ void oracle_trace(const OScene* s, const float* pos4, const float* dir4, int W, 
       fb_out[k] = outc.x; fb_out[k + 1] = outc.y; fb_out[k + 2] = outc.z; fb_out[k + 3] = 1.0f;
     }
     cs[tid].rays += F.c.rays; cs[tid].nodes += F.c.nodes; cs[tid].leaves += F.c.leaves; cs[tid].overflow += F.c.overflow;
+    cs[tid].capped += F.c.capped;
   });
   if (stats)
     for (auto& c : cs) {
       stats->rays += c.rays; stats->node_visits += c.nodes; stats->leaf_visits += c.leaves;
-      stats->stack_overflow += c.overflow;
+      stats->stack_overflow += c.overflow; stats->capped += c.capped;
     }
 }
 

@@ -16,6 +16,7 @@ from fspt_b200 import capi, scenes
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
 import make_reference_outputs as golden  # noqa: E402
+import test_reference_pin as T  # noqa: E402  the pin's case lists: one definition of the inputs of both pins
 
 pytestmark = pytest.mark.gpu
 
@@ -259,6 +260,110 @@ def test_cuda_against_the_reference_shaders_themselves(small_bunny):
         ctx.render(fr, 0, rc, rt)
         golden.check("cuda/tracer/accum_rgb", ctx.read_accum()[..., :3])
         golden.check("cuda/draw/rgba8", ctx.resolve(**REF_POST))
+    finally:
+        ctx.close()
+
+
+# ---------------------------------------------------------------------------------------------------------
+# The CUDA path on the inputs of tests/test_reference_pin.py: every output the reference's shaders computed there,
+# bit for bit, with no oracle in between
+def _pin_camera(name):
+    return T.CAMERA_4K if name == "3840x2160" else T.CAMERAS[T.CAMERA_IDS.index(name)]
+
+
+PIN_CAMERA_IDS = T.CAMERA_IDS + ["3840x2160"]
+BVH_OUTPUTS = ("index", "t", "count", "heat")
+
+
+def pinned_keys():
+    """The stored outputs the tests below check, in the order they check them."""
+    keys = ["camera/%s/%s" % (name, w) for name in PIN_CAMERA_IDS for w in ("pos", "dir")]
+    keys += ["bvh_test/%s/%s/%s" % (name, rays, w) for name in T.SCENES for rays in ("primary", "random")
+             for w in BVH_OUTPUTS]
+    keys += ["tracer/%s/tick%d" % (name, k) for name, _, _, ticks in T.TRACER_CASES for k in range(ticks)]
+    keys += ["tracer/bunny/theta%r" % theta for theta in T.THETAS]
+    keys += ["draw/%s" % p for p in T.POST_IDS]
+    return keys
+
+
+@pytest.mark.parametrize("name", PIN_CAMERA_IDS)
+def test_cuda_camera_against_the_stored_reference_outputs(name):
+    """camera.fs: the near-degenerate basis of the `down` camera (computed on the host, make_frame), the untiled
+    slot -> pixel order of the 37x53 frame, aperture 0.25, randBase 0 and the seed collisions at 3840x2160."""
+    W, H, P, I, fov, lens, rb = _pin_camera(name)
+    sa, _ = T.SCENES["quad_kat"]()
+    ctx = capi.Context(W, H)
+    try:
+        ctx.scene_upload(sa)
+        _, _, _, pos, d = ctx.debug_primary(ctx.frame(P, I, fov, lens, 0.0), rb)
+        golden.check("camera/%s/pos" % name, pos)
+        golden.check("camera/%s/dir" % name, d)
+    finally:
+        ctx.close()
+
+
+@pytest.mark.parametrize("name", list(T.SCENES))
+def test_cuda_bvh_test_against_the_stored_reference_outputs(name):
+    sa, cam = T.SCENES[name]()
+    W, H, rb = T.BVH_PRIMARY
+    ctx = capi.Context(W, H)
+    try:
+        ctx.scene_upload(sa)
+        idx, t, cnt, _, _ = ctx.debug_primary(_frame(ctx, cam), rb, want_rays=False)
+        for rays, (i, tt, c) in (("primary", (idx, t, cnt)), ("random", ctx.debug_trace(*T._random_rays(*T.BVH_RANDOM)))):
+            got = dict(index=i, t=tt, count=c, heat=c.astype(np.float32) * np.float32(0.001))  # bvh_test.fs:230-231
+            for w in BVH_OUTPUTS:
+                golden.check("bvh_test/%s/%s/%s" % (name, rays, w), got[w])
+    finally:
+        ctx.close()
+
+
+@pytest.mark.parametrize("name,W,H,ticks", T.TRACER_CASES)
+def test_cuda_tracer_against_the_stored_reference_outputs(name, W, H, ticks):
+    """The full RGBA accumulator after every tick (the stored alpha is tracer.fs:517's 1.0), one tick per call and all
+    ticks in one call.  No NaN sanitising and no effective refraction cap, like the reference."""
+    sa, cam = T.SCENES[name]()
+    rc, rt = scenes.rand_bases(ticks, T.TRACER_SEED)
+    ctx = capi.Context(W, H)
+    try:
+        ctx.scene_upload(sa)
+        ctx.set_param(capi.PARAM_SANITIZE_NAN, 0)
+        ctx.set_param(capi.PARAM_MAX_REFRACTIONS, 30000)  # the API's maximum; no path of these scenes reaches 64
+        fr = _frame(ctx, cam)
+        for k in range(ticks):
+            ctx.render(fr, k, rc[k:k + 1], rt[k:k + 1])
+            golden.check("tracer/%s/tick%d" % (name, k), ctx.read_accum())
+        ctx.clear()
+        ctx.render(fr, 0, rc, rt)
+        golden.check("tracer/%s/tick%d" % (name, ticks - 1), ctx.read_accum())
+    finally:
+        ctx.close()
+
+
+def test_cuda_rotated_environment_against_the_stored_reference_outputs():
+    sa, cam = T.SCENES["bunny"]()
+    W, H, rb_cam, rb_trace = T.THETA_CASE
+    ctx = capi.Context(W, H)
+    try:
+        ctx.scene_upload(sa)
+        ctx.set_param(capi.PARAM_SANITIZE_NAN, 0)
+        for theta in T.THETAS:
+            ctx.clear()
+            ctx.render(ctx.frame(cam["eye"], cam["dir"], cam["fov_scale"], scenes.lens_features(cam), theta), 0,
+                       [rb_cam], [rb_trace])
+            golden.check("tracer/bunny/theta%r" % theta, ctx.read_accum())
+    finally:
+        ctx.close()
+
+
+@pytest.mark.parametrize("i", range(len(T.POSTS)), ids=T.POST_IDS)
+def test_cuda_post_pass_against_the_stored_reference_outputs(i, oracle_mod):
+    """draw.fs on the pin's accumulator (a firefly, a black pixel), including scale 0.5 and max_sigma 0.5."""
+    fb = T._draw_input(oracle_mod)
+    ctx = capi.Context(fb.shape[1], fb.shape[0])
+    try:
+        ctx.write_accum(fb, 1)
+        golden.check("draw/%s" % T.POST_IDS[i], ctx.resolve(**T.POSTS[i]))
     finally:
         ctx.close()
 

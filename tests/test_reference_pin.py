@@ -46,14 +46,17 @@ def test_camera_fs(case, oracle_mod):
     golden.check("camera/%s/dir" % name, do)
 
 
+# config 5's resolution with the bunny camera
+CAMERA_4K = (3840, 2160, scenes.BUNNY_CAMERA["eye"], scenes.BUNNY_CAMERA["dir"], scenes.BUNNY_CAMERA["fov_scale"],
+             scenes.lens_features(scenes.BUNNY_CAMERA), 8191.25)
+
+
 def test_camera_fs_at_3840x2160(oracle_mod):
     """config 5's resolution: camera.fs:38 seeds with randBase + gl_FragCoord.x * resolution.y + gl_FragCoord.y, above
     2^23 at the right edge, where f32 spacing is 1 and rows start to share seeds (and with them lens samples);
     restatement and shader must collide identically."""
-    cam = scenes.BUNNY_CAMERA
-    lens = np.asarray(scenes.lens_features(cam), np.float32)
-    W, H = 3840, 2160
-    po, do = oracle_mod.camera(W, H, cam["eye"], cam["dir"], cam["fov_scale"], lens, 8191.25)
+    W, H, P, I, fov, lens, rb = CAMERA_4K
+    po, do = oracle_mod.camera(W, H, P, I, fov, np.asarray(lens, np.float32), rb)
     golden.check("camera/3840x2160/pos", po)
     golden.check("camera/3840x2160/dir", do)
     # the collisions are real: 64 rows of the last column share lens samples, 64 rows of column 100 do not
@@ -78,9 +81,13 @@ def _random_rays(n, seed, scale=2.0):
     return pos, d
 
 
+BVH_PRIMARY = (96, 64, 77.0)   # W, H, randBase of the primary rays of test_bvh_test_fs_index_t_count
+BVH_RANDOM = (20000, 5)        # count, seed of its random rays
+
+
 def _bvh_rays(oracle_mod, sa, cam):
     """(primary rays, random rays) of test_bvh_test_fs_index_t_count"""
-    return _primary(oracle_mod, sa, cam, 96, 64, 77.0), _random_rays(20000, 5)
+    return _primary(oracle_mod, sa, cam, *BVH_PRIMARY), _random_rays(*BVH_RANDOM)
 
 
 SCENES = {
@@ -107,6 +114,7 @@ def test_bvh_test_fs_index_t_count(name, oracle_mod):
 
 
 TRACER_CASES = [("bunny", 80, 48, 3), ("pbr_refractive", 64, 40, 3), ("quad_kat", 16, 16, 2), ("soup", 64, 36, 2)]
+TRACER_SEED = 41  # of scenes.rand_bases
 
 
 @pytest.mark.parametrize("name,W,H,ticks", TRACER_CASES)
@@ -114,7 +122,7 @@ def test_tracer_fs_accumulation(name, W, H, ticks, oracle_mod):
     """tracer.fs main() over consecutive ticks with the ping-ponged accumulation target (main.js:758-807)."""
     sa, cam = SCENES[name]()
     O = oracle_mod.Oracle(sa)
-    rc, rt = scenes.rand_bases(ticks, 41)
+    rc, rt = scenes.rand_bases(ticks, TRACER_SEED)
     fo = None
     for k in range(ticks):
         pos, d = _primary(oracle_mod, sa, cam, W, H, rc[k])
@@ -124,14 +132,16 @@ def test_tracer_fs_accumulation(name, W, H, ticks, oracle_mod):
 
 
 THETAS = (0.0, 0.37, -1.25)
+THETA_CASE = (48, 32, 3.5, 4242.0)  # W, H, camera randBase, tracer randBase of the bunny scene
 
 
 def test_tracer_fs_rotated_environment(oracle_mod):
     sa, cam = SCENES["bunny"]()
     O = oracle_mod.Oracle(sa)
+    W, H, rb_cam, rb_trace = THETA_CASE
     for theta in THETAS:
-        pos, d = _primary(oracle_mod, sa, cam, 48, 32, 3.5)
-        fo, _ = O.trace(pos, d, 48, 32, 0, 4242.0, theta, sanitize=0)
+        pos, d = _primary(oracle_mod, sa, cam, W, H, rb_cam)
+        fo, _ = O.trace(pos, d, W, H, 0, rb_trace, theta, sanitize=0)
         golden.check("tracer/bunny/theta%r" % theta, fo)
 
 
@@ -170,3 +180,14 @@ def test_atlas_blit_shader_of_texture_packer_js(res, corrected, sw, oracle_mod):
     ref = R.pack_layer(img, res, corrected, sw)
     assert beq(oracle_mod.pack_layer(img, res, corrected, sw), ref)
     assert beq(capi.pack_layer(img, res, corrected, sw), ref)
+
+
+def test_every_stored_output_is_also_checked_on_the_cuda_path():
+    """tests/test_gpu_parity.py holds the CUDA path to every output stored for this pin, driving it from the case lists
+    above.  A stored output those lists do not produce would be checked against the oracle only."""
+    import test_gpu_parity as G
+    with np.load(golden.PATH) as z:
+        stored = {k.rsplit(":", 1)[0] for k in z.files}
+    pinned = G.pinned_keys()
+    assert len(pinned) == len(set(pinned))
+    assert {k for k in stored if not k.startswith("cuda/")} == set(pinned)

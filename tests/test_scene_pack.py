@@ -103,11 +103,11 @@ def _chain(n, sa):
 
 def test_error_reports_of_the_pre_passes():
     sa, _ = scenes.bunny_class(subdiv=2, atlas_res=16, env_size=(64, 32))
-    ok = capi.debug_pack_scene(_chain(60, sa))               # depth 61: fits the reference's int stack[64]
-    assert ok["depth"] == 61 and ok["n_interior"] == 60
-    with pytest.raises(capi.FsptError) as e:                 # deeper than tracer.fs:368 allows
-        capi.debug_pack_scene(_chain(70, sa))
-    assert e.value.code == -4 and "stack" in str(e.value)
+    ok = capi.debug_pack_scene(_chain(63, sa))               # 64 levels: the sentinel + 63 deferred children fill the
+    assert ok["depth"] == 64 and ok["n_interior"] == 63      # reference's int stack[64] (tracer.fs:368) exactly
+    with pytest.raises(capi.FsptError) as e:                 # 65 levels: one deferred child more than the stack holds
+        capi.debug_pack_scene(_chain(64, sa))
+    assert e.value.code == -4 and "stack" in str(e.value) and "65 levels" in str(e.value)
     cyc = _chain(3, sa)
     cyc.bvh = cyc.bvh.copy()
     cyc.bvh.view(np.int32)[4, 0] = 0                         # an interior node points back at the root
