@@ -450,11 +450,11 @@ int stage_atlas(Ctx* c, const AtlasJob& J) {
     // the distinct varying layers are DMA'd from where they lie, the host does nothing but enqueue the copies.
     bool gpu_interleave = n_tex_mats > 0 && (J.src_pinned || raw_layers.size() * 2 <= (size_t)n_tex_mats * 4);
     if (const char* e = getenv("FSPT_ATLAS_INTERLEAVE")) gpu_interleave = n_tex_mats > 0 && !strcmp(e, "gpu");
-    const bool direct = gpu_interleave && J.src_pinned && !getenv("FSPT_ATLAS_NO_DIRECT");
+    const bool direct = gpu_interleave && J.src_pinned;
     c->atlas_in_place = direct;
-    // wire format of the staged GPU path: RGB, 3 bytes per texel (the shaders never read alpha, tracer.fs:453-456)
-    const bool rgb24 = gpu_interleave && !direct && !getenv("FSPT_ATLAS_RGBA_WIRE");
-    const size_t wire_layer_bytes = rgb24 ? layer_texels * 3 : layer_bytes;
+    // wire format of the staged GPU path: RGB, 3 bytes per texel (the shaders never read alpha, tracer.fs:453-456); the
+    // direct path copies the RGBA8 layers as they lie
+    const size_t wire_layer_bytes = direct ? layer_bytes : layer_texels * 3;
     if (!c->mat_arr || c->mat_R != R || c->mat_L != ML || c->mat_surface != gpu_interleave) {
       if (c->sc.mat_tex) cudaDestroyTextureObject(c->sc.mat_tex);
       c->sc.mat_tex = 0;
@@ -511,36 +511,31 @@ int stage_atlas(Ctx* c, const AtlasJob& J) {
           ACK(cudaMemcpyAsync(reinterpret_cast<uint8_t*>(c->d_raw) + ri * layer_bytes, J.atlas + (size_t)raw_layers[ri] * layer_bytes,
                               layer_bytes, cudaMemcpyHostToDevice, c->copy_stream));
       }
-      // work item = (raw layer, band of rows): copy into the pinned block, DMA the band
+      // work item = (raw layer, band of rows): drop the alpha channel into the pinned block, DMA the band
       const int bands = std::max(1, std::min(R, 16));
       pool.run(direct ? 0 : (int)raw_layers.size() * bands, J.workers, [&](int item) {
         const int ri = item / bands, band = item % bands;
         const size_t y0 = (size_t)R * band / bands, y1 = (size_t)R * (band + 1) / bands;
-        const size_t bpt = rgb24 ? 3 : 4;
-        const size_t off = (size_t)ri * wire_layer_bytes + y0 * R * bpt, bytes = (y1 - y0) * R * bpt;
+        const size_t off = (size_t)ri * wire_layer_bytes + y0 * R * 3, bytes = (y1 - y0) * R * 3;
         const uint8_t* src = J.atlas + (size_t)raw_layers[ri] * layer_bytes + y0 * R * 4;
-        if (!rgb24) {
-          memcpy(c->h_stage + off, src, bytes);
-        } else {
-          uint8_t* dst = c->h_stage + off;
-          const size_t n = (y1 - y0) * R;
-          size_t i = 0;
+        uint8_t* dst = c->h_stage + off;
+        const size_t n = (y1 - y0) * R;
+        size_t i = 0;
 #if defined(__SSSE3__)
-          // 4 texels (16 bytes) -> 12 bytes per shuffle; the 16-byte store's last 4 bytes are overwritten by the next one
-          const __m128i sh = _mm_setr_epi8(0, 1, 2, 4, 5, 6, 8, 9, 10, 12, 13, 14, -1, -1, -1, -1);
-          for (; i + 8 <= n; i += 4)
-            _mm_storeu_si128(reinterpret_cast<__m128i*>(dst + 3 * i),
-                             _mm_shuffle_epi8(_mm_loadu_si128(reinterpret_cast<const __m128i*>(src + 4 * i)), sh));
+        // 4 texels (16 bytes) -> 12 bytes per shuffle; the 16-byte store's last 4 bytes are overwritten by the next one
+        const __m128i sh = _mm_setr_epi8(0, 1, 2, 4, 5, 6, 8, 9, 10, 12, 13, 14, -1, -1, -1, -1);
+        for (; i + 8 <= n; i += 4)
+          _mm_storeu_si128(reinterpret_cast<__m128i*>(dst + 3 * i),
+                           _mm_shuffle_epi8(_mm_loadu_si128(reinterpret_cast<const __m128i*>(src + 4 * i)), sh));
 #endif
-          for (; i < n; ++i) { dst[3 * i] = src[4 * i]; dst[3 * i + 1] = src[4 * i + 1]; dst[3 * i + 2] = src[4 * i + 2]; }
-        }
+        for (; i < n; ++i) { dst[3 * i] = src[4 * i]; dst[3 * i + 1] = src[4 * i + 1]; dst[3 * i + 2] = src[4 * i + 2]; }
         std::lock_guard<std::mutex> g(mu);
         cudaError_t e = cudaMemcpyAsync(reinterpret_cast<uint8_t*>(c->d_raw) + off, c->h_stage + off, bytes, cudaMemcpyHostToDevice, c->copy_stream);
         if (e != cudaSuccess) cuda_err.store((int)e);
       });
       ACK(cudaMemcpyAsync(c->d_mat_src, mat_src, sizeof(MatSrc) * (size_t)n_tex_mats, cudaMemcpyHostToDevice, c->copy_stream));
       const dim3 blk(32, 8), grd((R + 31) / 32, (R + 7) / 8, n_tex_mats);
-      if (rgb24)
+      if (!direct)
         k_interleave_atlas<true><<<grd, blk, 0, c->copy_stream>>>(c->mat_surf, reinterpret_cast<const uint8_t*>(c->d_raw),
                                                                   reinterpret_cast<const MatSrc*>(c->d_mat_src), R, layer_texels);
       else
@@ -1079,10 +1074,9 @@ int fspt_create(fspt_ctx** out, int32_t width, int32_t height, int32_t device) {
     per_sm = std::max(1, per_sm);
     cudaFuncAttributes fa{};
     cudaFuncGetAttributes(&fa, kernel);
-    if (!getenv("FSPT_NO_CARVEOUT") && max_smem_sm > 0) {
+    if (max_smem_sm > 0) {
       const size_t need = (size_t)per_sm * (fa.sharedSizeBytes + 1024);  // + the per-CTA reservation
-      int pct = (int)std::min<size_t>(100, (need * 100 + (size_t)max_smem_sm - 1) / (size_t)max_smem_sm);
-      if (const char* e = getenv("FSPT_CARVEOUT_PCT")) pct = std::max(0, std::min(100, atoi(e)));  // measurement knob
+      const int pct = (int)std::min<size_t>(100, (need * 100 + (size_t)max_smem_sm - 1) / (size_t)max_smem_sm);
       cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     }
     return per_sm * c->sm_count;

@@ -23,8 +23,8 @@ __global__ void __launch_bounds__(256) k_camera(const FrameParams f, const float
   v3 o, d;
   int x, y;
   camera_ray(f, rb_cam, div_s, p, o, d, x, y);
-  st_path(ps.ro(p), make_float4(o.x, o.y, o.z, FSPT_MAX_T));
-  st_path(ps.rd(p), make_float4(d.x, d.y, d.z, __int_as_float(-1)));
+  ps.ro(p) = make_float4(o.x, o.y, o.z, FSPT_MAX_T);
+  ps.rd(p) = make_float4(d.x, d.y, d.z, __int_as_float(-1));
   if (cam_pos_out) {  // frame-sized targets
     const size_t px = (size_t)(y + f.ry0) * f.width + (size_t)(x + f.rx0);
     cam_pos_out[px] = make_float4(o.x, o.y, o.z, 1.0f);
@@ -282,18 +282,18 @@ __device__ __forceinline__ void write_sample(const ShadeArgs& A, int slot, v3 co
 __device__ __forceinline__ void shade_miss(const ShadeArgs& A, int pos) {
   const int slot_in = pos;  // record position in A.ps
   int slot = pos;           // path identity (pixel * S + sample); equals the position only in the first pass
-  const float4 d4 = ld_path(A.ps.rd(slot_in));
+  const float4 d4 = A.ps.rd(slot_in);
   const v3 rayDir = mk3(d4.x, d4.y, d4.z);
   const v3 env = env_sample(A.sc, rayDir, A.f.env_theta);
   v3 color;
   if (A.first) {
     color = add(mk3(0.0f, 0.0f, 0.0f), env);  // :443
   } else {
-    const float4 c4 = ld_path(A.ps.col(slot_in)), t4 = ld_path(A.ps.thr(slot_in));
+    const float4 c4 = A.ps.col(slot_in), t4 = A.ps.thr(slot_in);
     slot = __float_as_int(c4.w);
     color = mk3(c4.x, c4.y, c4.z);
     if (A.ps.sh[slot_in] == 2) {  // shadow.index == -1, :502-504
-      const float4 p4 = ld_path(A.ps.pend(slot_in));
+      const float4 p4 = A.ps.pend(slot_in);
       color = add(color, mk3(p4.x, p4.y, p4.z));
     }
     const v3 reflectance = mk3(t4.x, t4.y, t4.z);                 // accumulatedReflectance *= bsdfThroughput (:508) was
@@ -308,14 +308,14 @@ __device__ __forceinline__ void shade_miss(const ShadeArgs& A, int pos) {
 struct PathRecord { float4 w[6]; };
 __device__ __forceinline__ void store_record(const PathState& ps, int pos, const PathRecord& rec, bool shadow) {
   float4* dst = ps.rec + FSPT_PATH_WORDS * (size_t)pos;
-  st_path(dst[0], rec.w[0]); st_path(dst[1], rec.w[1]); st_path(dst[2], rec.w[3]); st_path(dst[3], rec.w[4]); st_path(dst[4], rec.w[5]);
+  dst[0] = rec.w[0]; dst[1] = rec.w[1]; dst[2] = rec.w[3]; dst[3] = rec.w[4]; dst[4] = rec.w[5];
   ps.sh[pos] = shadow ? 1 : 0;  // (every record: a stale 2 of an earlier bounce must not survive at this position)
 }
 template <bool MAT_TEX>
 __device__ __forceinline__ bool shade_hit(const ShadeArgs& A, int pos, bool& shadow, PathRecord& out) {
   const DeviceScene& sc = A.sc;
   int slot = pos;  // path identity; equals the record position only in the first pass
-  const float4 o4 = ld_path(A.ps.ro(pos)), d4 = ld_path(A.ps.rd(pos));
+  const float4 o4 = A.ps.ro(pos), d4 = A.ps.rd(pos);
   v3 rayOrigin = mk3(o4.x, o4.y, o4.z), rayDir = mk3(d4.x, d4.y, d4.z);
   const float hit_t = o4.w;
   const int hit_index = __float_as_int(d4.w);
@@ -327,8 +327,8 @@ __device__ __forceinline__ bool shade_hit(const ShadeArgs& A, int pos, bool& sha
     color = mk3(0.0f, 0.0f, 0.0f);
     reflectance = mk3(1.0f, 1.0f, 1.0f);
   } else {
-    const float4 c4 = ld_path(A.ps.col(pos)), t4 = ld_path(A.ps.thr(pos));
-    const float4 p4 = ld_path(A.ps.pend(pos));
+    const float4 c4 = A.ps.col(pos), t4 = A.ps.thr(pos);
+    const float4 p4 = A.ps.pend(pos);
     const int shadow_state = A.ps.sh[pos];
     slot = __float_as_int(c4.w);
     color = mk3(c4.x, c4.y, c4.z);
@@ -505,10 +505,6 @@ __device__ __forceinline__ bool shade_hit(const ShadeArgs& A, int pos, bool& sha
 #ifndef SHADE_THREADS
 #define SHADE_THREADS 256
 #endif
-#ifndef SHADE_BLOCK_APPEND
-#define SHADE_BLOCK_APPEND 0  /* 1: one atomicAdd per block and list instead of one per warp -- measured shade +2 % (the two
-                                 extra block barriers cost more than the 8x fewer same-address atomics save) */
-#endif
 #ifndef SHADE_MIN_BLOCKS
 #define SHADE_MIN_BLOCKS 4  // 64 registers, 32 warps/SM.  Measured shading time vs 128 threads x 6 blocks (80 regs):
                             // 128x5 +8 %, 128x7 -7 %, 128x8 -5.5 %, 224x4 -8 %, 256x4 -9 %, 448x2 -3 %, 64x14 -5.5 %
@@ -529,9 +525,6 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS) k_shade(const
   // SHADE_THREADS items of one kind, so hit shading and miss shading never share a warp (or a block)
   __shared__ int q_hit[2 * SHADE_THREADS], q_miss[2 * SHADE_THREADS];
   __shared__ int s_hits[SHADE_THREADS / 32], s_miss[SHADE_THREADS / 32];
-#if SHADE_BLOCK_APPEND
-  __shared__ int s_wc[SHADE_THREADS / 32], s_ws[SHADE_THREADS / 32], s_base[2];
-#endif
   const int n = A.counts_in[0];
   const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
   int nh = 0, nm = 0;  // queue fill, block-uniform
@@ -564,45 +557,16 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS) k_shade(const
       PathRecord rec;
       if ((int)threadIdx.x < take) cont = shade_hit<MAT_TEX>(A, q_hit[nh - take + threadIdx.x], shadow, rec);
       // stream compaction of the surviving paths: the new record goes to the next free position of ps_out
-#if SHADE_BLOCK_APPEND
-      // one atomicAdd per BLOCK and list instead of one per warp: the per-warp counts are prefix-summed in shared memory
-      // (the two counters of a launch are hit by every group of every block; 8x fewer same-address atomics)
-      const unsigned mc = __ballot_sync(0xffffffffu, cont), ms = __ballot_sync(0xffffffffu, shadow);
-      if (lane == 0) { s_wc[warp] = __popc(mc); s_ws[warp] = __popc(ms); }
-      __syncthreads();
-      if (threadIdx.x == 0) {
-        int tc = 0, ts = 0;
-#pragma unroll
-        for (int w = 0; w < SHADE_THREADS / 32; ++w) {
-          const int a = s_wc[w], b = s_ws[w];
-          s_wc[w] = tc; s_ws[w] = ts;
-          tc += a; ts += b;
-        }
-        const int bc = tc ? atomicAdd(A.counts_out + 0, tc) : 0;
-        const int bs = ts ? atomicAdd(A.counts_out + 1, ts) : 0;
-        s_base[0] = bc; s_base[1] = bs;
-      }
-      __syncthreads();
-      const unsigned lt2 = (1u << lane) - 1u;
-      const int pos_out = s_base[0] + s_wc[warp] + __popc(mc & lt2);
-      if (cont) store_record(A.ps_out, pos_out, rec, shadow);
-      if (shadow) {
-        float4* sr = A.shadow_rays_out + 2 * (size_t)(s_base[1] + s_ws[warp] + __popc(ms & lt2));
-        sr[0] = make_float4(rec.w[0].x, rec.w[0].y, rec.w[0].z, __int_as_float(pos_out));
-        sr[1] = rec.w[2];
-      }
-#else
       const int pos_out = append_pos(cont, A.counts_out + 0);
       if (cont) store_record(A.ps_out, pos_out, rec, shadow);
       {
         const int j = append_pos(shadow, A.counts_out + 1);
         if (shadow) {  // origin = the continuation ray's (tracer.fs:501), direction = the sampled environment direction
           float4* sr = A.shadow_rays_out + 2 * (size_t)j;
-          st_path(sr[0], make_float4(rec.w[0].x, rec.w[0].y, rec.w[0].z, __int_as_float(pos_out)));
-          st_path(sr[1], rec.w[2]);
+          sr[0] = make_float4(rec.w[0].x, rec.w[0].y, rec.w[0].z, __int_as_float(pos_out));
+          sr[1] = rec.w[2];
         }
       }
-#endif
       nh -= take;
       __syncthreads();
     }

@@ -52,25 +52,13 @@ struct TraceArgs {
 #ifndef TRACE_THREADS
 #define TRACE_THREADS 128
 #endif
-#ifndef TRACE_NODE_TEX
-#define TRACE_NODE_TEX 3   /* bit k: word k of the node record comes through the texture pipe, the others through the LSU
-                               (measured with 36 warps/SM: words 0,1 via TLD + words 2,3 via LDG is 0.5 % / 2.5 % faster than all
-                               four via TLD on the 82 k / 1 M-triangle scenes; all via LDG is 2 % / 11 % slower) */
-#endif
 #ifndef TRACE_REFILL
 #define TRACE_REFILL 16      /* a warp fetches new rays when fewer lanes than this still hold one (with 36 warps/SM:
                                 16 is 2.3 % faster than 12 on the 82 k-triangle scene, 1.8 % slower on 1 M triangles) */
 #endif
 #ifndef TRACE_SMEM_STACK
-#define TRACE_SMEM_STACK 12  /* stack entries per thread held in shared memory (0 = all in local memory) */
-#endif
-#ifndef TRACE_BCAST
-#define TRACE_BCAST 1        /* 1: ray origin / inverse direction are scalars, packed at the use site (ptxas folds the (x, x)
-                                pair into the `.F32` broadcast operand of FADD2 / FMUL2); 0: materialised (x, x) register pairs */
-#endif
-#ifndef TRACE_SMEM_RAY
-#define TRACE_SMEM_RAY 1     /* 1: per-ray values used by one phase only (1/d: interior steps, d: leaf steps, slot: retirement)
-                                live in shared memory [value][thread] instead of registers */
+#define TRACE_SMEM_STACK 12  /* stack entries per thread held in shared memory; the rest spill to local memory
+                                (0: every entry spills) */
 #endif
 #ifndef TRACE_MIN_BLOCKS
 #define TRACE_MIN_BLOCKS 9   /* resident CTAs per SM the register allocation is held to (9 x 128 threads = 56 registers) */
@@ -150,26 +138,23 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
   __syncthreads();
 
   // Per-lane on-chip state, ONE shared array laid out [row][thread] (bank = lane for any per-lane row: conflict-free):
-  //   rows 0..6  (TRACE_SMEM_RAY) ray values that only one phase reads -- d (leaf steps), 1/d (interior steps), record
-  //              position (retirement) -- so they stay out of the register file; their loads overlap the node /
-  //              triangle fetch of the same step;
-  //   rows 7..   (TRACE_SMEM_STACK) the first entries of the traversal stack; deeper entries spill to local memory.
+  //   rows 0..6  ray values that only one phase reads -- d (leaf steps), 1/d (interior steps), record position
+  //              (retirement) -- so they stay out of the register file; their loads overlap the node / triangle fetch
+  //              of the same step;
+  //   rows 7..   the first TRACE_SMEM_STACK entries of the traversal stack; deeper entries spill to local memory.
   // `lane_addr` is the 32-bit shared-window address of the thread's column, `sp` the BYTE offset of its next free stack
   // entry inside the column (row * 4 * TRACE_THREADS), so one register is the depth and (plus lane_addr) the address, and
   // "still in shared memory" is a comparison with a constant.  Every access is an explicit ld.shared / st.shared on
   // [lane_addr + offset]: when the arrays were indexed through C++ pointers ptxas rebuilt the shared-window base
   // (S2R SR_CgaCtaId + 3 instructions) in front of every push and pop, on the pop -> node-fetch dependency chain.  The
   // address is passed through an opaque `mov` once so that it lives in one register instead of being rematerialised.
-  constexpr int RAY_ROWS = TRACE_SMEM_RAY ? 7 : 0;
+  constexpr int RAY_ROWS = 7;
   constexpr unsigned ROW = 4u * TRACE_THREADS;
-#if TRACE_SMEM_RAY || TRACE_SMEM_STACK
   __shared__ int s_lane[(RAY_ROWS + TRACE_SMEM_STACK) * TRACE_THREADS];
   unsigned lane_addr;
   asm volatile("mov.u32 %0, %1;" : "=r"(lane_addr) : "r"((unsigned)__cvta_generic_to_shared(s_lane) + 4u * threadIdx.x));
 #define LANE_LD(dst, off) asm volatile("ld.shared.b32 %0, [%1];" : "=r"(dst) : "r"(lane_addr + (off)))
 #define LANE_ST(off, v) asm volatile("st.shared.b32 [%0], %1;" ::"r"(lane_addr + (off)), "r"(v))
-#endif
-#if TRACE_SMEM_STACK
   int spill[FSPT_STACK - TRACE_SMEM_STACK];
   constexpr unsigned SP0 = ROW * RAY_ROWS, SMEM_END = ROW * (RAY_ROWS + TRACE_SMEM_STACK);
 #define STACK_PUSH(v)                                                              \
@@ -185,36 +170,18 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
     if (sp < SMEM_END) LANE_LD(dst, sp);                                           \
     else dst = spill[(sp - SMEM_END) / ROW];                                       \
   } while (0)
-#else
-  int stack[FSPT_STACK];
-  constexpr unsigned SP0 = 0;
-#define STACK_PUSH(v) do { stack[sp++] = (v); } while (0)
-#define STACK_POP(dst) do { dst = stack[--sp]; } while (0)
-#endif
   int cur = FSPT_SENTINEL;
   unsigned sp = SP0;
   unsigned cnt = 0;  // visits of the current ray: low 16 bits all nodes, high 16 bits leaves (statistics; the bvh_test
                      // count of the WRITE_COUNT variant is kept separately and exact)
   int cnt_exact = 0;
   bool kind = false, have = false;
-#if TRACE_SMEM_RAY
   enum { R_DX = 0, R_DY = 1, R_DZ = 2, R_IX = 3, R_IY = 4, R_IZ = 5, R_SLOT = 6 };
 #define RAY_GET(row) ([&] { int v_; LANE_LD(v_, (row) * ROW); return v_; }())
 #define RAY_GETF(row) __int_as_float(RAY_GET(row))
 #define RAY_SET(row, v) LANE_ST((row) * ROW, (int)(v))
 #define RAY_SETF(row, v) LANE_ST((row) * ROW, __float_as_int(v))
-#else
-  enum { R_DX = 0, R_DY = 1, R_DZ = 2, R_IX = 3, R_IY = 4, R_IZ = 5, R_SLOT = 6 };
-  int r_val[7] = {0, 0, 0, 0, 0, 0, -1};  // constant indices only: registers
-#define RAY_GET(row) r_val[row]
-#define RAY_GETF(row) __int_as_float(r_val[row])
-#define RAY_SET(row, v) (r_val[row] = (int)(v))
-#define RAY_SETF(row, v) (r_val[row] = __float_as_int(v))
-#endif
   float ox = 0, oy = 0, oz = 0;
-#if !TRACE_BCAST
-  f32x2 ox2 = 0, oy2 = 0, oz2 = 0, ix2 = 0, iy2 = 0, iz2 = 0;
-#endif
   float tbest = FSPT_MAX_T;
   int ibest = -1;
   unsigned n_nodes = 0, n_leaves = 0;  // per thread and launch: far below 2^32 (touched at retirement only)
@@ -228,12 +195,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
     RAY_SET(R_SLOT, slot);
     RAY_SETF(R_DX, dx); RAY_SETF(R_DY, dy); RAY_SETF(R_DZ, dz);
     const float ix = 1.0f / dx, iy = 1.0f / dy, iz = 1.0f / dz;  // `vec3 inverse = 1.0 / ray.dir`, tracer.fs:318
-#if TRACE_BCAST
     RAY_SETF(R_IX, ix); RAY_SETF(R_IY, iy); RAY_SETF(R_IZ, iz);
-#else
-    ox2 = pack2(ox, ox); oy2 = pack2(oy, oy); oz2 = pack2(oz, oz);
-    ix2 = pack2(ix, ix); iy2 = pack2(iy, iy); iz2 = pack2(iz, iz);
-#endif
     have = true;
     tbest = FSPT_MAX_T; ibest = -1; cnt = 0; cnt_exact = 0;
     sp = SP0;
@@ -247,11 +209,11 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
     if (retire) {  // retire the finished ray
       const int slot = RAY_GET(R_SLOT);
       if (CAMERA) {
-        st_path(A.ps.ro(slot), make_float4(ox, oy, oz, tbest));
-        st_path(A.ps.rd(slot), make_float4(RAY_GETF(R_DX), RAY_GETF(R_DY), RAY_GETF(R_DZ), __int_as_float(ibest)));
+        A.ps.ro(slot) = make_float4(ox, oy, oz, tbest);
+        A.ps.rd(slot) = make_float4(RAY_GETF(R_DX), RAY_GETF(R_DY), RAY_GETF(R_DZ), __int_as_float(ibest));
       } else if (!kind) {
-        st_path_w(A.ps.ro(slot), tbest);
-        st_path_w(A.ps.rd(slot), __int_as_float(ibest));
+        A.ps.ro(slot).w = tbest;
+        A.ps.rd(slot).w = __int_as_float(ibest);
       } else {
         A.ps.sh[slot] = (ibest == -1) ? 2 : 3;  // the record's shadow-state byte
       }
@@ -285,7 +247,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
             // (origin | record position, direction | -), no indirection through a list
             kind = my >= n_cont;
             const float4* src = kind ? A.shadow_rays + 2 * (size_t)(my - n_cont) : &A.ps.ro(my);
-            const float4 o4 = ld_path(src[0]), d4 = ld_path(src[1]);
+            const float4 o4 = src[0], d4 = src[1];
             // shadow rays always; continuation rays when k_shade marked the path's last bounce (index word = -2)
             boolean_ray = A.anyhit && (kind || __float_as_int(d4.w) == -2);
             start_ray(o4, d4, kind ? __float_as_int(o4.w) : my);
@@ -310,19 +272,17 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
           if (WRITE_COUNT) cnt_exact++;
           cnt++;
           // The record's four words are split between the two L1 data pipes (texture fetch / LSU load): the
-          // kernel is bound by L1 wavefronts (ncu: l1tex data-pipe ~60 % busy), not by issue slots.
+          // kernel is bound by L1 wavefronts (ncu: l1tex data-pipe ~60 % busy), not by issue slots.  Measured with
+          // 36 warps/SM: words 0,1 via TLD + words 2,3 via LDG is 0.5 % / 2.5 % faster than all four via TLD on the
+          // 82 k / 1 M-triangle scenes; all four via LDG is 2 % / 11 % slower.
           const float4* np = A.nodes + 4 * (size_t)cur;
-          const float4 a = ((TRACE_NODE_TEX & 1) && NODE_TEX) ? tex1Dfetch<float4>(A.nodes_tex, 4 * cur) : __ldg(np);
-          const float4 b = ((TRACE_NODE_TEX & 2) && NODE_TEX) ? tex1Dfetch<float4>(A.nodes_tex, 4 * cur + 1) : __ldg(np + 1);
-          const float4 c = ((TRACE_NODE_TEX & 4) && NODE_TEX) ? tex1Dfetch<float4>(A.nodes_tex, 4 * cur + 2) : __ldg(np + 2);
-          const float4 df = ((TRACE_NODE_TEX & 8) && NODE_TEX) ? tex1Dfetch<float4>(A.nodes_tex, 4 * cur + 3) : __ldg(np + 3);
+          const float4 a = NODE_TEX ? tex1Dfetch<float4>(A.nodes_tex, 4 * cur) : __ldg(np);
+          const float4 b = NODE_TEX ? tex1Dfetch<float4>(A.nodes_tex, 4 * cur + 1) : __ldg(np + 1);
+          const float4 c = __ldg(np + 2);
+          const float4 df = __ldg(np + 3);
           const int cl = __float_as_int(df.x), cr = __float_as_int(df.y);
           float lh, rh;
-#if TRACE_BCAST
           slab_pair(a, b, c, bc2(ox), bc2(oy), bc2(oz), bc2(RAY_GETF(R_IX)), bc2(RAY_GETF(R_IY)), bc2(RAY_GETF(R_IZ)), lh, rh);
-#else
-          slab_pair(a, b, c, ox2, oy2, oz2, ix2, iy2, iz2, lh, rh);
-#endif
           const bool tl = lh < tbest, tr = rh < tbest;
           const bool right_first = lh > rh;                   // tracer.fs:384 (ties go left)
           if (tl && tr) {

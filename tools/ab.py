@@ -3,7 +3,7 @@
 fspt_b200/lib/variants/ (they travel to the GPU box with the snapshot) and prints the gpurun command that times the
 default build and every variant with tools/quick.py.
 
-  python tools/ab.py r16:-DTRACE_REFILL=16 nt0:-DTRACE_NODE_TEX=0 --scenes bunny soup
+  python tools/ab.py r16:-DTRACE_REFILL=16 st8:-DTRACE_SMEM_STACK=8 --scenes bunny soup
 """
 import argparse, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
