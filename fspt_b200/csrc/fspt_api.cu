@@ -43,6 +43,91 @@ namespace {
 
 thread_local std::string g_create_error;
 
+// A block of device memory (DevBuf) or page-locked host memory (PinnedBuf) that only grows: fit() keeps it when it is
+// large enough and re-allocates it otherwise.  Freed on destruction.
+template <class T, bool Pinned>
+struct GrowBuf {
+  T* p = nullptr;
+  size_t cap = 0;  // bytes
+  GrowBuf() = default;
+  GrowBuf(const GrowBuf&) = delete;
+  GrowBuf& operator=(const GrowBuf&) = delete;
+  ~GrowBuf() { release(); }
+  cudaError_t fit(size_t bytes) {
+    if (p && cap >= bytes) return cudaSuccess;
+    release();
+    void* q = nullptr;
+    const cudaError_t e = Pinned ? cudaMallocHost(&q, bytes) : cudaMalloc(&q, bytes);
+    if (e == cudaSuccess) { p = static_cast<T*>(q); cap = bytes; }
+    return e;
+  }
+  void release() {
+    if (p) { if (Pinned) cudaFreeHost(p); else cudaFree(p); }
+    p = nullptr; cap = 0;
+  }
+};
+template <class T> using DevBuf = GrowBuf<T, false>;
+template <class T> using PinnedBuf = GrowBuf<T, true>;
+
+// A CUDA array (2D when layers == 0, layered otherwise) with its texture object -- point-sampled, clamped, element
+// reads -- and, for an array a kernel writes, its surface object.  fit() keeps the array when the format, shape and
+// surface flag match and re-creates it otherwise.  Freed on destruction.
+struct TexArray {
+  cudaArray_t arr = nullptr;
+  cudaTextureObject_t tex = 0;
+  cudaSurfaceObject_t surf = 0;
+  cudaChannelFormatDesc fmt{};
+  int w = 0, h = 0, layers = 0;
+  bool surface = false;
+  TexArray() = default;
+  TexArray(const TexArray&) = delete;
+  TexArray& operator=(const TexArray&) = delete;
+  ~TexArray() { release(); }
+  cudaError_t fit(cudaChannelFormatDesc f, int w_, int h_, int layers_, bool surface_) {
+    if (arr && !memcmp(&f, &fmt, sizeof f) && w == w_ && h == h_ && layers == layers_ && surface == surface_)
+      return cudaSuccess;
+    release();
+    const unsigned flags = surface_ ? cudaArraySurfaceLoadStore : 0;
+    cudaError_t e = layers_ ? cudaMalloc3DArray(&arr, &f, make_cudaExtent(w_, h_, layers_), cudaArrayLayered | flags)
+                            : cudaMallocArray(&arr, &f, w_, h_, flags);
+    if (e != cudaSuccess) { arr = nullptr; return e; }
+    cudaResourceDesc rd = {};
+    rd.resType = cudaResourceTypeArray;
+    rd.res.array.array = arr;
+    cudaTextureDesc td = {};
+    td.addressMode[0] = td.addressMode[1] = td.addressMode[2] = cudaAddressModeClamp;
+    td.filterMode = cudaFilterModePoint;
+    td.readMode = cudaReadModeElementType;
+    e = cudaCreateTextureObject(&tex, &rd, &td, nullptr);
+    if (e == cudaSuccess && surface_) e = cudaCreateSurfaceObject(&surf, &rd);
+    if (e != cudaSuccess) { release(); return e; }
+    fmt = f; w = w_; h = h_; layers = layers_; surface = surface_;
+    return cudaSuccess;
+  }
+  void release() {
+    if (surf) cudaDestroySurfaceObject(surf);
+    if (tex) cudaDestroyTextureObject(tex);
+    if (arr) cudaFreeArray(arr);
+    arr = nullptr; tex = 0; surf = 0;
+    w = h = layers = 0; surface = false;
+  }
+};
+
+// A resident scene apart from its atlas: what fspt_scene_upload derived from the host buffers and what
+// fspt_scene_broadcast sends to the other ranks.  Both size the buffers by it (fit_scene) and make it the scene the
+// kernels read (publish_scene).
+struct SceneInfo {
+  uint64_t bytes_nodes, bytes_tris, bytes_shade, bytes_bins, scene_bytes;
+  int32_t root_ref, n_tris, n_interior, atlas_res, atlas_layers, env_w, env_h, n_bins, has_dielectric;
+};
+
+// The resident atlas: what stage_atlas made of the caller's layers and what phase 2 of fspt_scene_broadcast sends.
+struct AtlasInfo {
+  uint64_t bytes_layer_info, bytes_mat_info;
+  int32_t interleaved;  // 1: the material-interleaved array (one layer per textured material), 0: the plain RGBA8 array
+  int32_t res, layers;
+};
+
 struct Ctx {
   int device = 0, sm_count = 0;
   int width = 0, height = 0, n_pixels = 0;
@@ -55,23 +140,19 @@ struct Ctx {
   bool render_timed = false;
   std::string error;
 
-  // scene
-  bool has_scene = false, has_dielectric = false;
-  DeviceScene sc{};
-  void *d_nodes = nullptr, *d_tris = nullptr, *d_shade = nullptr, *d_bins = nullptr, *d_layer_info = nullptr;
-  cudaArray_t atlas_arr = nullptr, env_arr = nullptr, mat_arr = nullptr;
-  int mat_R = 0, mat_L = 0;
-  bool mat_surface = false;           // mat_arr was created with cudaArraySurfaceLoadStore (GPU-side interleave)
-  cudaSurfaceObject_t mat_surf = 0;   // write view of mat_arr for k_interleave_atlas
-  void* d_raw = nullptr;              // distinct varying atlas layers as uploaded (RGBA8), source of the GPU interleave
-  void* d_mat_src = nullptr;          // MatSrc per textured material
-  size_t cap_raw = 0, cap_mat_src = 0;
-  void* d_mat_info = nullptr;
-  size_t cap_mat_info = 0;
+  // scene: buffers and arrays are kept across uploads and reused when they fit
+  bool has_scene = false;
+  SceneInfo info{};
+  AtlasInfo atlas_info{};
+  DeviceScene sc{};  // the kernels' view, set by publish_scene / publish_atlas
+  DevBuf<uint8_t> d_nodes, d_tris, d_shade, d_bins;
+  DevBuf<uint2> d_layer_info;
+  DevBuf<int4> d_mat_info;
+  TexArray env, mat, atlas;           // mat: the material-interleaved atlas; atlas: the plain RGBA8 one (one of the two)
+  DevBuf<uint8_t> d_raw;              // distinct varying atlas layers as uploaded (RGBA8), source of the GPU interleave
+  DevBuf<uint8_t> d_mat_src;          // MatSrc per textured material
   cudaTextureObject_t nodes_tex = 0;  // the node array again as a linear texture (second L1 data pipe)
-  int atlas_R = 0, atlas_L = 0, env_W = 0, env_H = 0;       // dims of the resident arrays (reused across uploads)
-  size_t cap_nodes = 0, cap_tris = 0, cap_shade = 0, cap_bins = 0, cap_layer_info = 0;
-  uint8_t* h_stage = nullptr;                               // pinned staging for the atlas (one slot per layer)
+  PinnedBuf<uint8_t> h_stage;         // pinned staging for the atlas (one slot per layer)
   cudaStream_t copy_stream = nullptr;                       // atlas DMA, overlaps the primary traversal
   cudaEvent_t ev_atlas = nullptr;
   // fspt_scene_upload_async: the atlas part of the upload (constant-layer scan, host interleave into pinned memory,
@@ -85,21 +166,17 @@ struct Ctx {
   int atlas_rc = 0;            // outcome of the atlas part (written by the atlas thread, read after joining it)
   std::string atlas_error;
   HostPool* pool = nullptr;    // host workers of fspt_scene_upload (created at the first upload)
-  uint8_t* h_ring = nullptr;   // pinned ring the geometry records are staged through, chunk by chunk
-  size_t ring_bytes = 0;
+  PinnedBuf<uint8_t> h_ring;   // pinned ring the geometry records are staged through, chunk by chunk
   std::vector<cudaEvent_t> ev_ring;  // per ring slot: the copies that read it have completed
-  uint8_t* h_geo = nullptr;                                 // pinned block of the small tables (bins, layer / material tables) + env
-  size_t geo_stage_bytes = 0;
-  size_t stage_bytes = 0;
-  size_t scene_bytes = 0;
+  PinnedBuf<uint8_t> h_geo;    // pinned block of the small tables (bins, layer / material tables) + env
 
   // frame state
-  float4* d_fb = nullptr;          // accumulation target (RGBA32F)
-  float4* d_last_color = nullptr;
-  float4* d_sample_color = nullptr;
-  float4* d_cam_pos = nullptr;     // debug_primary only
-  float4* d_cam_dir = nullptr;
-  uchar4* d_rgba8 = nullptr;
+  DevBuf<float4> d_fb;             // accumulation target (RGBA32F)
+  DevBuf<float4> d_last_color;
+  DevBuf<float4> d_sample_color;
+  DevBuf<float4> d_cam_pos;        // debug_primary only
+  DevBuf<float4> d_cam_dir;
+  DevBuf<uchar4> d_rgba8;
   uint32_t next_tick = 0;
   uint64_t accum_samples = 0;
   int accum_mode = 0;
@@ -113,37 +190,35 @@ struct Ctx {
   size_t wave_paths = 0;
   PathState ps{};             // = ps2[0] (debug entry points)
   PathState ps2[2]{};         // dense path-record arrays, ping-pong: shade reads one, compacts survivors into the other
-  float4* d_shadow = nullptr; // shadow rays of the current bounce, dense: origin | record position, direction | -
-  int* d_counts = nullptr;    // set k at [2k, 2k+1] = (#continuation, #shadow), [32] fetch cursor (own cache line)
-  int* d_count_out = nullptr; // per-slot visit count (debug)
-  unsigned char* d_hit_flag = nullptr;  // hit / miss per record position
-  unsigned long long* d_stats = nullptr;  // rays, nodes, leaves, capped
-  float* d_rb = nullptr;      // rand bases of one render call: [0,cap) camera, [cap,2cap) tracer
+  DevBuf<float4> d_rec[2];    // what ps2[k] points to
+  DevBuf<unsigned char> d_sh[2];
+  DevBuf<float4> d_shadow;    // shadow rays of the current bounce, dense: origin | record position, direction | -
+  DevBuf<int> d_counts;       // set k at [2k, 2k+1] = (#continuation, #shadow), [32] fetch cursor (own cache line)
+  DevBuf<int> d_count_out;    // per-slot visit count (debug)
+  DevBuf<unsigned char> d_hit_flag;  // hit / miss per record position
+  DevBuf<unsigned long long> d_stats;  // rays, nodes, leaves, capped
+  DevBuf<float> d_rb;         // rand bases of one render call: [0,cap) camera, [cap,2cap) tracer
   // pinned staging, a ring of RB_SLOTS blocks of 2*rb_cap floats: a slot is rewritten only after the copy that last
   // read it has completed (its event), so fspt_render never waits for the GPU to drain
   static constexpr int RB_SLOTS = 8;
-  float* h_rb = nullptr;
+  PinnedBuf<float> h_rb;
   cudaEvent_t ev_rb[RB_SLOTS] = {};
   int rb_slot = 0;
   int rb_cap = 0;
   // refraction bounces beyond NUM_BOUNCES (tracer.fs:488): path counts polled two iterations behind the enqueue
   static constexpr int POLL_SLOTS = 8;
-  int* h_poll = nullptr;      // pinned
+  PinnedBuf<int> h_poll;
   cudaEvent_t ev_poll[POLL_SLOTS] = {};
   // collectives (fspt_comm_init): NCCL communicator over NVLink / NVSwitch
   ncclComm_t comm = nullptr;
   int comm_rank = 0, comm_world = 1;
   cudaEvent_t ev_red0 = nullptr, ev_red1 = nullptr;  // around the last fspt_reduce_accum
   bool reduce_timed = false;
-  void* d_lin = nullptr;      // linear staging of the environment + atlas arrays for fspt_scene_broadcast
-  size_t cap_lin = 0;
-  void* d_hdr = nullptr;      // broadcast headers
-  void* d_lin_env = nullptr;  // linear staging of the environment array (phase 1 of the broadcast)
-  size_t cap_lin_env = 0;
+  DevBuf<uint8_t> d_lin;      // linear staging of the atlas array for fspt_scene_broadcast (phase 2)
+  DevBuf<uint8_t> d_hdr;      // broadcast headers
+  DevBuf<uint8_t> d_lin_env;  // linear staging of the environment array (phase 1 of the broadcast)
   int bcast_pending_root = -1;  // >= 0: phase 2 of fspt_scene_broadcast (the atlas) has not been issued yet
   cudaEvent_t ev_bcast = nullptr;  // end of phase 1 on the context's stream
-  size_t bytes_nodes = 0, bytes_tris = 0, bytes_shade = 0, bytes_bins = 0, bytes_layer_info = 0,
-         bytes_mat_info = 0;
   int trace_blocks = 0, trace_blocks_cnt = 0, trace_blocks_cam = 0, shade_blocks = 0;
   int trace_blocks_nt = 0, trace_blocks_cnt_nt = 0, trace_blocks_cam_nt = 0;  // NODE_TEX = false instantiations
 
@@ -163,52 +238,79 @@ int fail(Ctx* c, int code, const char* fmt, ...) {
   return code;
 }
 
-#define CK(call)                                                                                  \
-  do {                                                                                            \
-    cudaError_t e_ = (call);                                                                      \
-    if (e_ != cudaSuccess) return fail(c, FSPT_E_CUDA, "%s failed: %s", #call, cudaGetErrorString(e_)); \
+// CK_INTO: the message of a failed call goes to `dst` (stage_atlas reports into atlas_error: it runs on the atlas thread
+// while the caller may write c->error)
+#define CK_INTO(dst, call)                                                                  \
+  do {                                                                                      \
+    cudaError_t e_ = (call);                                                                \
+    if (e_ != cudaSuccess) {                                                                \
+      (dst) = std::string(#call) + " failed: " + cudaGetErrorString(e_);                    \
+      return FSPT_E_CUDA;                                                                   \
+    }                                                                                       \
   } while (0)
+#define CK(call) CK_INTO(c->error, call)
 
-template <class T>
-void dfree(T*& p) {
-  if (p) cudaFree(p);
-  p = nullptr;
-}
-
-void free_scene(Ctx* c) {
-  if (c->sc.atlas) cudaDestroyTextureObject(c->sc.atlas);
-  if (c->sc.env) cudaDestroyTextureObject(c->sc.env);
-  if (c->nodes_tex) cudaDestroyTextureObject(c->nodes_tex);
-  c->nodes_tex = 0;
-  if (c->sc.mat_tex) cudaDestroyTextureObject(c->sc.mat_tex);
-  if (c->mat_surf) cudaDestroySurfaceObject(c->mat_surf);
-  c->mat_surf = 0; c->mat_surface = false;
-  dfree(c->d_raw); dfree(c->d_mat_src); c->cap_raw = c->cap_mat_src = 0;
-  if (c->atlas_arr) cudaFreeArray(c->atlas_arr);
-  if (c->env_arr) cudaFreeArray(c->env_arr);
-  if (c->mat_arr) cudaFreeArray(c->mat_arr);
-  c->atlas_arr = c->env_arr = c->mat_arr = nullptr;
-  c->mat_R = c->mat_L = 0;
-  dfree(c->d_mat_info); c->cap_mat_info = 0;
-  c->atlas_R = c->atlas_L = c->env_W = c->env_H = 0;
-  dfree(c->d_nodes); dfree(c->d_tris); dfree(c->d_shade); dfree(c->d_bins); dfree(c->d_layer_info);
-  c->cap_nodes = c->cap_tris = c->cap_shade = c->cap_bins = c->cap_layer_info = 0;
-  if (c->h_stage) cudaFreeHost(c->h_stage);
-  c->h_stage = nullptr; c->stage_bytes = 0;
-  if (c->h_geo) cudaFreeHost(c->h_geo);
-  c->h_geo = nullptr; c->geo_stage_bytes = 0;
-  c->sc = DeviceScene{};
-  c->has_scene = false;
-}
-
-// device buffer that is only re-allocated when it has to grow
-int ensure(Ctx* c, void*& p, size_t& cap, size_t bytes) {
-  if (p && cap >= bytes) return FSPT_OK;
-  if (p) cudaFree(p);
-  p = nullptr; cap = 0;
-  CK(cudaMalloc(&p, bytes));
-  cap = bytes;
+// A device array of 16-byte words as a linear texture (tex1Dfetch): the second L1 data path next to the LSU.  Arrays
+// beyond the 2^27-texel limit get no texture (0) and are read with plain loads.
+int linear_tex(Ctx* c, cudaTextureObject_t* tex, void* ptr, size_t bytes, bool allowed = true) {
+  if (*tex) cudaDestroyTextureObject(*tex);
+  *tex = 0;
+  if (!allowed || bytes / 16 > ((size_t)1 << 27) || bytes == 0) return FSPT_OK;
+  cudaResourceDesc r = {};
+  r.resType = cudaResourceTypeLinear;
+  r.res.linear.devPtr = ptr;
+  r.res.linear.desc = cudaCreateChannelDesc<float4>();
+  r.res.linear.sizeInBytes = bytes;
+  cudaTextureDesc t = {};
+  t.readMode = cudaReadModeElementType;
+  CK(cudaCreateTextureObject(tex, &r, &t, nullptr));
   return FSPT_OK;
+}
+
+// Storage for the scene `s` (reused when it fits): the geometry records, the bins and the environment array.
+int fit_scene(Ctx* c, const SceneInfo& s) {
+  CK(c->d_nodes.fit(s.bytes_nodes));
+  CK(c->d_tris.fit(s.bytes_tris));
+  CK(c->d_shade.fit(s.bytes_shade));
+  CK(c->d_bins.fit(s.bytes_bins));
+  CK(c->env.fit(cudaCreateChannelDesc<uchar4>(), s.env_w, s.env_h, 0, false));  // RGBA8 RGBE (main.js:170-180)
+  return FSPT_OK;
+}
+
+// Makes `s`, in the storage of fit_scene, the scene the kernels read (the atlas part: publish_atlas).
+int publish_scene(Ctx* c, const SceneInfo& s) {
+  // FSPT_NO_NODE_TEX: test knob for the LSU-only instantiation of k_trace
+  if (int rc = linear_tex(c, &c->nodes_tex, c->d_nodes.p, s.bytes_nodes, !getenv("FSPT_NO_NODE_TEX"))) return rc;
+  c->info = s;
+  DeviceScene& sc = c->sc;
+  sc.nodes = reinterpret_cast<const float4*>(c->d_nodes.p);
+  sc.tris = reinterpret_cast<const float4*>(c->d_tris.p);
+  sc.shade = reinterpret_cast<const float4*>(c->d_shade.p);
+  sc.bins = reinterpret_cast<const float4*>(c->d_bins.p);
+  sc.env = c->env.tex;
+  sc.root_ref = s.root_ref;
+  sc.n_tris = s.n_tris; sc.n_interior = s.n_interior;
+  sc.atlas_res = s.atlas_res; sc.atlas_layers = s.atlas_layers; sc.env_w = s.env_w; sc.env_h = s.env_h;
+  sc.n_bins = s.n_bins;
+  set_env_constants(sc);
+  return FSPT_OK;
+}
+
+// Makes one form of the atlas resident, `res` x `res` x `layers`, and frees the other: the material-interleaved array
+// (uint4 texels) or the plain RGBA8 one.
+cudaError_t fit_atlas(Ctx* c, bool interleaved, int res, int layers, bool surface) {
+  (interleaved ? c->atlas : c->mat).release();
+  return interleaved ? c->mat.fit(cudaCreateChannelDesc<uint4>(), res, res, layers, surface)
+                     : c->atlas.fit(cudaCreateChannelDesc<uchar4>(), res, res, layers, surface);
+}
+
+// Makes the resident atlas and its two tables the ones k_shade reads.
+void publish_atlas(Ctx* c, const AtlasInfo& a) {
+  c->atlas_info = a;
+  c->sc.mat_tex = c->mat.tex;
+  c->sc.atlas = c->atlas.tex;
+  c->sc.layer_info = c->d_layer_info.p;
+  c->sc.mat_info = c->d_mat_info.p;
 }
 
 int alloc_wave(Ctx* c) {
@@ -224,24 +326,26 @@ int alloc_wave(Ctx* c) {
   c->wave_paths = (size_t)S * c->n_pixels;
   const size_t W = c->wave_paths;
   for (int k = 0; k < 2; ++k) {
-    CK(cudaMalloc(&c->ps2[k].rec, W * 16 * FSPT_PATH_WORDS));
-    CK(cudaMalloc(&c->ps2[k].sh, W));
+    CK(c->d_rec[k].fit(W * 16 * FSPT_PATH_WORDS));
+    CK(c->d_sh[k].fit(W));
+    c->ps2[k].rec = c->d_rec[k].p;
+    c->ps2[k].sh = c->d_sh[k].p;
   }
   c->ps = c->ps2[0];
-  CK(cudaMalloc(&c->d_shadow, W * 32));
-  CK(cudaMalloc(&c->d_counts, 64 * sizeof(int)));  // [0..3] the two count pairs; [32] the fetch cursor, on its own 128-byte
-                                                   // line: every warp's atomicAdd hits it, nothing else should
-  CK(cudaMemset(c->d_counts, 0, 64 * sizeof(int)));
-  CK(cudaMalloc(&c->d_count_out, W * sizeof(int)));
-  CK(cudaMalloc(&c->d_hit_flag, W));
-  CK(cudaMalloc(&c->d_stats, 8 * sizeof(unsigned long long)));  // [0..3] live, [4..7] snapshot at render start
-  CK(cudaMemset(c->d_stats, 0, 8 * sizeof(unsigned long long)));
-  CK(cudaMalloc(&c->d_sample_color, W * 16));
+  CK(c->d_shadow.fit(W * 32));
+  CK(c->d_counts.fit(64 * sizeof(int)));  // [0..3] the two count pairs; [32] the fetch cursor, on its own 128-byte
+                                          // line: every warp's atomicAdd hits it, nothing else should
+  CK(cudaMemset(c->d_counts.p, 0, 64 * sizeof(int)));
+  CK(c->d_count_out.fit(W * sizeof(int)));
+  CK(c->d_hit_flag.fit(W));
+  CK(c->d_stats.fit(8 * sizeof(unsigned long long)));  // [0..3] live, [4..7] snapshot at render start
+  CK(cudaMemset(c->d_stats.p, 0, 8 * sizeof(unsigned long long)));
+  CK(c->d_sample_color.fit(W * 16));
   c->rb_cap = 64;
-  CK(cudaMalloc(&c->d_rb, 2 * (size_t)c->rb_cap * sizeof(float)));
-  CK(cudaMallocHost(&c->h_rb, Ctx::RB_SLOTS * 2 * (size_t)c->rb_cap * sizeof(float)));
+  CK(c->d_rb.fit(2 * (size_t)c->rb_cap * sizeof(float)));
+  CK(c->h_rb.fit(Ctx::RB_SLOTS * 2 * (size_t)c->rb_cap * sizeof(float)));
   for (auto& e : c->ev_rb) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-  CK(cudaMallocHost(&c->h_poll, Ctx::POLL_SLOTS * sizeof(int)));
+  CK(c->h_poll.fit(Ctx::POLL_SLOTS * sizeof(int)));
   for (auto& e : c->ev_poll) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   return FSPT_OK;
 }
@@ -309,7 +413,7 @@ int atlas_join(Ctx* c) {
   if (c->atlas_thread.joinable()) c->atlas_thread.join();
   const int rc = c->atlas_rc;
   c->atlas_rc = FSPT_OK;
-  if (rc) { c->has_scene = false; c->error = c->atlas_error; }
+  if (rc) { c->has_scene = false; c->error = "atlas upload: " + c->atlas_error; }
   return rc;
 }
 
@@ -351,17 +455,7 @@ inline void scan_layer_band(const uint8_t* atlas, size_t layer_texels, int item,
 }
 
 int stage_atlas(Ctx* c, const AtlasJob& J) {
-  auto afail = [&](int code, const char* what, cudaError_t e) {
-    char buf[256];
-    snprintf(buf, sizeof buf, "atlas upload: %s failed: %s", what, cudaGetErrorString(e));
-    c->atlas_error = buf;
-    return code;
-  };
-#define ACK(call)                                                         \
-  do {                                                                    \
-    cudaError_t e_ = (call);                                              \
-    if (e_ != cudaSuccess) return afail(FSPT_E_CUDA, #call, e_);          \
-  } while (0)
+  std::string& err = c->atlas_error;
   auto t_prev = std::chrono::steady_clock::now();
   auto lap = [&](const char* what) {
     if (!J.timing) return;
@@ -399,36 +493,27 @@ int stage_atlas(Ctx* c, const AtlasJob& J) {
   // pinned staging; quadruples can outnumber layers, so it is bounded against the plain atlas (4 x its bytes, at least
   // 256 MB) and against the free device memory, and any allocation failure falls back to the plain RGBA8 array.
   bool use_mat_tex = !getenv("FSPT_PLAIN_ATLAS");
+  const int ML = std::max(1, n_tex_mats);  // layers of the interleaved array
   {
     const size_t inter = (size_t)n_tex_mats * layer_texels * 16, plain = (size_t)L * layer_bytes;
     // the array of the previous upload is reused when it has the same shape: then nothing is allocated and the driver is
     // not asked for the free memory (cudaMemGetInfo is a resource-manager call: usually 0.1 ms, but 20-100 ms every few
     // dozen calls on the virtualised hosts measured, which showed up as spikes in the end-to-end step time)
-    const bool reuse = c->mat_arr && c->mat_R == R && c->mat_L == std::max(1, n_tex_mats);
+    const TexArray& mat = c->mat;
+    const bool reuse = mat.arr && mat.w == R && mat.layers == ML;
     size_t free_b = (size_t)48 << 30, total_b = 0;
     if (!reuse && cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { (void)cudaGetLastError(); free_b = (size_t)48 << 30; }
-    const size_t resident = c->mat_arr ? (size_t)c->mat_R * c->mat_R * 16 * (size_t)c->mat_L : 0;  // freed before the new one
+    const size_t resident = (size_t)mat.w * mat.h * 16 * (size_t)mat.layers;  // freed before the new one
     if (inter > std::max<size_t>(4 * plain, (size_t)256 << 20) || inter > ((size_t)48 << 30) ||
         (!reuse && inter > (free_b + resident) / 2))
       use_mat_tex = false;
     if (getenv("FSPT_FORCE_MAT_TEX")) use_mat_tex = true;  // test knob: exercise the allocation-failure fallback
   }
   lap("tables + sizing");
-  cudaChannelFormatDesc fmt = cudaCreateChannelDesc<uchar4>();
-  cudaResourceDesc rd = {};
-  rd.resType = cudaResourceTypeArray;
-  cudaTextureDesc td = {};
-  td.addressMode[0] = td.addressMode[1] = td.addressMode[2] = cudaAddressModeClamp;
-  td.filterMode = cudaFilterModePoint;
-  td.readMode = cudaReadModeElementType;
-  td.normalizedCoords = 0;
   std::atomic<int> cuda_err(0);
   std::mutex mu;  // serialises the enqueues of the staging items
   bool plain_atlas = !use_mat_tex;
   if (use_mat_tex) {
-    if (c->sc.atlas) { cudaDestroyTextureObject(c->sc.atlas); c->sc.atlas = 0; }
-    if (c->atlas_arr) { cudaFreeArray(c->atlas_arr); c->atlas_arr = nullptr; c->atlas_R = c->atlas_L = 0; }
-    const int ML = std::max(1, n_tex_mats);
     // Where the interleave runs.  On the host (default): the 16-byte texels are built in pinned memory and DMA'd.  On the
     // GPU: only the DISTINCT varying layers cross PCIe as raw RGBA8 and k_interleave_atlas builds the texels through a
     // surface -- a material with one image map and three colours then costs 1 layer of staging and DMA instead of 4.
@@ -455,61 +540,27 @@ int stage_atlas(Ctx* c, const AtlasJob& J) {
     // wire format of the staged GPU path: RGB, 3 bytes per texel (the shaders never read alpha, tracer.fs:453-456); the
     // direct path copies the RGBA8 layers as they lie
     const size_t wire_layer_bytes = direct ? layer_bytes : layer_texels * 3;
-    if (!c->mat_arr || c->mat_R != R || c->mat_L != ML || c->mat_surface != gpu_interleave) {
-      if (c->sc.mat_tex) cudaDestroyTextureObject(c->sc.mat_tex);
-      c->sc.mat_tex = 0;
-      if (c->mat_surf) cudaDestroySurfaceObject(c->mat_surf);
-      c->mat_surf = 0;
-      if (c->mat_arr) cudaFreeArray(c->mat_arr);
-      c->mat_arr = nullptr;
-      cudaChannelFormatDesc fmt4 = cudaCreateChannelDesc<uint4>();
-      c->mat_R = c->mat_L = 0;
-      const size_t max_ml = getenv("FSPT_FORCE_MAT_TEX") ? (size_t)atoi(getenv("FSPT_FORCE_MAT_TEX")) : (size_t)1 << 30;
-      if ((size_t)ML > max_ml ||  // (test knob: pretend the device cannot hold more than that many material layers)
-          cudaMalloc3DArray(&c->mat_arr, &fmt4, make_cudaExtent(R, R, ML),
-                            cudaArrayLayered | (gpu_interleave ? cudaArraySurfaceLoadStore : 0)) != cudaSuccess) {
-        (void)cudaGetLastError();
-        c->mat_arr = nullptr;
-        plain_atlas = true;
-      } else {
-        rd.res.array.array = c->mat_arr;
-        ACK(cudaCreateTextureObject(&c->sc.mat_tex, &rd, &td, nullptr));
-        if (gpu_interleave) ACK(cudaCreateSurfaceObject(&c->mat_surf, &rd));
-        c->mat_R = R; c->mat_L = ML; c->mat_surface = gpu_interleave;
-      }
+    const size_t max_ml = getenv("FSPT_FORCE_MAT_TEX") ? (size_t)atoi(getenv("FSPT_FORCE_MAT_TEX")) : (size_t)1 << 30;
+    if ((size_t)ML > max_ml ||  // (test knob: pretend the device cannot hold more than that many material layers)
+        fit_atlas(c, true, R, ML, gpu_interleave) != cudaSuccess) {
+      (void)cudaGetLastError();
+      plain_atlas = true;
     }
     const size_t need = gpu_interleave ? wire_layer_bytes * raw_layers.size() : layer_texels * 16 * (size_t)ML;
-    if (!plain_atlas && !direct && c->stage_bytes < need) {
-      if (c->h_stage) cudaFreeHost(c->h_stage);
-      c->h_stage = nullptr; c->stage_bytes = 0;
-      if (cudaMallocHost(&c->h_stage, need) != cudaSuccess) {
-        (void)cudaGetLastError();
-        c->h_stage = nullptr;
-        plain_atlas = true;
-      } else {
-        c->stage_bytes = need;
-      }
+    if (!plain_atlas && !direct && c->h_stage.fit(need) != cudaSuccess) {
+      (void)cudaGetLastError();
+      plain_atlas = true;
     }
     lap("arrays + pinned block");
     if (plain_atlas) {
       // could not hold the interleaved atlas: every material becomes "plain" (the tables are not consulted by k_shade<false>)
     } else if (gpu_interleave) {
-      if (!(c->d_raw && c->cap_raw >= need)) {
-        if (c->d_raw) cudaFree(c->d_raw);
-        c->d_raw = nullptr; c->cap_raw = 0;
-        ACK(cudaMalloc(&c->d_raw, need));
-        c->cap_raw = need;
-      }
-      if (!(c->d_mat_src && c->cap_mat_src >= sizeof(MatSrc) * (size_t)ML)) {
-        if (c->d_mat_src) cudaFree(c->d_mat_src);
-        c->d_mat_src = nullptr; c->cap_mat_src = 0;
-        ACK(cudaMalloc(&c->d_mat_src, sizeof(MatSrc) * (size_t)ML));
-        c->cap_mat_src = sizeof(MatSrc) * (size_t)ML;
-      }
+      CK_INTO(err, c->d_raw.fit(need));
+      CK_INTO(err, c->d_mat_src.fit(sizeof(MatSrc) * (size_t)ML));
       if (direct) {
         for (size_t ri = 0; ri < raw_layers.size(); ++ri)
-          ACK(cudaMemcpyAsync(reinterpret_cast<uint8_t*>(c->d_raw) + ri * layer_bytes, J.atlas + (size_t)raw_layers[ri] * layer_bytes,
-                              layer_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+          CK_INTO(err, cudaMemcpyAsync(c->d_raw.p + ri * layer_bytes, J.atlas + (size_t)raw_layers[ri] * layer_bytes,
+                                       layer_bytes, cudaMemcpyHostToDevice, c->copy_stream));
       }
       // work item = (raw layer, band of rows): drop the alpha channel into the pinned block, DMA the band
       const int bands = std::max(1, std::min(R, 16));
@@ -518,7 +569,7 @@ int stage_atlas(Ctx* c, const AtlasJob& J) {
         const size_t y0 = (size_t)R * band / bands, y1 = (size_t)R * (band + 1) / bands;
         const size_t off = (size_t)ri * wire_layer_bytes + y0 * R * 3, bytes = (y1 - y0) * R * 3;
         const uint8_t* src = J.atlas + (size_t)raw_layers[ri] * layer_bytes + y0 * R * 4;
-        uint8_t* dst = c->h_stage + off;
+        uint8_t* dst = c->h_stage.p + off;
         const size_t n = (y1 - y0) * R;
         size_t i = 0;
 #if defined(__SSSE3__)
@@ -530,19 +581,19 @@ int stage_atlas(Ctx* c, const AtlasJob& J) {
 #endif
         for (; i < n; ++i) { dst[3 * i] = src[4 * i]; dst[3 * i + 1] = src[4 * i + 1]; dst[3 * i + 2] = src[4 * i + 2]; }
         std::lock_guard<std::mutex> g(mu);
-        cudaError_t e = cudaMemcpyAsync(reinterpret_cast<uint8_t*>(c->d_raw) + off, c->h_stage + off, bytes, cudaMemcpyHostToDevice, c->copy_stream);
+        cudaError_t e = cudaMemcpyAsync(c->d_raw.p + off, c->h_stage.p + off, bytes, cudaMemcpyHostToDevice, c->copy_stream);
         if (e != cudaSuccess) cuda_err.store((int)e);
       });
-      ACK(cudaMemcpyAsync(c->d_mat_src, mat_src, sizeof(MatSrc) * (size_t)n_tex_mats, cudaMemcpyHostToDevice, c->copy_stream));
+      CK_INTO(err, cudaMemcpyAsync(c->d_mat_src.p, mat_src, sizeof(MatSrc) * (size_t)n_tex_mats, cudaMemcpyHostToDevice, c->copy_stream));
       const dim3 blk(32, 8), grd((R + 31) / 32, (R + 7) / 8, n_tex_mats);
       if (!direct)
-        k_interleave_atlas<true><<<grd, blk, 0, c->copy_stream>>>(c->mat_surf, reinterpret_cast<const uint8_t*>(c->d_raw),
-                                                                  reinterpret_cast<const MatSrc*>(c->d_mat_src), R, layer_texels);
+        k_interleave_atlas<true><<<grd, blk, 0, c->copy_stream>>>(c->mat.surf, c->d_raw.p,
+                                                                  reinterpret_cast<const MatSrc*>(c->d_mat_src.p), R, layer_texels);
       else
-        k_interleave_atlas<false><<<grd, blk, 0, c->copy_stream>>>(c->mat_surf, reinterpret_cast<const uint8_t*>(c->d_raw),
-                                                                   reinterpret_cast<const MatSrc*>(c->d_mat_src), R, layer_texels);
+        k_interleave_atlas<false><<<grd, blk, 0, c->copy_stream>>>(c->mat.surf, c->d_raw.p,
+                                                                   reinterpret_cast<const MatSrc*>(c->d_mat_src.p), R, layer_texels);
       c->atlas_launches.fetch_add(1);
-      ACK(cudaGetLastError());
+      CK_INTO(err, cudaGetLastError());
     } else {
       // work item = (textured material, band of rows): interleave the four source layers, DMA the band
       const int bands = std::max(1, std::min(R, 16));
@@ -554,7 +605,7 @@ int stage_atlas(Ctx* c, const AtlasJob& J) {
         const int y0 = (int)((long long)R * band / bands), y1 = (int)((long long)R * (band + 1) / bands);
         const uint32_t* src[4];
         for (int k = 0; k < 4; ++k) src[k] = reinterpret_cast<const uint32_t*>(J.atlas) + (size_t)mats[m][k] * layer_texels;
-        uint32_t* dst = reinterpret_cast<uint32_t*>(c->h_stage) + ((size_t)tl * layer_texels + (size_t)y0 * R) * 4;
+        uint32_t* dst = reinterpret_cast<uint32_t*>(c->h_stage.p) + ((size_t)tl * layer_texels + (size_t)y0 * R) * 4;
         const size_t i0 = (size_t)y0 * R, n = (size_t)(y1 - y0) * R;
         size_t i = 0;
 #if defined(__SSE2__)
@@ -581,7 +632,7 @@ int stage_atlas(Ctx* c, const AtlasJob& J) {
         }
         cudaMemcpy3DParms cp = {};
         cp.srcPtr = make_cudaPitchedPtr(dst, (size_t)R * 16, R, y1 - y0);
-        cp.dstArray = c->mat_arr;
+        cp.dstArray = c->mat.arr;
         cp.dstPos = make_cudaPos(0, y0, tl);
         cp.extent = make_cudaExtent(R, y1 - y0, 1);
         cp.kind = cudaMemcpyHostToDevice;
@@ -592,32 +643,14 @@ int stage_atlas(Ctx* c, const AtlasJob& J) {
     }
   }
   if (plain_atlas) {
-    if (c->sc.mat_tex) { cudaDestroyTextureObject(c->sc.mat_tex); c->sc.mat_tex = 0; }
-    if (c->mat_surf) { cudaDestroySurfaceObject(c->mat_surf); c->mat_surf = 0; }
-    c->mat_surface = false;
-    if (c->mat_arr) { cudaFreeArray(c->mat_arr); c->mat_arr = nullptr; c->mat_R = c->mat_L = 0; }
-    if (!c->atlas_arr || c->atlas_R != R || c->atlas_L != L) {
-      if (c->sc.atlas) cudaDestroyTextureObject(c->sc.atlas);
-      c->sc.atlas = 0;
-      if (c->atlas_arr) cudaFreeArray(c->atlas_arr);
-      c->atlas_arr = nullptr;
-      ACK(cudaMalloc3DArray(&c->atlas_arr, &fmt, make_cudaExtent(R, R, L), cudaArrayLayered));
-      rd.res.array.array = c->atlas_arr;
-      ACK(cudaCreateTextureObject(&c->sc.atlas, &rd, &td, nullptr));
-      c->atlas_R = R; c->atlas_L = L;
-    }
-    if (c->stage_bytes < layer_bytes * L) {
-      if (c->h_stage) cudaFreeHost(c->h_stage);
-      c->h_stage = nullptr; c->stage_bytes = 0;
-      ACK(cudaMallocHost(&c->h_stage, layer_bytes * L));
-      c->stage_bytes = layer_bytes * L;
-    }
+    CK_INTO(err, fit_atlas(c, false, R, L, false));
+    CK_INTO(err, c->h_stage.fit(layer_bytes * L));
     pool.run(L, J.workers, [&](int l) {
-      uint8_t* dst = c->h_stage + (size_t)l * layer_bytes;
+      uint8_t* dst = c->h_stage.p + (size_t)l * layer_bytes;
       memcpy(dst, J.atlas + (size_t)l * layer_bytes, layer_bytes);
       cudaMemcpy3DParms cp = {};
       cp.srcPtr = make_cudaPitchedPtr(dst, (size_t)R * 4, R, R);
-      cp.dstArray = c->atlas_arr;
+      cp.dstArray = c->atlas.arr;
       cp.dstPos = make_cudaPos(0, 0, l);
       cp.extent = make_cudaExtent(R, R, 1);
       cp.kind = cudaMemcpyHostToDevice;
@@ -626,43 +659,19 @@ int stage_atlas(Ctx* c, const AtlasJob& J) {
       if (e != cudaSuccess) cuda_err.store((int)e);
     });
   }
-  if (cuda_err.load()) return afail(FSPT_E_CUDA, "a staging copy", (cudaError_t)cuda_err.load());
+  if (cuda_err.load()) {
+    err = std::string("a staging copy failed: ") + cudaGetErrorString((cudaError_t)cuda_err.load());
+    return FSPT_E_CUDA;
+  }
   lap("stage + enqueue");
   // the two small tables k_shade reads next to the texels: same stream, so the same event covers them
-  auto grow = [&](void*& p, size_t& cap, size_t bytes) -> cudaError_t {
-    if (p && cap >= bytes) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr; cap = 0;
-    cudaError_t e = cudaMalloc(&p, bytes);
-    if (e == cudaSuccess) cap = bytes;
-    return e;
-  };
-  ACK(grow(c->d_layer_info, c->cap_layer_info, (size_t)L * 8));
-  ACK(grow(c->d_mat_info, c->cap_mat_info, J.n_mat_info * 4));
-  ACK(cudaMemcpyAsync(c->d_layer_info, layer_info, (size_t)L * 8, cudaMemcpyHostToDevice, c->copy_stream));
-  ACK(cudaMemcpyAsync(c->d_mat_info, mat_info, J.n_mat_info * 4, cudaMemcpyHostToDevice, c->copy_stream));
-  c->sc.layer_info = reinterpret_cast<const uint2*>(c->d_layer_info);
-  c->sc.mat_info = reinterpret_cast<const int4*>(c->d_mat_info);
-  c->bytes_layer_info = (size_t)L * 8; c->bytes_mat_info = J.n_mat_info * 4;
-  ACK(cudaEventRecord(c->ev_atlas, c->copy_stream));
-  return FSPT_OK;
-#undef ACK
-}
-
-// A device array of 16-byte words as a linear texture (tex1Dfetch): the second L1 data path next to the LSU.  Arrays
-// beyond the 2^27-texel limit get no texture (0) and are read with plain loads.
-int linear_tex(Ctx* c, cudaTextureObject_t* tex, void* ptr, size_t bytes, bool allowed = true) {
-  if (*tex) cudaDestroyTextureObject(*tex);
-  *tex = 0;
-  if (!allowed || bytes / 16 > ((size_t)1 << 27) || bytes == 0) return FSPT_OK;
-  cudaResourceDesc r = {};
-  r.resType = cudaResourceTypeLinear;
-  r.res.linear.devPtr = ptr;
-  r.res.linear.desc = cudaCreateChannelDesc<float4>();
-  r.res.linear.sizeInBytes = bytes;
-  cudaTextureDesc t = {};
-  t.readMode = cudaReadModeElementType;
-  CK(cudaCreateTextureObject(tex, &r, &t, nullptr));
+  const AtlasInfo a = {(uint64_t)L * 8, J.n_mat_info * 4, !plain_atlas, R, plain_atlas ? L : ML};
+  CK_INTO(err, c->d_layer_info.fit(a.bytes_layer_info));
+  CK_INTO(err, c->d_mat_info.fit(a.bytes_mat_info));
+  CK_INTO(err, cudaMemcpyAsync(c->d_layer_info.p, layer_info, a.bytes_layer_info, cudaMemcpyHostToDevice, c->copy_stream));
+  CK_INTO(err, cudaMemcpyAsync(c->d_mat_info.p, mat_info, a.bytes_mat_info, cudaMemcpyHostToDevice, c->copy_stream));
+  publish_atlas(c, a);
+  CK_INTO(err, cudaEventRecord(c->ev_atlas, c->copy_stream));
   return FSPT_OK;
 }
 
@@ -677,12 +686,12 @@ int launch_trace(Ctx* c, int which, bool hit_flags, bool write_count, const Fram
   A.anyhit = c->anyhit;
   A.nodes = c->sc.nodes; A.tris = c->sc.tris; A.root_ref = c->sc.root_ref; A.nodes_tex = c->nodes_tex;
   A.ps = c->ps2[which];
-  A.shadow_rays = c->d_shadow;
-  A.counts = c->d_counts + 2 * which;
-  A.next = c->d_counts + 32;
-  A.stats = c->d_stats;
-  A.count_out = write_count ? c->d_count_out : nullptr;
-  A.hit_flag = hit_flags ? c->d_hit_flag : nullptr;
+  A.shadow_rays = c->d_shadow.p;
+  A.counts = c->d_counts.p + 2 * which;
+  A.next = c->d_counts.p + 32;
+  A.stats = c->d_stats.p;
+  A.count_out = write_count ? c->d_count_out.p : nullptr;
+  A.hit_flag = hit_flags ? c->d_hit_flag.p : nullptr;
   record_trace_begin(c, cam ? 2 : 0);  // tag 2: the camera-fused primary launch of a wave
   if (A.nodes_tex) {
     if (cam) k_trace<false, true, true><<<c->trace_blocks_cam, TRACE_THREADS, 0, c->stream>>>(A);
@@ -700,7 +709,7 @@ int launch_trace(Ctx* c, int which, bool hit_flags, bool write_count, const Fram
 }
 
 int set_counts(Ctx* c, int n_cont, int n_shadow) {  // also zeroes #hit, #miss and the fetch cursor
-  k_set_counts<<<1, 1, 0, c->stream>>>(c->d_counts, n_cont, n_shadow);
+  k_set_counts<<<1, 1, 0, c->stream>>>(c->d_counts.p, n_cont, n_shadow);
   CK(cudaGetLastError());
   return FSPT_OK;
 }
@@ -732,21 +741,18 @@ FrameParams make_frame(const Ctx* c, const fspt_frame_params* f, bool whole_fram
 int stage_rand_bases(Ctx* c, const float* cam, const float* trace, int n) {
   if (n > c->rb_cap) {  // grow (rare): everything in flight must finish first
     CK(cudaStreamSynchronize(c->stream));
-    dfree(c->d_rb);
-    if (c->h_rb) cudaFreeHost(c->h_rb);
-    c->h_rb = nullptr;
     c->rb_cap = std::max(n, 2 * c->rb_cap);
-    CK(cudaMalloc(&c->d_rb, 2 * (size_t)c->rb_cap * sizeof(float)));
-    CK(cudaMallocHost(&c->h_rb, Ctx::RB_SLOTS * 2 * (size_t)c->rb_cap * sizeof(float)));
+    CK(c->d_rb.fit(2 * (size_t)c->rb_cap * sizeof(float)));
+    CK(c->h_rb.fit(Ctx::RB_SLOTS * 2 * (size_t)c->rb_cap * sizeof(float)));
   }
   if (n <= 0) return FSPT_OK;
   const int slot = c->rb_slot;
   c->rb_slot = (slot + 1) % Ctx::RB_SLOTS;
   CK(cudaEventSynchronize(c->ev_rb[slot]));  // returns at once unless RB_SLOTS calls are still queued
-  float* h = c->h_rb + (size_t)slot * 2 * c->rb_cap;
+  float* h = c->h_rb.p + (size_t)slot * 2 * c->rb_cap;
   memcpy(h, cam, (size_t)n * sizeof(float));
   if (trace) memcpy(h + c->rb_cap, trace, (size_t)n * sizeof(float));
-  CK(cudaMemcpyAsync(c->d_rb, h, 2 * (size_t)c->rb_cap * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  CK(cudaMemcpyAsync(c->d_rb.p, h, 2 * (size_t)c->rb_cap * sizeof(float), cudaMemcpyHostToDevice, c->stream));
   CK(cudaEventRecord(c->ev_rb[slot], c->stream));
   return FSPT_OK;
 }
@@ -763,15 +769,15 @@ int render_wave(Ctx* c, const FrameParams& fp, uint32_t first_tick, int S, const
   ShadeArgs A;
   A.f = fp;
   A.rb_trace = rb_trace;
-  A.hit_flag = c->d_hit_flag;
-  A.shadow_rays_out = c->d_shadow;
-  A.sample_color = c->d_sample_color;
-  A.capped = c->d_stats + 3;
+  A.hit_flag = c->d_hit_flag.p;
+  A.shadow_rays_out = c->d_shadow.p;
+  A.sample_color = c->d_sample_color.p;
+  A.capped = c->d_stats.p + 3;
   A.n_samples = S;
   A.div_s = make_fastdiv((unsigned)S, c->wave_paths);
   A.max_refractions = c->max_refractions;
   A.anyhit = c->anyhit;
-  const int hard_cap = FSPT_NUM_BOUNCES + 1 + (c->has_dielectric ? c->max_refractions + 2 : 0);
+  const int hard_cap = FSPT_NUM_BOUNCES + 1 + (c->info.has_dielectric ? c->max_refractions + 2 : 0);
   // atlas of the last upload: an asynchronous upload's staging thread is joined HERE, with the primary traversal already
   // running on the GPU (the event it records has to exist before the stream can be made to wait on it); then the DMA
   // itself is waited for on the device (no-op once it has completed)
@@ -784,12 +790,12 @@ int render_wave(Ctx* c, const FrameParams& fp, uint32_t first_tick, int S, const
   int cur = 0;
   for (int b = 0; b < hard_cap; ++b) {
     const int nxt = cur ^ 1;
-    CK(cudaMemsetAsync(c->d_counts + 2 * nxt, 0, 2 * sizeof(int), c->stream));
+    CK(cudaMemsetAsync(c->d_counts.p + 2 * nxt, 0, 2 * sizeof(int), c->stream));
     A.first = (b == 0);
     A.ps = c->ps2[cur];
     A.ps_out = c->ps2[nxt];
-    A.counts_in = c->d_counts + 2 * cur;
-    A.counts_out = c->d_counts + 2 * nxt;
+    A.counts_in = c->d_counts.p + 2 * cur;
+    A.counts_out = c->d_counts.p + 2 * nxt;
     record_trace_begin(c, 1);
     if (c->sc.mat_tex) k_shade<true><<<c->shade_blocks, SHADE_THREADS, 1024, c->stream>>>(A);
     else k_shade<false><<<c->shade_blocks, SHADE_THREADS, 1024, c->stream>>>(A);
@@ -798,24 +804,24 @@ int render_wave(Ctx* c, const FrameParams& fp, uint32_t first_tick, int S, const
     CK(cudaGetLastError());
     cur = nxt;
     if (b >= FSPT_NUM_BOUNCES) {
-      if (!c->has_dielectric) break;  // every surviving path had i == NUM_BOUNCES: nothing was appended
+      if (!c->info.has_dielectric) break;  // every surviving path had i == NUM_BOUNCES: nothing was appended
       // Refractions do not count as bounces (`i--`, tracer.fs:488), so paths may survive.  The number of live paths is
       // copied out after every extra iteration, but the host reads the value of TWO iterations ago: the GPU always has
       // work queued and never waits for the host; at most two empty iterations (kernels that find zero items) are wasted.
       const int k = b % Ctx::POLL_SLOTS;
-      CK(cudaMemcpyAsync(c->h_poll + k, c->d_counts + 2 * cur, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+      CK(cudaMemcpyAsync(c->h_poll.p + k, c->d_counts.p + 2 * cur, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
       CK(cudaEventRecord(c->ev_poll[k], c->stream));
       if (b >= FSPT_NUM_BOUNCES + 2) {
         const int k2 = (b - 2) % Ctx::POLL_SLOTS;
         CK(cudaEventSynchronize(c->ev_poll[k2]));
-        if (c->h_poll[k2] == 0) break;
+        if (c->h_poll.p[k2] == 0) break;
       }
     }
-    CK(cudaMemsetAsync(c->d_counts + 32, 0, sizeof(int), c->stream));  // fetch cursor
+    CK(cudaMemsetAsync(c->d_counts.p + 32, 0, sizeof(int), c->stream));  // fetch cursor
     rc = launch_trace(c, cur, true, false);  // tracer.fs:501,507
     if (rc) return rc;
   }
-  k_accumulate<<<(P + 255) / 256, 256, 0, c->stream>>>(c->d_sample_color, c->d_fb, c->d_last_color, fp.rx0, fp.ry0, fp.rw,
+  k_accumulate<<<(P + 255) / 256, 256, 0, c->stream>>>(c->d_sample_color.p, c->d_fb.p, c->d_last_color.p, fp.rx0, fp.ry0, fp.rw,
                                                        fp.rh, fp.width, S, first_tick, c->accum_mode, c->sanitize);
   c->stats.kernel_launches++;
   CK(cudaGetLastError());
@@ -879,15 +885,14 @@ void comm_free(Ctx* c) {
 
 // what a receiving rank has to know before the buffers of fspt_scene_broadcast arrive
 struct SceneHeader {
-  uint64_t bytes_nodes, bytes_tris, bytes_shade, bytes_bins, bytes_layer_info, bytes_mat_info, scene_bytes;
-  int32_t root_ref, n_tris, n_interior, atlas_res, atlas_layers, env_w, env_h, n_bins;
-  int32_t mat_R, mat_L, use_mat_tex, has_dielectric, magic;
+  SceneInfo scene;
+  int32_t magic;
 };
 
 // what a receiving rank has to know before the atlas part of fspt_scene_broadcast arrives (phase 2)
 struct SceneHeader2 {
-  uint64_t bytes_layer_info, bytes_mat_info;
-  int32_t mat_R, mat_L, use_mat_tex, magic;
+  AtlasInfo atlas;
+  int32_t magic;
 };
 
 // The scene resident on `root` -> every other rank, device to device over NVLink: the records fspt_scene_upload built
@@ -909,7 +914,7 @@ int broadcast_phase2(Ctx* c) {
   SceneHeader2 h;
   memset(&h, 0, sizeof h);
   static_assert(sizeof(SceneHeader2) <= 128, "header buffer");
-  uint8_t* d_hdr2 = reinterpret_cast<uint8_t*>(c->d_hdr) + 256;
+  uint8_t* d_hdr2 = c->d_hdr.p + 256;
   // the collectives of one communicator run one after the other: this one starts behind phase 1 (its last collective
   // recorded the event), not behind the traversal launch that may have been enqueued since
   CK(cudaStreamWaitEvent(c->copy_stream, c->ev_bcast, 0));
@@ -917,10 +922,7 @@ int broadcast_phase2(Ctx* c) {
     int rcj = atlas_join(c);  // the root's atlas part ends here at the latest; its outcome travels in the header
     if (rcj) h.magic = -1;    // the ranks must not wait for an atlas that will not come
     else {
-      h.bytes_layer_info = c->bytes_layer_info; h.bytes_mat_info = c->bytes_mat_info;
-      h.use_mat_tex = c->sc.mat_tex ? 1 : 0;
-      h.mat_R = h.use_mat_tex ? c->mat_R : c->atlas_R;
-      h.mat_L = h.use_mat_tex ? c->mat_L : c->atlas_L;
+      h.atlas = c->atlas_info;
       h.magic = 0x46535032;
     }
     CK(cudaMemcpyAsync(d_hdr2, &h, sizeof h, cudaMemcpyHostToDevice, c->copy_stream));
@@ -932,76 +934,38 @@ int broadcast_phase2(Ctx* c) {
     CK(cudaStreamSynchronize(c->copy_stream));
     if (h.magic != 0x46535032) { c->has_scene = false; return fail(c, FSPT_E_NCCL, "fspt_scene_broadcast: rank %d has no atlas to send (its upload failed)", root); }
   }
-  const size_t texel = h.use_mat_tex ? 16 : 4;
-  const size_t atlas_bytes = (size_t)h.mat_R * h.mat_R * texel * (size_t)h.mat_L;
-  int rc;
-  if ((rc = ensure(c, c->d_lin, c->cap_lin, atlas_bytes))) return rc;
-  uint8_t* lin = reinterpret_cast<uint8_t*>(c->d_lin);
+  const AtlasInfo& a = h.atlas;
+  const size_t texel = a.interleaved ? 16 : 4;
+  const size_t atlas_bytes = (size_t)a.res * a.res * texel * (size_t)a.layers;
+  CK(c->d_lin.fit(atlas_bytes));
+  uint8_t* lin = c->d_lin.p;
   cudaMemcpy3DParms cp = {};
-  cp.extent = make_cudaExtent(h.mat_R, h.mat_R, h.mat_L);
+  cp.extent = make_cudaExtent(a.res, a.res, a.layers);
   cp.kind = cudaMemcpyDeviceToDevice;
   if (is_root) {
     // the atlas DMA of the upload runs on this same stream (in order)
-    cp.srcArray = h.use_mat_tex ? c->mat_arr : c->atlas_arr;
-    cp.dstPtr = make_cudaPitchedPtr(lin, (size_t)h.mat_R * texel, h.mat_R, h.mat_R);
+    cp.srcArray = (a.interleaved ? c->mat : c->atlas).arr;
+    cp.dstPtr = make_cudaPitchedPtr(lin, (size_t)a.res * texel, a.res, a.res);
     CK(cudaMemcpy3DAsync(&cp, c->copy_stream));
   } else {
     // storage on the receiving side: same reuse rules as fspt_scene_upload
-    if ((rc = ensure(c, c->d_layer_info, c->cap_layer_info, h.bytes_layer_info))) return rc;
-    if ((rc = ensure(c, c->d_mat_info, c->cap_mat_info, h.bytes_mat_info))) return rc;
-    cudaResourceDesc rd = {};
-    rd.resType = cudaResourceTypeArray;
-    cudaTextureDesc td = {};
-    td.addressMode[0] = td.addressMode[1] = td.addressMode[2] = cudaAddressModeClamp;
-    td.filterMode = cudaFilterModePoint;
-    td.readMode = cudaReadModeElementType;
-    cudaChannelFormatDesc fmt = cudaCreateChannelDesc<uchar4>();
-    if (h.use_mat_tex) {
-      if (c->sc.atlas) { cudaDestroyTextureObject(c->sc.atlas); c->sc.atlas = 0; }
-      if (c->atlas_arr) { cudaFreeArray(c->atlas_arr); c->atlas_arr = nullptr; c->atlas_R = c->atlas_L = 0; }
-      if (!c->mat_arr || c->mat_R != h.mat_R || c->mat_L != h.mat_L) {
-        if (c->sc.mat_tex) cudaDestroyTextureObject(c->sc.mat_tex);
-        c->sc.mat_tex = 0;
-        if (c->mat_surf) cudaDestroySurfaceObject(c->mat_surf);
-        c->mat_surf = 0; c->mat_surface = false;
-        if (c->mat_arr) cudaFreeArray(c->mat_arr);
-        c->mat_arr = nullptr;
-        cudaChannelFormatDesc fmt4 = cudaCreateChannelDesc<uint4>();
-        CK(cudaMalloc3DArray(&c->mat_arr, &fmt4, make_cudaExtent(h.mat_R, h.mat_R, h.mat_L), cudaArrayLayered));
-        rd.res.array.array = c->mat_arr;
-        CK(cudaCreateTextureObject(&c->sc.mat_tex, &rd, &td, nullptr));
-        c->mat_R = h.mat_R; c->mat_L = h.mat_L;
-      }
-    } else {
-      if (c->sc.mat_tex) { cudaDestroyTextureObject(c->sc.mat_tex); c->sc.mat_tex = 0; }
-      if (c->mat_surf) { cudaDestroySurfaceObject(c->mat_surf); c->mat_surf = 0; }
-      c->mat_surface = false;
-      if (c->mat_arr) { cudaFreeArray(c->mat_arr); c->mat_arr = nullptr; c->mat_R = c->mat_L = 0; }
-      if (!c->atlas_arr || c->atlas_R != h.mat_R || c->atlas_L != h.mat_L) {
-        if (c->sc.atlas) cudaDestroyTextureObject(c->sc.atlas);
-        c->sc.atlas = 0;
-        if (c->atlas_arr) cudaFreeArray(c->atlas_arr);
-        c->atlas_arr = nullptr;
-        CK(cudaMalloc3DArray(&c->atlas_arr, &fmt, make_cudaExtent(h.mat_R, h.mat_R, h.mat_L), cudaArrayLayered));
-        rd.res.array.array = c->atlas_arr;
-        CK(cudaCreateTextureObject(&c->sc.atlas, &rd, &td, nullptr));
-        c->atlas_R = h.mat_R; c->atlas_L = h.mat_L;
-      }
-    }
+    c->has_scene = false;
+    CK(c->d_layer_info.fit(a.bytes_layer_info));
+    CK(c->d_mat_info.fit(a.bytes_mat_info));
+    CK(fit_atlas(c, a.interleaved, a.res, a.layers, false));
   }
   NK(N->GroupStart());
-  NK(N->Broadcast(c->d_layer_info, c->d_layer_info, h.bytes_layer_info, ncclUint8, root, c->comm, c->copy_stream));
-  NK(N->Broadcast(c->d_mat_info, c->d_mat_info, h.bytes_mat_info, ncclUint8, root, c->comm, c->copy_stream));
+  NK(N->Broadcast(c->d_layer_info.p, c->d_layer_info.p, a.bytes_layer_info, ncclUint8, root, c->comm, c->copy_stream));
+  NK(N->Broadcast(c->d_mat_info.p, c->d_mat_info.p, a.bytes_mat_info, ncclUint8, root, c->comm, c->copy_stream));
   NK(N->Broadcast(lin, lin, atlas_bytes, ncclUint8, root, c->comm, c->copy_stream));
   NK(N->GroupEnd());
   c->stats.kernel_launches += 4;
   if (!is_root) {
-    cp.srcPtr = make_cudaPitchedPtr(lin, (size_t)h.mat_R * texel, h.mat_R, h.mat_R);
-    cp.dstArray = h.use_mat_tex ? c->mat_arr : c->atlas_arr;
+    cp.srcPtr = make_cudaPitchedPtr(lin, (size_t)a.res * texel, a.res, a.res);
+    cp.dstArray = (a.interleaved ? c->mat : c->atlas).arr;
     CK(cudaMemcpy3DAsync(&cp, c->copy_stream));
-    c->bytes_layer_info = h.bytes_layer_info; c->bytes_mat_info = h.bytes_mat_info;
-    c->sc.layer_info = reinterpret_cast<const uint2*>(c->d_layer_info);
-    c->sc.mat_info = reinterpret_cast<const int4*>(c->d_mat_info);
+    publish_atlas(c, a);
+    c->has_scene = true;
   }
   // what the first shading launch waits for; later collectives on the context's stream come behind it as well
   CK(cudaEventRecord(c->ev_atlas, c->copy_stream));
@@ -1011,7 +975,7 @@ int broadcast_phase2(Ctx* c) {
 
 int pull_stats(Ctx* c) {
   unsigned long long h[8];
-  CK(cudaMemcpy(h, c->d_stats, sizeof h, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(h, c->d_stats.p, sizeof h, cudaMemcpyDeviceToHost));
   c->stats.rays = h[0]; c->stats.node_visits = h[1]; c->stats.leaf_visits = h[2]; c->stats.capped_paths = h[3];
   c->stats.last_rays = h[0] - h[4]; c->stats.last_node_visits = h[1] - h[5]; c->stats.last_leaf_visits = h[2] - h[6];
   return FSPT_OK;
@@ -1040,28 +1004,27 @@ int fspt_create(fspt_ctx** out, int32_t width, int32_t height, int32_t device) {
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, device) != cudaSuccess || prop.major != 10)
     return fail(c, FSPT_E_CUDA, "device %d is sm_%d%d; kernels are built for sm_100a only", device, prop.major, prop.minor);
-  Ctx* ctx = new Ctx();
-  c = ctx;
+  c = new Ctx();
   c->device = device; c->sm_count = prop.multiProcessorCount;
   c->width = width; c->height = height; c->n_pixels = width * height;
   c->rx0 = c->ry0 = 0; c->rw = width; c->rh = height;
-  cudaError_t err;
-#define CKC(call) if ((err = (call)) != cudaSuccess) { g_create_error = std::string(#call) + ": " + cudaGetErrorString(err); delete ctx; return FSPT_E_CUDA; }
-  CKC(cudaSetDevice(device));
-  CKC(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-  CKC(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-  CKC(cudaEventCreateWithFlags(&c->ev_atlas, cudaEventDisableTiming));
-  CKC(cudaEventCreate(&c->ev_begin));
-  CKC(cudaEventCreate(&c->ev_end));
-  CKC(cudaMalloc(&c->d_fb, (size_t)c->n_pixels * 16));
-  CKC(cudaMemset(c->d_fb, 0, (size_t)c->n_pixels * 16));
-  CKC(cudaMalloc(&c->d_last_color, (size_t)c->n_pixels * 16));
-  CKC(cudaMalloc(&c->d_cam_pos, (size_t)c->n_pixels * 16));
-  CKC(cudaMalloc(&c->d_cam_dir, (size_t)c->n_pixels * 16));
-  CKC(cudaMalloc(&c->d_rgba8, (size_t)c->n_pixels * 4));
-#undef CKC
-  int rc = alloc_wave(c);
-  if (rc) { g_create_error = c->error; fspt_destroy(reinterpret_cast<fspt_ctx*>(c)); return rc; }
+  auto init = [c]() -> int {
+    const size_t px16 = (size_t)c->n_pixels * 16;
+    CK(cudaSetDevice(c->device));
+    CK(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
+    CK(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
+    CK(cudaEventCreateWithFlags(&c->ev_atlas, cudaEventDisableTiming));
+    CK(cudaEventCreate(&c->ev_begin));
+    CK(cudaEventCreate(&c->ev_end));
+    CK(c->d_fb.fit(px16));
+    CK(cudaMemset(c->d_fb.p, 0, px16));
+    CK(c->d_last_color.fit(px16));
+    CK(c->d_cam_pos.fit(px16));
+    CK(c->d_cam_dir.fit(px16));
+    CK(c->d_rgba8.fit((size_t)c->n_pixels * 4));
+    return alloc_wave(c);
+  };
+  if (int rc = init()) { g_create_error = c->error; fspt_destroy(reinterpret_cast<fspt_ctx*>(c)); return rc; }
   // persistent grids: resident CTAs per SM x SM count.  The traversal kernel keeps its short stacks and a few per-ray
   // values in shared memory; everything else of the unified array should stay L1 (BVH nodes and leaf blocks live
   // there), so the carveout is set to what the resident CTAs need and no more.
@@ -1103,22 +1066,13 @@ void fspt_destroy(fspt_ctx* ctx) {
   if (c->stream) cudaStreamSynchronize(c->stream);
   if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
   delete c->pool;
-  c->pool = nullptr;
-  if (c->h_ring) cudaFreeHost(c->h_ring);
+  linear_tex(c, &c->nodes_tex, nullptr, 0);  // (destroys it)
   for (auto e : c->ev_ring) cudaEventDestroy(e);
-  free_scene(c);
-  dfree(c->d_fb); dfree(c->d_last_color); dfree(c->d_sample_color); dfree(c->d_cam_pos); dfree(c->d_cam_dir); dfree(c->d_rgba8);
-  dfree(c->ps2[0].rec); dfree(c->ps2[1].rec); dfree(c->ps2[0].sh); dfree(c->ps2[1].sh);
-  dfree(c->d_shadow);
-  dfree(c->d_counts); dfree(c->d_count_out); dfree(c->d_hit_flag); dfree(c->d_stats); dfree(c->d_rb);
-  if (c->h_rb) cudaFreeHost(c->h_rb);
-  if (c->h_poll) cudaFreeHost(c->h_poll);
   for (auto e : c->ev_rb) if (e) cudaEventDestroy(e);
   for (auto e : c->ev_poll) if (e) cudaEventDestroy(e);
   comm_free(c);
   if (c->ev_red0) cudaEventDestroy(c->ev_red0);
   if (c->ev_red1) cudaEventDestroy(c->ev_red1);
-  dfree(c->d_lin); dfree(c->d_hdr); dfree(c->d_lin_env);
   if (c->ev_bcast) cudaEventDestroy(c->ev_bcast);
   if (c->ev_env) cudaEventDestroy(c->ev_env);
   for (auto e : c->ev_trace) cudaEventDestroy(e);
@@ -1127,7 +1081,7 @@ void fspt_destroy(fspt_ctx* ctx) {
   if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
   if (c->ev_atlas) cudaEventDestroy(c->ev_atlas);
   if (c->stream) cudaStreamDestroy(c->stream);
-  delete c;
+  delete c;  // frees the buffers and arrays
 }
 
 // fspt_scene_upload / fspt_scene_upload_async.
@@ -1178,9 +1132,7 @@ static int scene_upload_impl(fspt_ctx* ctx, const fspt_scene_desc* s, bool async
     const int rcp = scene_prepass(pool, hw, s, pre);
     if (rcp) return fail(c, rcp, "%s", pre.error.c_str());
   }
-  const std::vector<int32_t>& ref = pre.ref;
   std::vector<std::array<int, 4>>& mats = pre.mats;
-  const bool dielectric = pre.dielectric;
   const size_t NI = pre.NI();
   lap("node + material pre-pass");
 
@@ -1190,41 +1142,25 @@ static int scene_upload_impl(fspt_ctx* ctx, const fspt_scene_desc* s, bool async
   const size_t o_bins = 0, o_layer = o_bins + al((size_t)s->env_bins * 16), o_mat = o_layer + al((size_t)L * 8),
                o_matsrc = o_mat + al(std::max<size_t>(32, mats.size() * 32)),
                o_env = o_matsrc + al(std::max<size_t>(32, mats.size() * sizeof(MatSrc))), small_bytes = o_env + al(env_bytes);
-  if (c->geo_stage_bytes < small_bytes) {
-    if (c->h_geo) cudaFreeHost(c->h_geo);
-    c->h_geo = nullptr; c->geo_stage_bytes = 0;
-    CK(cudaMallocHost(&c->h_geo, small_bytes));
-    c->geo_stage_bytes = small_bytes;
-  }
-  uint8_t* hg = c->h_geo;
+  CK(c->h_geo.fit(small_bytes));
+  uint8_t* hg = c->h_geo.p;
   float* bins = reinterpret_cast<float*>(hg + o_bins);
   const size_t n_mat_info = std::max<size_t>(8, mats.size() * 8);
   // ---- device buffers, environment array
+  SceneInfo si;
+  si.bytes_nodes = std::max<size_t>(NI, 1) * 64;
+  si.bytes_tris = (size_t)(T + 3) * 48;
+  si.bytes_shade = (size_t)T * 192;
+  si.bytes_bins = (size_t)s->env_bins * 16;
+  si.scene_bytes = (size_t)N * 36 + (size_t)T * (36 + 48 + 108 + 24) + (size_t)s->atlas_res * s->atlas_res * 4 * L +
+                   env_bytes + (size_t)s->env_bins * 8;
+  si.root_ref = pre.ref[0];
+  si.n_tris = T; si.n_interior = (int)NI;
+  si.atlas_res = s->atlas_res; si.atlas_layers = L; si.env_w = s->env_width; si.env_h = s->env_height;
+  si.n_bins = s->env_bins;
+  si.has_dielectric = pre.dielectric;
   int rc_;
-  const size_t nodes_bytes = std::max<size_t>(NI, 1) * 64, tris_bytes = (size_t)(T + 3) * 48, shade_bytes = (size_t)T * 192,
-               bins_bytes = (size_t)s->env_bins * 16;
-  if ((rc_ = ensure(c, c->d_nodes, c->cap_nodes, nodes_bytes))) return rc_;
-  if ((rc_ = ensure(c, c->d_tris, c->cap_tris, tris_bytes))) return rc_;
-  if ((rc_ = ensure(c, c->d_shade, c->cap_shade, shade_bytes))) return rc_;
-  if ((rc_ = ensure(c, c->d_bins, c->cap_bins, bins_bytes))) return rc_;
-  if (!c->env_arr || c->env_W != s->env_width || c->env_H != s->env_height) {  // 2D array, RGBA8 RGBE (main.js:170-180)
-    cudaChannelFormatDesc fmt = cudaCreateChannelDesc<uchar4>();
-    cudaResourceDesc rd = {};
-    rd.resType = cudaResourceTypeArray;
-    cudaTextureDesc td = {};
-    td.addressMode[0] = td.addressMode[1] = td.addressMode[2] = cudaAddressModeClamp;
-    td.filterMode = cudaFilterModePoint;
-    td.readMode = cudaReadModeElementType;
-    td.normalizedCoords = 0;
-    if (c->sc.env) cudaDestroyTextureObject(c->sc.env);
-    c->sc.env = 0;
-    if (c->env_arr) cudaFreeArray(c->env_arr);
-    c->env_arr = nullptr;
-    CK(cudaMallocArray(&c->env_arr, &fmt, s->env_width, s->env_height));
-    rd.res.array.array = c->env_arr;
-    CK(cudaCreateTextureObject(&c->sc.env, &rd, &td, nullptr));
-    c->env_W = s->env_width; c->env_H = s->env_height;
-  }
+  if ((rc_ = fit_scene(c, si))) return rc_;
   // ---- work items of the staging region: bands of the environment (+ the bins), node chunks, triangle chunks -- each
   // DMA'd the moment it is complete -- and, behind them, the constant-layer scan of the atlas, which the workers that
   // run out of geometry pick up.  Chunks are sized so that a small scene still gives every worker a few items; each
@@ -1249,12 +1185,7 @@ static int scene_upload_impl(fspt_ctx* ctx, const fspt_scene_desc* s, bool async
   int n_slots = (int)std::max<size_t>(1, std::min<size_t>((size_t)n_geo_items, std::max<size_t>(2 * (size_t)workers, ((size_t)256 << 20) / slot_bytes)));
   if (const char* e = getenv("FSPT_RING_SLOTS")) n_slots = std::max(1, std::min(n_slots, atoi(e)));  // test knob: force slot reuse
   const bool ring_wraps = n_geo_items > n_slots;  // otherwise every chunk has a slot of its own and no event is needed
-  if (c->ring_bytes < slot_bytes * (size_t)n_slots) {
-    if (c->h_ring) cudaFreeHost(c->h_ring);
-    c->h_ring = nullptr; c->ring_bytes = 0;
-    CK(cudaMallocHost(&c->h_ring, slot_bytes * (size_t)n_slots));
-    c->ring_bytes = slot_bytes * (size_t)n_slots;
-  }
+  CK(c->h_ring.fit(slot_bytes * (size_t)n_slots));
   while ((int)c->ev_ring.size() < n_slots) {
     cudaEvent_t e;
     CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -1282,9 +1213,9 @@ static int scene_upload_impl(fspt_ctx* ctx, const fspt_scene_desc* s, bool async
       const int y0 = (int)((long long)s->env_height * item / n_env_items), y1 = (int)((long long)s->env_height * (item + 1) / n_env_items);
       const uint8_t* src = s->env + y0 * pitch;   // page-locked by the caller (fspt_host_register): DMA'd where it lies
       if (!src_env_pinned) { memcpy(hg + o_env + y0 * pitch, src, (size_t)(y1 - y0) * pitch); src = hg + o_env + y0 * pitch; }
-      cudaError_t e = item == 0 ? cudaMemcpyAsync(c->d_bins, bins, bins_bytes, cudaMemcpyHostToDevice, c->stream) : cudaSuccess;
+      cudaError_t e = item == 0 ? cudaMemcpyAsync(c->d_bins.p, bins, si.bytes_bins, cudaMemcpyHostToDevice, c->stream) : cudaSuccess;
       if (e == cudaSuccess)
-        e = cudaMemcpy2DToArrayAsync(c->env_arr, 0, y0, src, pitch, pitch, y1 - y0, cudaMemcpyHostToDevice, c->stream);
+        e = cudaMemcpy2DToArrayAsync(c->env.arr, 0, y0, src, pitch, pitch, y1 - y0, cudaMemcpyHostToDevice, c->stream);
       if (e != cudaSuccess) dma_err.store((int)e);
       return;
     }
@@ -1298,7 +1229,7 @@ static int scene_upload_impl(fspt_ctx* ctx, const fspt_scene_desc* s, bool async
       while (slot_done[slot].load(std::memory_order_acquire) != ring_item - n_slots) std::this_thread::yield();
       cudaEventSynchronize(c->ev_ring[slot]);
     }
-    uint8_t* hs = c->h_ring + (size_t)slot * slot_bytes;
+    uint8_t* hs = c->h_ring.p + (size_t)slot * slot_bytes;
     cudaError_t e = cudaSuccess;
     if (ring_item < n_node_items) {
       const size_t k0 = (size_t)ring_item * node_chunk, k1 = std::min(NI, k0 + node_chunk);
@@ -1307,16 +1238,16 @@ static int scene_upload_impl(fspt_ctx* ctx, const fspt_scene_desc* s, bool async
       const int bad = pack_node_chunk(s, pre, k0, k1, nodes, &bl, &br);
       if (bad >= 0) geo_fail(FSPT_E_INVALID, "node %d: child index out of range (%d, %d)", bad, bl, br);
       const size_t bytes = NI ? (k1 - k0) * 64 : 64;
-      e = cudaMemcpyAsync(reinterpret_cast<uint8_t*>(c->d_nodes) + k0 * 64, nodes, bytes, cudaMemcpyHostToDevice, c->stream);
+      e = cudaMemcpyAsync(c->d_nodes.p + k0 * 64, nodes, bytes, cudaMemcpyHostToDevice, c->stream);
       if (e == cudaSuccess && ring_wraps) e = cudaEventRecord(c->ev_ring[slot], c->stream);
     } else {
       const int t0 = (ring_item - n_node_items) * tri_chunk, t1 = std::min(T + 3, t0 + tri_chunk), ts = std::min(T, t1);
       float* tris = reinterpret_cast<float*>(hs);
       float* shade = reinterpret_cast<float*>(hs + (size_t)tri_chunk * 48);
       pack_tri_chunk(s, pre, t0, t1, tris, shade);
-      e = cudaMemcpyAsync(reinterpret_cast<uint8_t*>(c->d_tris) + (size_t)t0 * 48, tris, (size_t)(t1 - t0) * 48, cudaMemcpyHostToDevice, c->stream);
+      e = cudaMemcpyAsync(c->d_tris.p + (size_t)t0 * 48, tris, (size_t)(t1 - t0) * 48, cudaMemcpyHostToDevice, c->stream);
       if (e == cudaSuccess && ts > t0)
-        e = cudaMemcpyAsync(reinterpret_cast<uint8_t*>(c->d_shade) + (size_t)t0 * 192, shade, (size_t)(ts - t0) * 192, cudaMemcpyHostToDevice, c->stream);
+        e = cudaMemcpyAsync(c->d_shade.p + (size_t)t0 * 192, shade, (size_t)(ts - t0) * 192, cudaMemcpyHostToDevice, c->stream);
       if (e == cudaSuccess && ring_wraps) e = cudaEventRecord(c->ev_ring[slot], c->stream);
     }
     if (e != cudaSuccess) dma_err.store((int)e);
@@ -1329,21 +1260,7 @@ static int scene_upload_impl(fspt_ctx* ctx, const fspt_scene_desc* s, bool async
     CK(cudaEventRecord(c->ev_env, c->stream));
   }
   lap("geometry + env + layer scan");
-  // env: test knob for the LSU-only instantiation of k_trace
-  if ((rc_ = linear_tex(c, &c->nodes_tex, c->d_nodes, nodes_bytes, !getenv("FSPT_NO_NODE_TEX")))) return rc_;
-  c->sc.nodes = reinterpret_cast<const float4*>(c->d_nodes);
-  c->sc.tris = reinterpret_cast<const float4*>(c->d_tris);
-  c->sc.shade = reinterpret_cast<const float4*>(c->d_shade);
-  c->sc.bins = reinterpret_cast<const float4*>(c->d_bins);
-  c->bytes_nodes = nodes_bytes; c->bytes_tris = tris_bytes; c->bytes_shade = shade_bytes; c->bytes_bins = bins_bytes;
-  c->sc.root_ref = ref[0];
-  c->sc.n_tris = T; c->sc.n_interior = (int)NI;
-  c->sc.atlas_res = s->atlas_res; c->sc.atlas_layers = s->atlas_layers; c->sc.env_w = s->env_width; c->sc.env_h = s->env_height;
-  c->sc.n_bins = s->env_bins;
-  set_env_constants(c->sc);
-  c->has_dielectric = dielectric;
-  c->scene_bytes = (size_t)N * 36 + (size_t)T * (36 + 48 + 108 + 24) + (size_t)s->atlas_res * s->atlas_res * 4 * s->atlas_layers +
-                   env_bytes + (size_t)s->env_bins * 8;
+  if ((rc_ = publish_scene(c, si))) return rc_;
   // ---- the atlas part: here, or on the context's atlas thread (the caller's atlas stays borrowed until it is joined).
   // Measured alternatives (e2e step of the bench scene, asynchronous upload, 29.4 ms as built): the layer scan inside the
   // atlas part instead of the staging region 29.8 (the upload returns 0.2 ms earlier but the atlas lands 0.7 ms later, and
@@ -1377,7 +1294,7 @@ static int scene_upload_impl(fspt_ctx* ctx, const fspt_scene_desc* s, bool async
     });
     lap("atlas part handed to its thread");
   } else {
-    if ((rc_ = stage_atlas(c, job))) { c->error = c->atlas_error; return rc_; }
+    if ((rc_ = stage_atlas(c, job))) { c->error = "atlas upload: " + c->atlas_error; return rc_; }
     lap("atlas part");
   }
   if (geo.code != FSPT_OK) return fail(c, geo.code, "%s", geo.msg);
@@ -1457,7 +1374,7 @@ int fspt_clear(fspt_ctx* ctx) {
   Ctx* c = reinterpret_cast<Ctx*>(ctx);
   if (!c) return FSPT_E_INVALID;
   CK(cudaSetDevice(c->device));
-  CK(cudaMemsetAsync(c->d_fb, 0, (size_t)c->n_pixels * 16, c->stream));
+  CK(cudaMemsetAsync(c->d_fb.p, 0, (size_t)c->n_pixels * 16, c->stream));
   c->next_tick = 0;
   c->accum_samples = 0;
   c->stats.samples = 0;
@@ -1474,7 +1391,7 @@ int fspt_render(fspt_ctx* ctx, const fspt_frame_params* frame, uint32_t first_ti
   CK(cudaSetDevice(c->device));
   const FrameParams fp = make_frame(c, frame);
   c->ev_trace_used = 0;
-  CK(cudaMemcpyAsync(c->d_stats + 4, c->d_stats, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
+  CK(cudaMemcpyAsync(c->d_stats.p + 4, c->d_stats.p, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
   // all rand bases of this call go up in one copy: [0,cap) camera, [cap,2cap) tracer
   {
     int rc0 = stage_rand_bases(c, rand_base_camera, rand_base_tracer, n_samples);
@@ -1486,7 +1403,7 @@ int fspt_render(fspt_ctx* ctx, const fspt_frame_params* frame, uint32_t first_ti
   const int wave_S = (int)std::max<size_t>(1, std::min<size_t>((size_t)c->wave_cap, c->wave_paths / ((size_t)fp.rw * fp.rh)));
   for (int done = 0; done < n_samples;) {
     const int S = std::min(wave_S, n_samples - done);
-    int rc = render_wave(c, fp, first_tick + (uint32_t)done, S, c->d_rb + done, c->d_rb + c->rb_cap + done);
+    int rc = render_wave(c, fp, first_tick + (uint32_t)done, S, c->d_rb.p + done, c->d_rb.p + c->rb_cap + done);
     if (rc) return rc;
     done += S;
   }
@@ -1516,11 +1433,11 @@ int fspt_resolve(fspt_ctx* ctx, const fspt_post_params* post, uint8_t* rgba8_out
   CK(cudaSetDevice(c->device));
   dim3 blk(32, 8), grd((c->width + 31) / 32, (c->height + 7) / 8);
   const int use_div = c->accum_mode == 1;  // sum mode: every pixel is divided by its own sample count (alpha channel)
-  k_post<<<grd, blk, 0, c->stream>>>(c->d_fb, c->d_rgba8, c->width, c->height, post->exposure, post->saturation,
+  k_post<<<grd, blk, 0, c->stream>>>(c->d_fb.p, c->d_rgba8.p, c->width, c->height, post->exposure, post->saturation,
                                      post->denoise ? 1 : 0, post->max_sigma, post->scale, use_div);
   c->stats.kernel_launches++;
   CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(rgba8_out, c->d_rgba8, (size_t)c->n_pixels * 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(rgba8_out, c->d_rgba8.p, (size_t)c->n_pixels * 4, cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
   return FSPT_OK;
 }
@@ -1529,7 +1446,7 @@ int fspt_read_accum(fspt_ctx* ctx, float* out) {
   Ctx* c = reinterpret_cast<Ctx*>(ctx);
   if (!c || !out) return FSPT_E_INVALID;
   CK(cudaSetDevice(c->device));
-  CK(cudaMemcpyAsync(out, c->d_fb, (size_t)c->n_pixels * 16, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(out, c->d_fb.p, (size_t)c->n_pixels * 16, cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
   return FSPT_OK;
 }
@@ -1538,7 +1455,7 @@ int fspt_write_accum(fspt_ctx* ctx, const float* in, uint32_t next_tick) {
   Ctx* c = reinterpret_cast<Ctx*>(ctx);
   if (!c || !in) return FSPT_E_INVALID;
   CK(cudaSetDevice(c->device));
-  CK(cudaMemcpyAsync(c->d_fb, in, (size_t)c->n_pixels * 16, cudaMemcpyHostToDevice, c->stream));
+  CK(cudaMemcpyAsync(c->d_fb.p, in, (size_t)c->n_pixels * 16, cudaMemcpyHostToDevice, c->stream));
   CK(cudaStreamSynchronize(c->stream));
   c->next_tick = next_tick;
   c->accum_samples = next_tick;
@@ -1557,7 +1474,7 @@ int fspt_accum_device_ptr(fspt_ctx* ctx, void** dptr, uint64_t* n_floats, uint64
   if (!c) return FSPT_E_INVALID;
   CK(cudaSetDevice(c->device));
   CK(cudaStreamSynchronize(c->stream));
-  if (dptr) *dptr = c->d_fb;
+  if (dptr) *dptr = c->d_fb.p;
   if (n_floats) *n_floats = (uint64_t)c->n_pixels * 4;
   if (n_samples) *n_samples = c->accum_samples;
   return FSPT_OK;
@@ -1582,7 +1499,7 @@ int fspt_debug_primary(fspt_ctx* ctx, const fspt_frame_params* frame, float rand
     int rc0 = stage_rand_bases(c, &rand_base_camera, nullptr, 1);
     if (rc0) return rc0;
   }
-  k_camera<<<(P + 255) / 256, 256, 0, c->stream>>>(fp, c->d_rb, P, make_fastdiv(1u, (unsigned long long)P), c->ps, c->d_cam_pos, c->d_cam_dir);
+  k_camera<<<(P + 255) / 256, 256, 0, c->stream>>>(fp, c->d_rb.p, P, make_fastdiv(1u, (unsigned long long)P), c->ps, c->d_cam_pos.p, c->d_cam_dir.p);
   c->stats.kernel_launches++;
   int rc = set_counts(c, P, 0);
   if (rc) return rc;
@@ -1595,7 +1512,7 @@ int fspt_debug_primary(fspt_ctx* ctx, const fspt_frame_params* frame, float rand
   std::vector<int> cnt(P);
   CK(cudaMemcpy2D(ro.data(), 16, c->ps.rec + 0, 16 * FSPT_PATH_WORDS, 16, P, cudaMemcpyDeviceToHost));
   CK(cudaMemcpy2D(rdv.data(), 16, c->ps.rec + 1, 16 * FSPT_PATH_WORDS, 16, P, cudaMemcpyDeviceToHost));
-  CK(cudaMemcpy(cnt.data(), c->d_count_out, (size_t)P * 4, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(cnt.data(), c->d_count_out.p, (size_t)P * 4, cudaMemcpyDeviceToHost));
   for (int j = 0; j < P; ++j) {
     int x, y;
     if (fp.tiled) {
@@ -1608,8 +1525,8 @@ int fspt_debug_primary(fspt_ctx* ctx, const fspt_frame_params* frame, float rand
     if (index_out) memcpy(&index_out[px], &rdv[j].w, 4);
     if (count_out) count_out[px] = cnt[j];
   }
-  if (pos4_out) CK(cudaMemcpy(pos4_out, c->d_cam_pos, (size_t)P * 16, cudaMemcpyDeviceToHost));
-  if (dir4_out) CK(cudaMemcpy(dir4_out, c->d_cam_dir, (size_t)P * 16, cudaMemcpyDeviceToHost));
+  if (pos4_out) CK(cudaMemcpy(pos4_out, c->d_cam_pos.p, (size_t)P * 16, cudaMemcpyDeviceToHost));
+  if (dir4_out) CK(cudaMemcpy(dir4_out, c->d_cam_dir.p, (size_t)P * 16, cudaMemcpyDeviceToHost));
   return pull_stats(c);
 }
 
@@ -1633,7 +1550,7 @@ int fspt_debug_trace(fspt_ctx* ctx, const float* pos4, const float* dir4, int32_
     ro.resize(n); rdv.resize(n); cnt.resize(n);
     CK(cudaMemcpy2DAsync(ro.data(), 16, c->ps.rec + 0, 16 * FSPT_PATH_WORDS, 16, n, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaMemcpy2DAsync(rdv.data(), 16, c->ps.rec + 1, 16 * FSPT_PATH_WORDS, 16, n, cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaMemcpyAsync(cnt.data(), c->d_count_out, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(cnt.data(), c->d_count_out.p, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     for (int i = 0; i < n; ++i) {
       if (t_out) t_out[done + i] = ro[i].w;
@@ -1649,7 +1566,7 @@ int fspt_debug_last_color(fspt_ctx* ctx, float* out) {
   Ctx* c = reinterpret_cast<Ctx*>(ctx);
   if (!c || !out) return FSPT_E_INVALID;
   CK(cudaSetDevice(c->device));
-  CK(cudaMemcpyAsync(out, c->d_last_color, (size_t)c->n_pixels * 16, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(out, c->d_last_color.p, (size_t)c->n_pixels * 16, cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
   return FSPT_OK;
 }
@@ -1658,11 +1575,10 @@ int fspt_debug_math(fspt_ctx* ctx, int32_t fn, const float* x, const float* y, f
   Ctx* c = reinterpret_cast<Ctx*>(ctx);
   if (!c || !x || !out || n < 0) return FSPT_E_INVALID;
   CK(cudaSetDevice(c->device));
-  float* buf = nullptr;  // one allocation (x | y | out), released on every path
+  DevBuf<float> buf;  // one allocation (x | y | out), released on every path
   const size_t stride = (size_t)n + 1;
-  CK(cudaMalloc(&buf, 3 * stride * 4));
-  struct Free { float* p; ~Free() { cudaFree(p); } } guard{buf};
-  float *dx = buf, *dy = buf + stride, *dout = buf + 2 * stride;
+  CK(buf.fit(3 * stride * 4));
+  float *dx = buf.p, *dy = buf.p + stride, *dout = buf.p + 2 * stride;
   CK(cudaMemcpy(dx, x, (size_t)n * 4, cudaMemcpyHostToDevice));
   if (y) CK(cudaMemcpy(dy, y, (size_t)n * 4, cudaMemcpyHostToDevice)); else CK(cudaMemset(dy, 0, (size_t)n * 4));
   if (n) k_debug_math<<<(n + 255) / 256, 256, 0, c->stream>>>(fn, dx, dy, dout, n);
@@ -1743,7 +1659,7 @@ int fspt_comm_init(fspt_ctx* ctx, const uint8_t* id_bytes, int32_t rank, int32_t
   memcpy(&id, id_bytes, sizeof id);
   NK(N->CommInitRank(&c->comm, world, id, rank));
   c->comm_rank = rank; c->comm_world = world;
-  if (!c->d_hdr) CK(cudaMalloc(&c->d_hdr, 512));  // [0, 256) geometry header, [256, 512) atlas header
+  CK(c->d_hdr.fit(512));  // [0, 256) geometry header, [256, 512) atlas header
   return FSPT_OK;
 }
 
@@ -1770,7 +1686,7 @@ int fspt_reduce_accum(fspt_ctx* ctx, int32_t root) {
   NcclApi* N = nccl_api();
   if (!c->ev_red0) { CK(cudaEventCreate(&c->ev_red0)); CK(cudaEventCreate(&c->ev_red1)); }
   CK(cudaEventRecord(c->ev_red0, c->stream));
-  NK(N->Reduce(c->d_fb, c->d_fb, (size_t)c->n_pixels * 4, ncclFloat32, ncclSum, root, c->comm, c->stream));
+  NK(N->Reduce(c->d_fb.p, c->d_fb.p, (size_t)c->n_pixels * 4, ncclFloat32, ncclSum, root, c->comm, c->stream));
   CK(cudaEventRecord(c->ev_red1, c->stream));
   c->reduce_timed = true;
   c->stats.kernel_launches++;
@@ -1794,80 +1710,41 @@ int fspt_scene_broadcast(fspt_ctx* ctx, int32_t root) {
   static_assert(sizeof(SceneHeader) <= 256, "header buffer");
   if (!c->ev_bcast) CK(cudaEventCreateWithFlags(&c->ev_bcast, cudaEventDisableTiming));
   if (is_root) {
-    h.bytes_nodes = c->bytes_nodes; h.bytes_tris = c->bytes_tris; h.bytes_shade = c->bytes_shade;
-    h.bytes_bins = c->bytes_bins;
-    h.scene_bytes = c->scene_bytes;
-    h.root_ref = c->sc.root_ref; h.n_tris = c->sc.n_tris; h.n_interior = c->sc.n_interior;
-    h.atlas_res = c->sc.atlas_res; h.atlas_layers = c->sc.atlas_layers; h.env_w = c->sc.env_w; h.env_h = c->sc.env_h;
-    h.n_bins = c->sc.n_bins;
-    h.has_dielectric = c->has_dielectric ? 1 : 0;
+    h.scene = c->info;
     h.magic = 0x46535054;
-    CK(cudaMemcpyAsync(c->d_hdr, &h, sizeof h, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(c->d_hdr.p, &h, sizeof h, cudaMemcpyHostToDevice, c->stream));
   } else {
     CK(cudaStreamSynchronize(c->stream));  // nothing of the previous scene may still be in flight
     CK(cudaStreamSynchronize(c->copy_stream));
   }
-  NK(N->Broadcast(c->d_hdr, c->d_hdr, sizeof h, ncclUint8, root, c->comm, c->stream));
+  NK(N->Broadcast(c->d_hdr.p, c->d_hdr.p, sizeof h, ncclUint8, root, c->comm, c->stream));
   if (!is_root) {
-    CK(cudaMemcpyAsync(&h, c->d_hdr, sizeof h, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(&h, c->d_hdr.p, sizeof h, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     if (h.magic != 0x46535054) return fail(c, FSPT_E_NCCL, "fspt_scene_broadcast: bad header from rank %d", root);
   }
-  const size_t env_bytes = (size_t)h.env_w * h.env_h * 4;
-  if ((rc = ensure(c, c->d_lin_env, c->cap_lin_env, env_bytes))) return rc;
-  uint8_t* lin = reinterpret_cast<uint8_t*>(c->d_lin_env);
+  const SceneInfo& si = h.scene;
+  const size_t env_pitch = (size_t)si.env_w * 4, env_bytes = env_pitch * si.env_h;
+  CK(c->d_lin_env.fit(env_bytes));
+  uint8_t* lin = c->d_lin_env.p;
   if (is_root) {
-    CK(cudaMemcpy2DFromArrayAsync(lin, (size_t)h.env_w * 4, c->env_arr, 0, 0, (size_t)h.env_w * 4, h.env_h,
-                                  cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaMemcpy2DFromArrayAsync(lin, env_pitch, c->env.arr, 0, 0, env_pitch, si.env_h, cudaMemcpyDeviceToDevice, c->stream));
   } else {
     // storage on the receiving side: same reuse rules as fspt_scene_upload
     c->has_scene = false;
-    if ((rc = ensure(c, c->d_nodes, c->cap_nodes, h.bytes_nodes))) return rc;
-    if ((rc = ensure(c, c->d_tris, c->cap_tris, h.bytes_tris))) return rc;
-    if ((rc = ensure(c, c->d_shade, c->cap_shade, h.bytes_shade))) return rc;
-    if ((rc = ensure(c, c->d_bins, c->cap_bins, h.bytes_bins))) return rc;
-    if (!c->env_arr || c->env_W != h.env_w || c->env_H != h.env_h) {
-      cudaResourceDesc rd = {};
-      rd.resType = cudaResourceTypeArray;
-      cudaTextureDesc td = {};
-      td.addressMode[0] = td.addressMode[1] = td.addressMode[2] = cudaAddressModeClamp;
-      td.filterMode = cudaFilterModePoint;
-      td.readMode = cudaReadModeElementType;
-      cudaChannelFormatDesc fmt = cudaCreateChannelDesc<uchar4>();
-      if (c->sc.env) cudaDestroyTextureObject(c->sc.env);
-      c->sc.env = 0;
-      if (c->env_arr) cudaFreeArray(c->env_arr);
-      c->env_arr = nullptr;
-      CK(cudaMallocArray(&c->env_arr, &fmt, h.env_w, h.env_h));
-      rd.res.array.array = c->env_arr;
-      CK(cudaCreateTextureObject(&c->sc.env, &rd, &td, nullptr));
-      c->env_W = h.env_w; c->env_H = h.env_h;
-    }
+    if ((rc = fit_scene(c, si))) return rc;
   }
   NK(N->GroupStart());
-  NK(N->Broadcast(c->d_nodes, c->d_nodes, h.bytes_nodes, ncclUint8, root, c->comm, c->stream));
-  NK(N->Broadcast(c->d_tris, c->d_tris, h.bytes_tris, ncclUint8, root, c->comm, c->stream));
-  NK(N->Broadcast(c->d_shade, c->d_shade, h.bytes_shade, ncclUint8, root, c->comm, c->stream));
-  NK(N->Broadcast(c->d_bins, c->d_bins, h.bytes_bins, ncclUint8, root, c->comm, c->stream));
+  NK(N->Broadcast(c->d_nodes.p, c->d_nodes.p, si.bytes_nodes, ncclUint8, root, c->comm, c->stream));
+  NK(N->Broadcast(c->d_tris.p, c->d_tris.p, si.bytes_tris, ncclUint8, root, c->comm, c->stream));
+  NK(N->Broadcast(c->d_shade.p, c->d_shade.p, si.bytes_shade, ncclUint8, root, c->comm, c->stream));
+  NK(N->Broadcast(c->d_bins.p, c->d_bins.p, si.bytes_bins, ncclUint8, root, c->comm, c->stream));
   NK(N->Broadcast(lin, lin, env_bytes, ncclUint8, root, c->comm, c->stream));
   NK(N->GroupEnd());
   c->stats.kernel_launches += 6;
   if (!is_root) {
-    CK(cudaMemcpy2DToArrayAsync(c->env_arr, 0, 0, lin, (size_t)h.env_w * 4, (size_t)h.env_w * 4, h.env_h,
-                                cudaMemcpyDeviceToDevice, c->stream));
-    if ((rc = linear_tex(c, &c->nodes_tex, c->d_nodes, h.bytes_nodes))) return rc;
-    c->bytes_nodes = h.bytes_nodes; c->bytes_tris = h.bytes_tris; c->bytes_shade = h.bytes_shade;
-    c->bytes_bins = h.bytes_bins;
-    c->sc.nodes = reinterpret_cast<const float4*>(c->d_nodes);
-    c->sc.tris = reinterpret_cast<const float4*>(c->d_tris);
-    c->sc.shade = reinterpret_cast<const float4*>(c->d_shade);
-    c->sc.bins = reinterpret_cast<const float4*>(c->d_bins);
-    c->sc.root_ref = h.root_ref; c->sc.n_tris = h.n_tris; c->sc.n_interior = h.n_interior;
-    c->sc.atlas_res = h.atlas_res; c->sc.atlas_layers = h.atlas_layers; c->sc.env_w = h.env_w; c->sc.env_h = h.env_h;
-    c->sc.n_bins = h.n_bins;
-    set_env_constants(c->sc);
-    c->has_dielectric = h.has_dielectric != 0;
-    c->scene_bytes = h.scene_bytes;
+    CK(cudaMemcpy2DToArrayAsync(c->env.arr, 0, 0, lin, env_pitch, env_pitch, si.env_h, cudaMemcpyDeviceToDevice, c->stream));
+    if ((rc = publish_scene(c, si))) return rc;
     c->has_scene = true;
   }
   CK(cudaEventRecord(c->ev_bcast, c->stream));

@@ -84,6 +84,22 @@ def _worker(rank, world, port, out_dir):
     ctx.reduce_accum(0)
     if rank == 0:
         np.save(os.path.join(out_dir, "sum_after.npy"), ctx.read_accum())
+    # (7) a scene of another atlas resolution and environment size: the receiver re-creates every array (a non-power-of-
+    # two environment, refractive materials); (8) the same scene with plain atlas layers on the wire: the receiver
+    # switches from the interleaved array to the plain one; (9) and back.  Every rank renders all ticks of the whole frame.
+    sp, cam_p = scenes.pbr_scene(atlas_res=64, subdiv=2, env_size=(96, 48))
+    fr_p = ctx.frame(cam_p["eye"], cam_p["dir"], cam_p["fov_scale"], scenes.lens_features(cam_p), cam_p["env_theta"])
+    ctx.set_accum_mode(0)
+    for step, plain in ((7, False), (8, True), (9, False)):
+        if rank == 0:
+            if plain:
+                os.environ["FSPT_PLAIN_ATLAS"] = "1"
+            ctx.scene_upload(sp)
+            os.environ.pop("FSPT_PLAIN_ATLAS", None)
+        ctx.scene_broadcast(0)
+        ctx.clear()
+        ctx.render(fr_p, 0, rc, rt)
+        np.save(os.path.join(out_dir, "step%d_rank%d.npy" % (step, rank)), ctx.read_accum())
     ctx.close()
     dist.destroy_process_group()
 
@@ -130,3 +146,11 @@ def test_two_gpu_sample_sharding_matches_oracle(tmp_path, oracle_mod):
     sum1 = np.load(tmp_path / "sum1.npy")
     assert np.array_equal(sum1[..., :3].view(np.uint32), (z + cols[0]).view(np.uint32)) and np.all(sum1[..., 3] == 1)
     assert np.array_equal(np.load(tmp_path / "sum_after.npy").view(np.uint32), first.view(np.uint32))
+    # a received scene renders the bits of the uploaded one: new array shapes, plain atlas layers, interleaved again
+    # (the plain and the interleaved atlas sample the same bits, test_gpu_api.py::test_plain_atlas_fallback_is_bit_identical)
+    step7 = np.load(tmp_path / "step7_rank0.npy")
+    assert float(step7[..., :3].max()) > 0.0
+    for step in (7, 8, 9):
+        r0, r1 = np.load(tmp_path / ("step%d_rank0.npy" % step)), np.load(tmp_path / ("step%d_rank1.npy" % step))
+        assert np.array_equal(r0.view(np.uint32), r1.view(np.uint32)), step
+        assert np.array_equal(r0.view(np.uint32), step7.view(np.uint32)), step
