@@ -25,7 +25,7 @@ def main():
     W, H = [int(x) for x in a.res.lower().split("x")]
     t0 = time.time()
     if a.scene in ("bunny", "soup", "pbr"):
-        sa, cam = {"bunny": scenes.bunny_class, "soup": scenes.sphere_soup, "pbr": scenes.pbr_scene}[a.scene]()
+        sa, cam = {"bunny": scenes.bunny_class, "soup": scenes.sphere_soup, "pbr": scenes.pbr_scene}[a.scene](device=a.device)
         pt = PathTracer(sa, (W, H), cam, device=a.device, seed=a.seed)
     else:
         pt = PathTracer.from_scene(a.scene, (W, H), device=a.device, seed=a.seed)

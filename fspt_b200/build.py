@@ -39,18 +39,20 @@ def build(force=False, verbose=False, defines=(), out=None):
     os.makedirs(os.path.dirname(lib), exist_ok=True)
     tag = "" if out is None else "_" + os.path.basename(out).replace(".so", "")
     obj_cu = os.path.join(OUT_DIR, "fspt_api%s.o" % tag)
+    obj_bvh = os.path.join(OUT_DIR, "bvh_device.o")
     host = ["bvh_builder", "atlas_packer"]
     objs = [os.path.join(OUT_DIR, h + ".o") for h in host]
     cmds = [[NVCC] + NVCC_FLAGS + list(defines) + ["-c", os.path.join(CSRC, "fspt_api.cu"), "-o", obj_cu]]
+    cmds += [[NVCC] + NVCC_FLAGS + ["-c", os.path.join(CSRC, "bvh_device.cu"), "-o", obj_bvh]]
     cmds += [["g++"] + CXX_FLAGS + ["-c", os.path.join(CSRC, h + ".cpp"), "-o", o] for h, o in zip(host, objs)]
-    cmds += [[NVCC, "-shared", "-o", lib, obj_cu] + objs + ["-Xlinker", "--no-undefined", "-lpthread"]]
+    cmds += [[NVCC, "-shared", "-o", lib, obj_cu, obj_bvh] + objs + ["-Xlinker", "--no-undefined", "-lpthread"]]
     for cmd in cmds:
         r = subprocess.run(cmd, capture_output=True, text=True)
         if verbose or r.returncode != 0:
             sys.stderr.write(" ".join(cmd) + "\n" + r.stdout + r.stderr)
         if r.returncode != 0:
             raise RuntimeError("build failed: " + " ".join(cmd))
-        if cmd[0] == NVCC and "-c" in cmd and out is None:
+        if cmd[0] == NVCC and "-c" in cmd and out is None and obj_cu in cmd:
             with open(os.path.join(OUT_DIR, "ptxas.log"), "w") as f:
                 f.write(r.stderr)
     return lib

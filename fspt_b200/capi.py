@@ -55,7 +55,7 @@ EXPORTS = [
     "fspt_debug_last_color", "fspt_debug_math", "fspt_debug_read_bandwidth", "fspt_get_stats", "fspt_synchronize", "fspt_bvh_build", "fspt_bvh_build2",
     "fspt_env_bins", "fspt_pack_layer", "fspt_set_param", "fspt_set_tile", "fspt_comm_unique_id", "fspt_comm_init",
     "fspt_comm_destroy", "fspt_reduce_accum", "fspt_scene_broadcast", "fspt_scene_upload_async", "fspt_scene_upload_wait",
-    "fspt_host_register", "fspt_host_unregister", "fspt_debug_pack_scene",
+    "fspt_host_register", "fspt_host_unregister", "fspt_debug_pack_scene", "fspt_bvh_build_device", "fspt_device_check",
 ]
 PARAM_ANYHIT, PARAM_MAX_REFRACTIONS, PARAM_SANITIZE_NAN = 1, 2, 3
 
@@ -144,6 +144,30 @@ def bvh_build(verts, max_tris=4, n_threads=0, box_verts=None):
     if rc != FSPT_OK:
         raise FsptError(rc, "fspt_bvh_build failed (degenerate input: the JavaScript builder would not terminate)")
     return nodes[: n.value].copy(), order, int(depth.value)
+
+
+def bvh_build_device(verts, max_tris=4, box_verts=None, device=0):
+    """fspt_bvh_build_device: the same tree as bvh_build, built on CUDA device `device`.  Returns (nodes, order, depth)."""
+    lib = load()
+    verts = np.ascontiguousarray(verts, dtype=np.float64).reshape(-1, 9)
+    T = verts.shape[0]
+    if box_verts is not None:
+        box_verts = np.ascontiguousarray(box_verts, dtype=np.float64).reshape(-1, 9)
+        assert box_verts.shape == verts.shape
+    nodes = np.empty((2 * T + 1, 9), np.float32)
+    order = np.empty(T, np.int32)
+    n = C.c_int32(0)
+    depth = C.c_int32(0)
+    rc = lib.fspt_bvh_build_device(C.c_int32(device), ptr(verts), ptr(box_verts), C.c_int32(T), C.c_int32(max_tris),
+                                   ptr(nodes), ptr(order), C.byref(n), C.byref(depth))
+    if rc != FSPT_OK:
+        raise FsptError(rc, (lib.fspt_last_error(None) or b"").decode())
+    return nodes[: n.value].copy(), order, int(depth.value)
+
+
+def device_usable(device=0):
+    """fspt_device_check: True when CUDA device `device` is an sm_100 device the library's kernels run on."""
+    return load().fspt_device_check(C.c_int32(device)) == FSPT_OK
 
 
 def env_bins(rgba8):

@@ -25,23 +25,9 @@
 #include <vector>
 
 #include "../../include/fspt_b200.h"
+#include "bvh_sah.h"
 
 namespace {
-
-struct Aabb {
-  double mn[3], mx[3];
-  void reset() { for (int k = 0; k < 3; ++k) { mn[k] = INFINITY; mx[k] = -INFINITY; } }
-  // Math.min / Math.max (vector.js:55-61) incl. their signed-zero rule (-0 < +0); inputs are never NaN (checked)
-  static double lo(double a, double b) { return a < b ? a : (b < a ? b : (signbit(a) ? a : b)); }
-  static double hi(double a, double b) { return a < b ? b : (b < a ? a : (signbit(a) ? b : a)); }
-  void grow(const Aabb& b) {
-    for (int k = 0; k < 3; ++k) { mn[k] = lo(mn[k], b.mn[k]); mx[k] = hi(mx[k], b.mx[k]); }
-  }
-  double area() const {  // BoundingBox.getSurfaceArea, bvh.js:137-142
-    double xl = mx[0] - mn[0], yl = mx[1] - mn[1], zl = mx[2] - mn[2];
-    return (xl * yl + xl * zl + yl * zl) * 2;
-  }
-};
 
 struct BuildNode { Aabb box; int32_t left, right, lo, hi; };  // left < 0 => leaf over idx[0][lo,hi)
 
@@ -133,7 +119,7 @@ void split_parallel(Ctx& c, int32_t lo, int32_t hi, double parent, double& best,
       bb.grow(c.tb[ix[i]]);
       const double sAf = bb.area(), sAb = sback[i];
       const int32_t kk = i - lo;
-      const double cost = 1 + (sAf / parent) * 1 * (double)(kk + 1) + (sAb / parent) * 1 * (double)(n - 1 - kk);
+      const double cost = sah_cost(sAf, sAb, parent, kk, n);
       if (cost < bst) { bst = cost; bi = kk + 1; }
     }
     cbest[item] = bst; cbest_i[item] = bi;
@@ -180,7 +166,7 @@ int32_t build(Ctx& c, int32_t lo, int32_t hi, int d) {
       bb.grow(c.tb[ix[i]]);
       const double sAf = bb.area(), sAb = sback[i];
       const int32_t k = i - lo;
-      const double cost = 1 + (sAf / parent) * 1 * (double)(k + 1) + (sAb / parent) * 1 * (double)(n - 1 - k);
+      const double cost = sah_cost(sAf, sAb, parent, k, n);
       if (cost < best) { best = cost; best_i = k + 1; best_axis = axis; }
     }
   }
@@ -288,19 +274,17 @@ extern "C" int fspt_bvh_build2(const double* verts, const double* box_verts, int
       for (int v = 0; v < 3; ++v)
         for (int k = 0; k < 3; ++k) {
           double x = bv[(size_t)i * 9 + v * 3 + k];
-          if (!(x == x) || isinf(x)) { bad.store(1); return; }
-          b.mn[k] = Aabb::lo(x, b.mn[k]);
-          b.mx[k] = Aabb::hi(x, b.mx[k]);
+          if (!finite_coord(x)) { bad.store(1); return; }
+          b.add_point(x, k);
         }
-      for (int k = 0; k < 3; ++k) cen[k][i] = (b.mn[k] + b.mx[k]) * 0.5;  // centroid, bvh.js:130-135
+      for (int k = 0; k < 3; ++k) cen[k][i] = b.centroid(k);
       if (box_verts) {
         Aabb& n = nb[i]; n.reset();
         for (int v = 0; v < 3; ++v)
           for (int k = 0; k < 3; ++k) {
             double x = verts[(size_t)i * 9 + v * 3 + k];
-            if (!(x == x) || isinf(x)) { bad.store(1); return; }
-            n.mn[k] = Aabb::lo(x, n.mn[k]);
-            n.mx[k] = Aabb::hi(x, n.mx[k]);
+            if (!finite_coord(x)) { bad.store(1); return; }
+            n.add_point(x, k);
           }
       }
     }

@@ -39,9 +39,13 @@
 #include "shade.cuh"
 #include "traverse.cuh"
 
+namespace fspt {
+thread_local std::string g_create_error;  // fspt_last_error(NULL); the device BVH builder (bvh_device.cu) reports here too
+}
+
 namespace {
 
-thread_local std::string g_create_error;
+using fspt::g_create_error;
 
 // A block of device memory (DevBuf) or page-locked host memory (PinnedBuf) that only grows: fit() keeps it when it is
 // large enough and re-allocates it otherwise.  Freed on destruction.

@@ -35,7 +35,7 @@ class PathTracer:
         """PathTracer(scenePath, ...) (main.js:915-950 -> start(), :879-913): compile the scene JSON, upload,
         shoot the autofocus ray."""
         from . import scene_json
-        sa, cam = scene_json.load_scene(scene_path, asset_root)
+        sa, cam = scene_json.load_scene(scene_path, asset_root, device=device)
         pt = cls(sa, resolution, cam, device=device, seed=seed, exposure=cam.get("exposure", 1.0),
                  max_samples=cam.get("samples", 2000), **kw)
         if autofocus:

@@ -2,6 +2,7 @@
 (main.js:284-445) -- materials -> atlas layers, BVH build, the flatten loop, environment + radiance bins --
 producing the exact flattened arrays the reference uploads (SURVEY.md appendix A), ready for
 fspt_scene_upload.  Host-side only; BVH construction and env bins run in the native library."""
+import functools
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -109,8 +110,22 @@ def material_row(m):
                      m["emittance"][0], m["emittance"][1], m["emittance"][2], m["ior"], m["dielectric"], 0], np.float64)
 
 
-def flatten(triangle_sets, atlas, env, bins, normalize=None, n_threads=0, builder=None):
-    """new BVH(geometry, 4) + serializeTree + the flatten loop (main.js:337-392) + light buffers (:394-401)."""
+# Scenes of at least this many triangles build their BVH on the GPU when one is usable (both builders give the same tree).
+DEVICE_BVH_MIN_TRIS = 1 << 17
+
+
+def default_bvh_builder(n_tris, device=0):
+    """The builder flatten uses when it is given none: fspt_bvh_build_device on `device` for large scenes on a machine
+    with a usable sm_100 device, the host builder otherwise.  A device build that fails raises; it is not retried on the
+    host."""
+    if n_tris >= DEVICE_BVH_MIN_TRIS and capi.device_usable(device):
+        return functools.partial(capi.bvh_build_device, device=device)
+    return capi.bvh_build
+
+
+def flatten(triangle_sets, atlas, env, bins, normalize=None, n_threads=0, builder=None, device=0):
+    """new BVH(geometry, 4) + serializeTree + the flatten loop (main.js:337-392) + light buffers (:394-401).
+    builder: bvh_build-like callable; default default_bvh_builder(T, device)."""
     verts = np.concatenate([t.verts for t in triangle_sets], axis=0)
     build_verts = verts
     if normalize:
@@ -120,7 +135,7 @@ def flatten(triangle_sets, atlas, env, bins, normalize=None, n_threads=0, builde
         longest = float(max(max(mx[0] - mn[0], mx[1] - mn[1]), mx[2] - mn[2]))
         centroid = (mn + mx) * 0.5
         verts = (verts - centroid) * (2 * normalize / longest)
-    builder = builder or capi.bvh_build
+    builder = builder or default_bvh_builder(verts.shape[0], device)
     box = build_verts if normalize else None
     nodes, order, depth = (builder(verts, 4, n_threads, box_verts=box) if builder is capi.bvh_build
                            else builder(verts, 4, box_verts=box))

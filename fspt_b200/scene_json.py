@@ -148,8 +148,9 @@ def canvas_roundtrip(rgba):
     return out
 
 
-def compile_scene(scene, asset_root, read_text=None, load_img=None, n_threads=0, emulate_canvas=True):
-    """initBVH (main.js:284-445).  scene: dict (parsed JSON).  Returns (SceneArrays, camera dict)."""
+def compile_scene(scene, asset_root, read_text=None, load_img=None, n_threads=0, emulate_canvas=True, device=0):
+    """initBVH (main.js:284-445).  scene: dict (parsed JSON).  Returns (SceneArrays, camera dict).
+    device: the CUDA device a large scene's BVH may be built on (scene.default_bvh_builder)."""
     read_text = read_text or (lambda p: open(os.path.join(asset_root, p)).read())
     load_img = load_img or (lambda p: load_image(os.path.join(asset_root, p)))
     env = scene.get("environment")
@@ -190,7 +191,8 @@ def compile_scene(scene, asset_root, read_text=None, load_img=None, n_threads=0,
             ts.material = get_material(p, parsed["materials"].get(gname, {}), packer, assets, base)
             sets.append(ts)
     packer.setAndGetResolution()
-    sa = flatten(sets, packer.getPixels(), env_px, bins, normalize=scene.get("normalize"), n_threads=n_threads)
+    sa = flatten(sets, packer.getPixels(), env_px, bins, normalize=scene.get("normalize"), n_threads=n_threads,
+                 device=device)
     cam = dict(eye=scene.get("cameraPos") or [0, 0, 2], dir=scene.get("cameraDir") or [0, 0, -1],
                fov_scale=scene.get("fovScale") or 0.5, env_theta=scene.get("environmentTheta") or 0,
                aperture=0.02, focal_depth=2.0, exposure=scene.get("exposure") or 1.0,

@@ -18,7 +18,7 @@ def _env(env_size, kind="sun", host=None):
     return env, (host or capi).env_bins(env)
 
 
-def bunny_class(subdiv=6, atlas_res=2048, env_size=(2048, 1024), textured=True, host=None):
+def bunny_class(subdiv=6, atlas_res=2048, env_size=(2048, 1024), textured=True, host=None, device=0):
     """scene/bunny.json with the missing bunny replaced by a lumpy icosphere (20*4^subdiv triangles) and the
     dungeon maps by procedural PBR maps.  Props, transforms and material constants follow scene/bunny.json:6-41.
     host: the module that supplies the host-side scene compilers bvh_build / env_bins / pack_layer -- default the
@@ -43,10 +43,10 @@ def bunny_class(subdiv=6, atlas_res=2048, env_size=(2048, 1024), textured=True, 
         for p in props[1:]:
             for k in ("diffuse", "metallicRoughness", "normal", "emission"):
                 p.pop(k, None)
-    return compile_props(props, assets, atlas_res, _env(env_size, host=host), host=host), dict(BUNNY_CAMERA)
+    return compile_props(props, assets, atlas_res, _env(env_size, host=host), host=host, device=device), dict(BUNNY_CAMERA)
 
 
-def compile_props(props, assets, atlas_res, env_and_bins, n_threads=0, builder=None, host=None):
+def compile_props(props, assets, atlas_res, env_and_bins, n_threads=0, builder=None, host=None, device=0):
     packer = TexturePacker(atlas_res, pack_layer=host.pack_layer if host else None)
     if host is not None and builder is None:
         builder = host.bvh_build
@@ -59,7 +59,7 @@ def compile_props(props, assets, atlas_res, env_and_bins, n_threads=0, builder=N
     packer.setAndGetResolution()
     atlas = packer.getPixels()
     env, bins = env_and_bins
-    return flatten(sets, atlas, env, bins, n_threads=n_threads, builder=builder)
+    return flatten(sets, atlas, env, bins, n_threads=n_threads, builder=builder, device=device)
 
 
 def quad_scene(env_size=(64, 32)):
@@ -70,8 +70,13 @@ def quad_scene(env_size=(64, 32)):
                                                            env_theta=0.0, aperture=0.0, focal_depth=2.0)
 
 
-def sphere_soup(subdiv=7, n_soup=672320, seed=1234, env_size=(2048, 1024), albedo=0.8):
-    """BASELINE config 3: subdivided icosphere + uniform random triangle soup, Lambert rho = 0.8, aperture 0."""
+def sphere_soup_verts(subdiv=7, n_soup=672320, seed=1234):
+    """The (T, 9) float64 vertices sphere_soup builds its BVH from (the inputs of BVH builder measurements and tests)."""
+    props = _sphere_soup_props(subdiv, n_soup, seed, 0.8)
+    return np.concatenate([mesh_to_triangles(p["mesh"][0], p["mesh"][1], p).verts for p in props], axis=0)
+
+
+def _sphere_soup_props(subdiv, n_soup, seed, albedo):
     v, f = pr.icosphere(subdiv)
     props = [dict(mesh=(v, f, None), scale=0.5, rotate=[], translate=[0, 0, 0], diffuse=[albedo] * 3,
                   emittance=[0, 0, 0], metallicRoughness=[0, 1.0, 0], normals="smooth")]
@@ -82,11 +87,17 @@ def sphere_soup(subdiv=7, n_soup=672320, seed=1234, env_size=(2048, 1024), albed
         sf = np.arange(sv.shape[0], dtype=np.int64).reshape(-1, 3)
         sa_props = props + [dict(mesh=(sv, sf, None), scale=1, rotate=[], translate=[0, 0, 0], diffuse=[albedo] * 3,
                                  emittance=[0, 0, 0], metallicRoughness=[0, 1.0, 0], normals="flat")]
+    return sa_props
+
+
+def sphere_soup(subdiv=7, n_soup=672320, seed=1234, env_size=(2048, 1024), albedo=0.8, device=0):
+    """BASELINE config 3: subdivided icosphere + uniform random triangle soup, Lambert rho = 0.8, aperture 0."""
+    sa_props = _sphere_soup_props(subdiv, n_soup, seed, albedo)
     cam = dict(eye=[0, 0.3, 2.6], dir=[0, -0.1, -1], fov_scale=0.5, env_theta=0.25, aperture=0.0, focal_depth=2.0)
-    return compile_props(sa_props, {}, 4, _env(env_size)), cam
+    return compile_props(sa_props, {}, 4, _env(env_size), device=device), cam
 
 
-def pbr_scene(atlas_res=2048, subdiv=5, env_size=(2048, 1024)):
+def pbr_scene(atlas_res=2048, subdiv=5, env_size=(2048, 1024), device=0):
     """BASELINE config 4: textured quads + spheres with all four maps + one refractive prop (dielectric >= 0)."""
     v, f = pr.icosphere(subdiv)
     assets = {}
@@ -108,7 +119,7 @@ def pbr_scene(atlas_res=2048, subdiv=5, env_size=(2048, 1024)):
              normals="smooth", diffuse=[1.0, 0.8, 0.3], metallicRoughness=[1.0, 0.25, 0]),
     ]
     cam = dict(eye=[-0.2, 0.35, 2.0], dir=[0.08, -0.3, -1.0], fov_scale=0.5, env_theta=1.66, aperture=0.01, focal_depth=2.0)
-    return compile_props(props, assets, atlas_res, _env(env_size)), cam
+    return compile_props(props, assets, atlas_res, _env(env_size), device=device), cam
 
 
 def lens_features(cam):

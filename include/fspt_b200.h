@@ -242,6 +242,18 @@ int fspt_bvh_build(const double* verts, int32_t n_tris, int32_t max_tris, float*
 int fspt_bvh_build2(const double* verts, const double* box_verts, int32_t n_tris, int32_t max_tris, float* nodes_out,
                     int32_t* order_out, int32_t* n_nodes_out, int32_t* depth_out, int32_t n_threads);
 
+/* The same tree built on CUDA device `device` (sm_100 only): bit-identical to fspt_bvh_build2 on the same inputs, the same
+ * outputs (nodes_out, order_out, n_nodes, depth) and the same refusals with the same codes (FSPT_E_INVALID for NaN / inf
+ * vertices or bad arguments, FSPT_E_LIMIT where bvh.js would not terminate).  Synchronous: the call uploads the vertices,
+ * builds, downloads the results, frees its device memory and stream and restores the caller's current device; it does
+ * not synchronise the device, so a live context there keeps running.  Text of a failure through fspt_last_error(NULL).
+ * Without a usable sm_100 device it fails with FSPT_E_CUDA (no CPU fallback). */
+int fspt_bvh_build_device(int32_t device, const double* verts, const double* box_verts, int32_t n_tris, int32_t max_tris,
+                          float* nodes_out, int32_t* order_out, int32_t* n_nodes_out, int32_t* depth_out);
+/* FSPT_OK when `device` is a usable sm_100 device (what the device entry points need), FSPT_E_CUDA or FSPT_E_INVALID with
+ * text through fspt_last_error(NULL) otherwise.  Lets a host choose between the two builders without trying one. */
+int fspt_device_check(int32_t device);
+
 /* ProcessEnvRadiance(img) (env_sampler.js:1-74) on an RGBA8 RGBE image; bins_out capacity in u16. */
 int fspt_env_bins(const uint8_t* rgba8, int32_t width, int32_t height, uint16_t* bins_out, int32_t capacity,
                   int32_t* n_u16_out);
