@@ -137,6 +137,8 @@ struct Ctx {
   int width = 0, height = 0, n_pixels = 0;
   int rx0 = 0, ry0 = 0, rw = 0, rh = 0;  // the pixel rectangle this context renders (fspt_set_tile); default = frame
   cudaStream_t stream = nullptr;
+  cudaStream_t stream2 = nullptr;     // the second row band of a render (render_wave); forked from and joined to `stream`
+  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   cudaEvent_t ev_begin = nullptr, ev_end = nullptr;
   std::vector<cudaEvent_t> ev_trace;  // pairs around traversal (tag 0) / shading (tag 1) launches of the last render
   std::vector<int> ev_tag;
@@ -197,7 +199,10 @@ struct Ctx {
   DevBuf<float4> d_rec[2];    // what ps2[k] points to
   DevBuf<unsigned char> d_sh[2];
   DevBuf<float4> d_shadow;    // shadow rays of the current bounce, dense: origin | record position, direction | -
-  DevBuf<int> d_counts;       // set k at [2k, 2k+1] = (#continuation, #shadow), [32] fetch cursor (own cache line)
+  // per band b, from b * BAND_INTS: set k at [2k, 2k+1] = (#continuation, #shadow), [32] traversal fetch cursor, [64]
+  // shading tile cursor -- each cursor on a 128-byte line of its own: every warp's (block's) atomicAdd hits it
+  static constexpr int BAND_INTS = 96;
+  DevBuf<int> d_counts;
   DevBuf<int> d_count_out;    // per-slot visit count (debug)
   DevBuf<unsigned char> d_hit_flag;  // hit / miss per record position
   DevBuf<unsigned long long> d_stats;  // rays, nodes, leaves, capped
@@ -211,8 +216,8 @@ struct Ctx {
   int rb_cap = 0;
   // refraction bounces beyond NUM_BOUNCES (tracer.fs:488): path counts polled two iterations behind the enqueue
   static constexpr int POLL_SLOTS = 8;
-  PinnedBuf<int> h_poll;
-  cudaEvent_t ev_poll[POLL_SLOTS] = {};
+  PinnedBuf<int> h_poll;                   // [band * POLL_SLOTS + slot]
+  cudaEvent_t ev_poll[2][POLL_SLOTS] = {};
   // collectives (fspt_comm_init): NCCL communicator over NVLink / NVSwitch
   ncclComm_t comm = nullptr;
   int comm_rank = 0, comm_world = 1;
@@ -337,9 +342,8 @@ int alloc_wave(Ctx* c) {
   }
   c->ps = c->ps2[0];
   CK(c->d_shadow.fit(W * 32));
-  CK(c->d_counts.fit(64 * sizeof(int)));  // [0..3] the two count pairs; [32] the fetch cursor, on its own 128-byte
-                                          // line: every warp's atomicAdd hits it, nothing else should
-  CK(cudaMemset(c->d_counts.p, 0, 64 * sizeof(int)));
+  CK(c->d_counts.fit(2 * Ctx::BAND_INTS * sizeof(int)));
+  CK(cudaMemset(c->d_counts.p, 0, 2 * Ctx::BAND_INTS * sizeof(int)));
   CK(c->d_count_out.fit(W * sizeof(int)));
   CK(c->d_hit_flag.fit(W));
   CK(c->d_stats.fit(8 * sizeof(unsigned long long)));  // [0..3] live, [4..7] snapshot at render start
@@ -349,22 +353,28 @@ int alloc_wave(Ctx* c) {
   CK(c->d_rb.fit(2 * (size_t)c->rb_cap * sizeof(float)));
   CK(c->h_rb.fit(Ctx::RB_SLOTS * 2 * (size_t)c->rb_cap * sizeof(float)));
   for (auto& e : c->ev_rb) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-  CK(c->h_poll.fit(Ctx::POLL_SLOTS * sizeof(int)));
-  for (auto& e : c->ev_poll) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  CK(c->h_poll.fit(2 * Ctx::POLL_SLOTS * sizeof(int)));
+  for (auto& band : c->ev_poll)
+    for (auto& e : band) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   return FSPT_OK;
 }
 
 // ---- traversal launch helpers ---------------------------------------------------------------------------
-void record_trace_begin(Ctx* c, int tag = 0) {
+// Band b of a render (render_wave) runs on its own stream and has its own counts and cursors; band 0 is the context's
+// stream, which every other entry point uses.
+cudaStream_t band_stream(const Ctx* c, int band) { return band ? c->stream2 : c->stream; }
+int* band_counts(const Ctx* c, int band) { return c->d_counts.p + Ctx::BAND_INTS * band; }
+
+void record_trace_begin(Ctx* c, cudaStream_t s, int tag = 0) {
   if (c->ev_trace_used + 2 > c->ev_trace.size()) {
     for (int i = 0; i < 2; ++i) { cudaEvent_t e; cudaEventCreate(&e); c->ev_trace.push_back(e); }
   }
   if (c->ev_tag.size() < c->ev_trace.size() / 2) c->ev_tag.resize(c->ev_trace.size() / 2);
   c->ev_tag[c->ev_trace_used / 2] = tag;
-  cudaEventRecord(c->ev_trace[c->ev_trace_used], c->stream);
+  cudaEventRecord(c->ev_trace[c->ev_trace_used], s);
 }
-void record_trace_end(Ctx* c) {
-  cudaEventRecord(c->ev_trace[c->ev_trace_used + 1], c->stream);
+void record_trace_end(Ctx* c, cudaStream_t s) {
+  cudaEventRecord(c->ev_trace[c->ev_trace_used + 1], s);
   c->ev_trace_used += 2;
 }
 
@@ -393,8 +403,11 @@ __global__ void __launch_bounds__(256) k_interleave_atlas(cudaSurfaceObject_t su
   surf2DLayeredwrite(v, surf, x * 16, y, blockIdx.z);
 }
 
+// counts = band_counts().  The shading tile cursor [64] is zeroed here at the start of every wave; between the shading
+// launches of a wave, k_shade puts it back to 0 itself (the block that draws a launch's last ticket), which holds as long
+// as every launch runs to completion with the grid it was launched with.
 __global__ void k_set_counts(int* counts, int n_cont, int n_shadow) {
-  counts[0] = n_cont; counts[1] = n_shadow; counts[2] = 0; counts[3] = 0; counts[32] = 0;
+  counts[0] = n_cont; counts[1] = n_shadow; counts[2] = 0; counts[3] = 0; counts[32] = 0; counts[64] = 0;
 }
 
 // true when `p` points into page-locked host memory (cudaHostRegister / cudaMallocHost, by whoever): DMA can read it in place
@@ -679,43 +692,72 @@ int stage_atlas(Ctx* c, const AtlasJob& J) {
   return FSPT_OK;
 }
 
-// Traverses the continuation ray of every record of array `which` (d_counts[2*which] of them) + d_counts[2*which+1]
-// shadow rays (d_shadow); results go into the records, plus one hit/miss byte per position (for k_shade).
-int launch_trace(Ctx* c, int which, bool hit_flags, bool write_count, const FrameParams* cam = nullptr,
-                 const float* rb_cam = nullptr, int n_samples = 1) {
+// The path records, shadow rays, hit flags and sample colours of a band: its slice of the wave's arrays, from path `off`.
+struct BandSlice {
+  PathState ps[2];
+  float4* shadow;
+  unsigned char* hit_flag;
+  float4* sample_color;
+};
+BandSlice band_slice(const Ctx* c, size_t off) {
+  BandSlice b;
+  for (int k = 0; k < 2; ++k) {
+    b.ps[k].rec = c->ps2[k].rec + FSPT_PATH_WORDS * off;
+    b.ps[k].sh = c->ps2[k].sh + off;
+  }
+  b.shadow = c->d_shadow.p + 2 * off;
+  b.hit_flag = c->d_hit_flag.p + off;
+  b.sample_color = c->d_sample_color.p + off;
+  return b;
+}
+
+// Traverses the continuation ray of every record of array `which` (counts[2*which] of them) + counts[2*which+1]
+// shadow rays of band `band` (slice `sl`); results go into the records, plus one hit/miss byte per position (for k_shade).
+int launch_trace(Ctx* c, int band, const BandSlice& sl, int which, bool hit_flags, bool write_count,
+                 const FrameParams* cam = nullptr, const float* rb_cam = nullptr, int n_samples = 1) {
   TraceArgs A;
   if (cam) A.f = *cam; else memset(&A.f, 0, sizeof A.f);
   A.rb_cam = rb_cam; A.n_samples = n_samples;
   A.div_s = make_fastdiv((unsigned)std::max(1, n_samples), c->wave_paths);
   A.anyhit = c->anyhit;
   A.nodes = c->sc.nodes; A.tris = c->sc.tris; A.root_ref = c->sc.root_ref; A.nodes_tex = c->nodes_tex;
-  A.ps = c->ps2[which];
-  A.shadow_rays = c->d_shadow.p;
-  A.counts = c->d_counts.p + 2 * which;
-  A.next = c->d_counts.p + 32;
+  A.ps = sl.ps[which];
+  A.shadow_rays = sl.shadow;
+  A.counts = band_counts(c, band) + 2 * which;
+  A.next = band_counts(c, band) + 32;
   A.stats = c->d_stats.p;
   A.count_out = write_count ? c->d_count_out.p : nullptr;
-  A.hit_flag = hit_flags ? c->d_hit_flag.p : nullptr;
-  record_trace_begin(c, cam ? 2 : 0);  // tag 2: the camera-fused primary launch of a wave
+  A.hit_flag = hit_flags ? sl.hit_flag : nullptr;
+  const cudaStream_t s = band_stream(c, band);
+  record_trace_begin(c, s, cam ? 2 : 0);  // tag 2: the camera-fused primary launch of a wave
   if (A.nodes_tex) {
-    if (cam) k_trace<false, true, true><<<c->trace_blocks_cam, TRACE_THREADS, 0, c->stream>>>(A);
-    else if (write_count) k_trace<true, false, true><<<c->trace_blocks_cnt, TRACE_THREADS, 0, c->stream>>>(A);
-    else k_trace<false, false, true><<<c->trace_blocks, TRACE_THREADS, 0, c->stream>>>(A);
+    if (cam) k_trace<false, true, true><<<c->trace_blocks_cam, TRACE_THREADS, 0, s>>>(A);
+    else if (write_count) k_trace<true, false, true><<<c->trace_blocks_cnt, TRACE_THREADS, 0, s>>>(A);
+    else k_trace<false, false, true><<<c->trace_blocks, TRACE_THREADS, 0, s>>>(A);
   } else {  // node array beyond the linear-texture limit
-    if (cam) k_trace<false, true, false><<<c->trace_blocks_cam_nt, TRACE_THREADS, 0, c->stream>>>(A);
-    else if (write_count) k_trace<true, false, false><<<c->trace_blocks_cnt_nt, TRACE_THREADS, 0, c->stream>>>(A);
-    else k_trace<false, false, false><<<c->trace_blocks_nt, TRACE_THREADS, 0, c->stream>>>(A);
+    if (cam) k_trace<false, true, false><<<c->trace_blocks_cam_nt, TRACE_THREADS, 0, s>>>(A);
+    else if (write_count) k_trace<true, false, false><<<c->trace_blocks_cnt_nt, TRACE_THREADS, 0, s>>>(A);
+    else k_trace<false, false, false><<<c->trace_blocks_nt, TRACE_THREADS, 0, s>>>(A);
   }
-  record_trace_end(c);
+  record_trace_end(c, s);
   c->stats.kernel_launches++;
   CK(cudaGetLastError());
   return FSPT_OK;
 }
 
-int set_counts(Ctx* c, int n_cont, int n_shadow) {  // also zeroes #hit, #miss and the fetch cursor
-  k_set_counts<<<1, 1, 0, c->stream>>>(c->d_counts.p, n_cont, n_shadow);
+int set_counts(Ctx* c, int band, int n_cont, int n_shadow) {  // also zeroes #hit, #miss and both cursors
+  k_set_counts<<<1, 1, 0, band_stream(c, band)>>>(band_counts(c, band), n_cont, n_shadow);
   CK(cudaGetLastError());
   return FSPT_OK;
+}
+
+// The rectangle p renders and the slot -> pixel mapping that goes with it.
+void set_rect(FrameParams& p, int rx0, int ry0, int rw, int rh) {
+  p.rx0 = rx0; p.ry0 = ry0; p.rw = rw; p.rh = rh;
+  p.tiled = (p.rw % 8 == 0 && p.rh % 4 == 0) ? 1 : 0;
+  // slot -> pixel: one division by the tiles per row (dividend: a tile index) or by the row width (dividend: a pixel index)
+  p.div_row = p.tiled ? make_fastdiv((unsigned)(p.rw >> 3), ((unsigned long long)p.rw * p.rh) >> 5)
+                      : make_fastdiv((unsigned)p.rw, (unsigned long long)p.rw * p.rh);
 }
 
 FrameParams make_frame(const Ctx* c, const fspt_frame_params* f, bool whole_frame = false) {
@@ -731,12 +773,8 @@ FrameParams make_frame(const Ctx* c, const fspt_frame_params* f, bool whole_fram
     p.basis_y[0] = by.x; p.basis_y[1] = by.y; p.basis_y[2] = by.z;
   }
   p.width = c->width; p.height = c->height;
-  p.rx0 = whole_frame ? 0 : c->rx0; p.ry0 = whole_frame ? 0 : c->ry0;
-  p.rw = whole_frame ? c->width : c->rw; p.rh = whole_frame ? c->height : c->rh;
-  p.tiled = (p.rw % 8 == 0 && p.rh % 4 == 0) ? 1 : 0;
-  // slot -> pixel: one division by the tiles per row (dividend: a tile index) or by the row width (dividend: a pixel index)
-  p.div_row = p.tiled ? make_fastdiv((unsigned)(p.rw >> 3), ((unsigned long long)p.rw * p.rh) >> 5)
-                      : make_fastdiv((unsigned)p.rw, (unsigned long long)p.rw * p.rh);
+  if (whole_frame) set_rect(p, 0, 0, c->width, c->height);
+  else set_rect(p, c->rx0, c->ry0, c->rw, c->rh);
   return p;
 }
 
@@ -761,21 +799,48 @@ int stage_rand_bases(Ctx* c, const float* cam, const float* trace, int n) {
   return FSPT_OK;
 }
 
-// One wave.  Path records are dense arrays that ping-pong: set k = (array ps2[k], counts d_counts[2k .. 2k+1] =
-// #records, #shadow rays); the shadow list holds record positions; fetch cursor at d_counts[32].
+// Paths a band must hold before a rectangle is split into two bands.  Measured on a B200: two bands of 0.32 M paths
+// (800x800, 1 spp) render 3 % faster than one band, two of 29 M (1280x720, 64 spp) 0.6 % faster; smaller bands were
+// not measured, so below 2^18 paths per band a wave stays one chain of launches.
+#ifndef FSPT_BAND_MIN_PATHS
+#define FSPT_BAND_MIN_PATHS (1 << 18)
+#endif
+
+// A wave of the rectangle fp is rendered as up to two row bands, each on its own stream (band_stream) with its own slice
+// of the path arrays: every launch of a wave waits for the whole previous one, and the other band's CTAs fill the SMs
+// while one band's launch ramps up or drains.  A pixel's samples do not depend on the rectangle that renders it, so
+// the split changes no result.  The first band gets a multiple of 4 rows: a tiled rectangle gives two tiled bands.
+int split_bands(const FrameParams& fp, int S, FrameParams band[2]) {
+  const int rows0 = (fp.rh / 2) & ~3;
+  band[0] = fp;
+  if (rows0 == 0 || (size_t)S * fp.rw * rows0 < (size_t)FSPT_BAND_MIN_PATHS) return 1;
+  band[1] = fp;
+  set_rect(band[0], fp.rx0, fp.ry0, fp.rw, rows0);
+  set_rect(band[1], fp.rx0, fp.ry0 + rows0, fp.rw, fp.rh - rows0);
+  return 2;
+}
+
+// One wave.  Path records are dense arrays that ping-pong: set k = (array ps[k], counts band_counts()[2k .. 2k+1] =
+// #records, #shadow rays); the shadow list holds record positions.  The bands' launches are enqueued interleaved, so
+// that each stream always has its next launch queued behind the running one.
 int render_wave(Ctx* c, const FrameParams& fp, uint32_t first_tick, int S, const float* rb_cam, const float* rb_trace) {
-  const int P = fp.rw * fp.rh;
-  const int n_paths = S * P;
-  int rc = set_counts(c, n_paths, 0);
-  if (rc) return rc;
-  rc = launch_trace(c, 0, true, false, &fp, rb_cam, S);  // camera.fs + primary rays (tracer.fs:440), fused
-  if (rc) return rc;
+  FrameParams bfp[2];
+  const int nb = split_bands(fp, S, bfp);
+  BandSlice sl[2];
+  int cur[2] = {0, 0};
+  bool live[2] = {true, nb > 1};
+  for (int b = 0, off = 0; b < nb; ++b) {
+    sl[b] = band_slice(c, (size_t)off);
+    const int n_paths = S * bfp[b].rw * bfp[b].rh;
+    off += n_paths;
+    int rc = set_counts(c, b, n_paths, 0);
+    if (rc) return rc;
+    rc = launch_trace(c, b, sl[b], 0, true, false, &bfp[b], rb_cam, S);  // camera.fs + primary rays (tracer.fs:440), fused
+    if (rc) return rc;
+  }
+  int rc;
   ShadeArgs A;
-  A.f = fp;
   A.rb_trace = rb_trace;
-  A.hit_flag = c->d_hit_flag.p;
-  A.shadow_rays_out = c->d_shadow.p;
-  A.sample_color = c->d_sample_color.p;
   A.capped = c->d_stats.p + 3;
   A.n_samples = S;
   A.div_s = make_fastdiv((unsigned)S, c->wave_paths);
@@ -790,45 +855,67 @@ int render_wave(Ctx* c, const FrameParams& fp, uint32_t first_tick, int S, const
   if ((rc = broadcast_phase2(c))) return rc;
   if ((rc = atlas_join(c))) return rc;
   A.sc = c->sc;  // (the atlas part sets the texture objects and table pointers)
-  CK(cudaStreamWaitEvent(c->stream, c->ev_atlas, 0));
-  int cur = 0;
-  for (int b = 0; b < hard_cap; ++b) {
-    const int nxt = cur ^ 1;
-    CK(cudaMemsetAsync(c->d_counts.p + 2 * nxt, 0, 2 * sizeof(int), c->stream));
-    A.first = (b == 0);
-    A.ps = c->ps2[cur];
-    A.ps_out = c->ps2[nxt];
-    A.counts_in = c->d_counts.p + 2 * cur;
-    A.counts_out = c->d_counts.p + 2 * nxt;
-    record_trace_begin(c, 1);
-    if (c->sc.mat_tex) k_shade<true><<<c->shade_blocks, SHADE_THREADS, 1024, c->stream>>>(A);
-    else k_shade<false><<<c->shade_blocks, SHADE_THREADS, 1024, c->stream>>>(A);
-    record_trace_end(c);
+  for (int b = 0; b < nb; ++b) CK(cudaStreamWaitEvent(band_stream(c, b), c->ev_atlas, 0));
+  for (int it = 0; it < hard_cap && (live[0] || live[1]); ++it) {
+    for (int b = 0; b < nb; ++b) {
+      if (!live[b]) continue;
+      const cudaStream_t s = band_stream(c, b);
+      int* counts = band_counts(c, b);
+      const int nxt = cur[b] ^ 1;
+      CK(cudaMemsetAsync(counts + 2 * nxt, 0, 2 * sizeof(int), s));
+      A.f = bfp[b];
+      A.hit_flag = sl[b].hit_flag;
+      A.shadow_rays_out = sl[b].shadow;
+      A.sample_color = sl[b].sample_color;
+      A.first = (it == 0);
+      A.ps = sl[b].ps[cur[b]];
+      A.ps_out = sl[b].ps[nxt];
+      A.counts_in = counts + 2 * cur[b];
+      A.counts_out = counts + 2 * nxt;
+      A.tile_next = counts + 64;
+      record_trace_begin(c, s, 1);
+      if (c->sc.mat_tex) k_shade<true><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
+      else k_shade<false><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
+      record_trace_end(c, s);
+      c->stats.kernel_launches++;
+      CK(cudaGetLastError());
+      cur[b] = nxt;
+    }
+    for (int b = 0; b < nb; ++b) {
+      if (!live[b]) continue;
+      const cudaStream_t s = band_stream(c, b);
+      int* counts = band_counts(c, b);
+      if (it >= FSPT_NUM_BOUNCES) {
+        // every surviving path had i == NUM_BOUNCES: nothing was appended
+        if (!c->info.has_dielectric) { live[b] = false; continue; }
+        // Refractions do not count as bounces (`i--`, tracer.fs:488), so paths may survive.  The number of live paths
+        // is copied out after every extra iteration, but the host reads the value of TWO iterations ago: the GPU always
+        // has work queued and never waits for the host; at most two empty iterations (kernels that find zero items) are
+        // wasted.  Each band polls and stops on its own.
+        int* poll = c->h_poll.p + b * Ctx::POLL_SLOTS;
+        const int k = it % Ctx::POLL_SLOTS;
+        CK(cudaMemcpyAsync(poll + k, counts + 2 * cur[b], sizeof(int), cudaMemcpyDeviceToHost, s));
+        CK(cudaEventRecord(c->ev_poll[b][k], s));
+        if (it >= FSPT_NUM_BOUNCES + 2) {
+          const int k2 = (it - 2) % Ctx::POLL_SLOTS;
+          CK(cudaEventSynchronize(c->ev_poll[b][k2]));
+          if (poll[k2] == 0) { live[b] = false; continue; }
+        }
+      }
+      CK(cudaMemsetAsync(counts + 32, 0, sizeof(int), s));  // fetch cursor
+      rc = launch_trace(c, b, sl[b], cur[b], true, false);  // tracer.fs:501,507
+      if (rc) return rc;
+    }
+  }
+  for (int b = 0; b < nb; ++b) {
+    const FrameParams& f = bfp[b];
+    const int P = f.rw * f.rh;
+    k_accumulate<<<(P + 255) / 256, 256, 0, band_stream(c, b)>>>(sl[b].sample_color, c->d_fb.p, c->d_last_color.p, f.rx0,
+                                                                 f.ry0, f.rw, f.rh, f.width, S, first_tick,
+                                                                 c->accum_mode, c->sanitize);
     c->stats.kernel_launches++;
     CK(cudaGetLastError());
-    cur = nxt;
-    if (b >= FSPT_NUM_BOUNCES) {
-      if (!c->info.has_dielectric) break;  // every surviving path had i == NUM_BOUNCES: nothing was appended
-      // Refractions do not count as bounces (`i--`, tracer.fs:488), so paths may survive.  The number of live paths is
-      // copied out after every extra iteration, but the host reads the value of TWO iterations ago: the GPU always has
-      // work queued and never waits for the host; at most two empty iterations (kernels that find zero items) are wasted.
-      const int k = b % Ctx::POLL_SLOTS;
-      CK(cudaMemcpyAsync(c->h_poll.p + k, c->d_counts.p + 2 * cur, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-      CK(cudaEventRecord(c->ev_poll[k], c->stream));
-      if (b >= FSPT_NUM_BOUNCES + 2) {
-        const int k2 = (b - 2) % Ctx::POLL_SLOTS;
-        CK(cudaEventSynchronize(c->ev_poll[k2]));
-        if (c->h_poll.p[k2] == 0) break;
-      }
-    }
-    CK(cudaMemsetAsync(c->d_counts.p + 32, 0, sizeof(int), c->stream));  // fetch cursor
-    rc = launch_trace(c, cur, true, false);  // tracer.fs:501,507
-    if (rc) return rc;
   }
-  k_accumulate<<<(P + 255) / 256, 256, 0, c->stream>>>(c->d_sample_color.p, c->d_fb.p, c->d_last_color.p, fp.rx0, fp.ry0, fp.rw,
-                                                       fp.rh, fp.width, S, first_tick, c->accum_mode, c->sanitize);
-  c->stats.kernel_launches++;
-  CK(cudaGetLastError());
   return FSPT_OK;
 }
 
@@ -1017,6 +1104,9 @@ int fspt_create(fspt_ctx** out, int32_t width, int32_t height, int32_t device) {
     CK(cudaSetDevice(c->device));
     CK(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     CK(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
+    CK(cudaStreamCreateWithFlags(&c->stream2, cudaStreamNonBlocking));
+    CK(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
     CK(cudaEventCreateWithFlags(&c->ev_atlas, cudaEventDisableTiming));
     CK(cudaEventCreate(&c->ev_begin));
     CK(cudaEventCreate(&c->ev_end));
@@ -1069,11 +1159,13 @@ void fspt_destroy(fspt_ctx* ctx) {
   c->bcast_pending_root = -1;  // (no collective in a destructor)
   if (c->stream) cudaStreamSynchronize(c->stream);
   if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
+  if (c->stream2) cudaStreamSynchronize(c->stream2);
   delete c->pool;
   linear_tex(c, &c->nodes_tex, nullptr, 0);  // (destroys it)
   for (auto e : c->ev_ring) cudaEventDestroy(e);
   for (auto e : c->ev_rb) if (e) cudaEventDestroy(e);
-  for (auto e : c->ev_poll) if (e) cudaEventDestroy(e);
+  for (auto& band : c->ev_poll)
+    for (auto e : band) if (e) cudaEventDestroy(e);
   comm_free(c);
   if (c->ev_red0) cudaEventDestroy(c->ev_red0);
   if (c->ev_red1) cudaEventDestroy(c->ev_red1);
@@ -1083,6 +1175,9 @@ void fspt_destroy(fspt_ctx* ctx) {
   if (c->ev_begin) cudaEventDestroy(c->ev_begin);
   if (c->ev_end) cudaEventDestroy(c->ev_end);
   if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
+  if (c->stream2) cudaStreamDestroy(c->stream2);
+  if (c->ev_fork) cudaEventDestroy(c->ev_fork);
+  if (c->ev_join) cudaEventDestroy(c->ev_join);
   if (c->ev_atlas) cudaEventDestroy(c->ev_atlas);
   if (c->stream) cudaStreamDestroy(c->stream);
   delete c;  // frees the buffers and arrays
@@ -1402,15 +1497,31 @@ int fspt_render(fspt_ctx* ctx, const fspt_frame_params* frame, uint32_t first_ti
     if (rc0) return rc0;
   }
   CK(cudaEventRecord(c->ev_begin, c->stream));
+  // the second band's stream starts behind the rand-base copy and is joined back before ev_end, so everything after the
+  // render (timing, reduce, post-pass, read-back, collectives) stays ordered on c->stream alone
+  CK(cudaEventRecord(c->ev_fork, c->stream));
+  CK(cudaStreamWaitEvent(c->stream2, c->ev_fork, 0));
   // samples in flight per wave: the path-state arrays hold wave_paths records; a tile of the frame keeps more samples
   // in flight than the whole frame would (3840x2160 whole: 8, one of 8 tiles: 64)
   const int wave_S = (int)std::max<size_t>(1, std::min<size_t>((size_t)c->wave_cap, c->wave_paths / ((size_t)fp.rw * fp.rh)));
-  for (int done = 0; done < n_samples;) {
+  int rc = FSPT_OK;
+  for (int done = 0; done < n_samples && !rc;) {
     const int S = std::min(wave_S, n_samples - done);
-    int rc = render_wave(c, fp, first_tick + (uint32_t)done, S, c->d_rb.p + done, c->d_rb.p + c->rb_cap + done);
-    if (rc) return rc;
+    if (done > 0 && S != wave_S) {
+      // The last, shorter wave splits the rectangle differently (other slice offsets, perhaps one band only), so its
+      // bands may touch slices and pixel rows the other stream's band of the previous wave still works on: both streams
+      // wait for each other here.  Waves of equal S keep each band on its own stream, slice and rows.
+      CK(cudaEventRecord(c->ev_fork, c->stream));
+      CK(cudaEventRecord(c->ev_join, c->stream2));
+      CK(cudaStreamWaitEvent(c->stream2, c->ev_fork, 0));
+      CK(cudaStreamWaitEvent(c->stream, c->ev_join, 0));
+    }
+    rc = render_wave(c, fp, first_tick + (uint32_t)done, S, c->d_rb.p + done, c->d_rb.p + c->rb_cap + done);
     done += S;
   }
+  CK(cudaEventRecord(c->ev_join, c->stream2));  // (also after a failed wave: no work may be left outside c->stream)
+  CK(cudaStreamWaitEvent(c->stream, c->ev_join, 0));
+  if (rc) return rc;
   CK(cudaEventRecord(c->ev_end, c->stream));
   c->render_timed = true;
   c->next_tick = first_tick + (uint32_t)n_samples;
@@ -1505,10 +1616,10 @@ int fspt_debug_primary(fspt_ctx* ctx, const fspt_frame_params* frame, float rand
   }
   k_camera<<<(P + 255) / 256, 256, 0, c->stream>>>(fp, c->d_rb.p, P, make_fastdiv(1u, (unsigned long long)P), c->ps, c->d_cam_pos.p, c->d_cam_dir.p);
   c->stats.kernel_launches++;
-  int rc = set_counts(c, P, 0);
+  int rc = set_counts(c, 0, P, 0);
   if (rc) return rc;
   c->ev_trace_used = 0;
-  rc = launch_trace(c, 0, false, true);
+  rc = launch_trace(c, 0, band_slice(c, 0), 0, false, true);
   if (rc) return rc;
   CK(cudaStreamSynchronize(c->stream));
   // un-swizzle path slots -> pixels on the host
@@ -1546,10 +1657,10 @@ int fspt_debug_trace(fspt_ctx* ctx, const float* pos4, const float* dir4, int32_
     const int n = (int)std::min<int64_t>((int64_t)c->wave_paths, n_rays - done);
     CK(cudaMemcpy2DAsync(c->ps.rec + 0, 16 * FSPT_PATH_WORDS, pos4 + 4 * done, 16, 16, n, cudaMemcpyHostToDevice, c->stream));
     CK(cudaMemcpy2DAsync(c->ps.rec + 1, 16 * FSPT_PATH_WORDS, dir4 + 4 * done, 16, 16, n, cudaMemcpyHostToDevice, c->stream));
-    int rc = set_counts(c, n, 0);
+    int rc = set_counts(c, 0, n, 0);
     if (rc) return rc;
     c->ev_trace_used = 0;
-    rc = launch_trace(c, 0, false, true);
+    rc = launch_trace(c, 0, band_slice(c, 0), 0, false, true);
     if (rc) return rc;
     ro.resize(n); rdv.resize(n); cnt.resize(n);
     CK(cudaMemcpy2DAsync(ro.data(), 16, c->ps.rec + 0, 16 * FSPT_PATH_WORDS, 16, n, cudaMemcpyDeviceToHost, c->stream));

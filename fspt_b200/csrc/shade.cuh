@@ -231,6 +231,7 @@ struct ShadeArgs {
                               // direction | -.  (A list of record positions made the traversal kernel's shadow-ray
                               // fetch two dependent gathers over two sectors; this is one contiguous 32-byte read.)
   int* counts_out;            // [0] continuation, [1] shadow
+  int* tile_next;             // tile cursor, 0 between launches (k_shade resets it); on a 128-byte line of its own
   float4* sample_color;       // [pixel][sample-in-wave] final un-clamped path colour
   unsigned long long* capped; // paths stopped by the refraction cap
   int n_samples;              // samples in flight in this wave (slot = pixel * n_samples + sample)
@@ -529,7 +530,20 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS) k_shade(const
   const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
   int nh = 0, nm = 0;  // queue fill, block-uniform
   const int n_tiles = (n + SHADE_THREADS - 1) / SHADE_THREADS;
-  for (int tile = blockIdx.x;; tile += gridDim.x) {
+  // Tiles are handed out by a cursor, so a block that becomes resident late (behind another launch) takes less work
+  // instead of a fixed share.  Every block draws tickets until it gets one >= n_tiles, so a launch draws exactly
+  // n_tiles + gridDim.x of them; the block that draws the last one puts the cursor back to 0 for the next launch.
+  __shared__ int s_tile;
+  const unsigned last_ticket = (unsigned)n_tiles + gridDim.x - 1u;
+  auto fetch_tile = [&]() {
+    const int t = atomicAdd(A.tile_next, 1);
+    if ((unsigned)t == last_ticket) atomicExch(A.tile_next, 0);
+    s_tile = t;
+  };
+  if (threadIdx.x == 0) fetch_tile();
+  __syncthreads();
+  for (;;) {
+    const int tile = s_tile;
     const bool last = tile >= n_tiles;  // one extra round drains the partial groups
     if (!last) {
       const int it = tile * SHADE_THREADS + threadIdx.x;
@@ -539,6 +553,7 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS) k_shade(const
       const unsigned mh = __ballot_sync(0xffffffffu, hit), mm = __ballot_sync(0xffffffffu, live && !hit);
       if (lane == 0) { s_hits[warp] = __popc(mh); s_miss[warp] = __popc(mm); }
       __syncthreads();
+      if (threadIdx.x == 0) fetch_tile();  // every thread has read s_tile; the next barrier publishes the new one
       int hits_before = 0, miss_before = 0, t_hit = 0, t_miss = 0;
 #pragma unroll
       for (int w = 0; w < SHADE_THREADS / 32; ++w) {

@@ -95,6 +95,9 @@ typedef struct fspt_stats {
   double reduce_ms;       /* CUDA-event time of the last fspt_reduce_accum (NCCL reduce on the context's stream) */
   double primary_trace_ms; /* part of trace_ms spent in the camera + primary-ray launches (camera.fs + the first
                               intersectScene of tracer.fs main, :440) of the last fspt_render */
+  /* trace_ms, shade_ms and primary_trace_ms are sums of per-launch event times.  A large wave is rendered as two
+   * row bands on two streams whose launches overlap, so trace_ms + shade_ms can exceed render_ms; render_ms is the
+   * wall time of the render on the device. */
 } fspt_stats;
 
 int fspt_abi_version(void);

@@ -33,7 +33,9 @@ for r in range(a.reps + 1):
         import zlib
         crc = zlib.crc32(pt.accumulation().tobytes())
         n = W * H * a.spp
-        print("render %.2f ms  trace %.2f  shade %.2f  other %.2f | %.1f Mpaths/s %.1f Mrays/s | V/ray %.1f L/ray %.2f | crc %08x" % (
-            st["render_ms"], st["trace_ms"], st["shade_ms"], st["render_ms"] - st["trace_ms"] - st["shade_ms"],
+        # trace and shade are summed launch times; the two row bands of a wave overlap, so "overlap" = how much their
+        # sum exceeds the render (negative: time outside those launches -- accumulation, small launches, gaps)
+        print("render %.2f ms  trace %.2f  shade %.2f  overlap %.2f | %.1f Mpaths/s %.1f Mrays/s | V/ray %.1f L/ray %.2f | crc %08x" % (
+            st["render_ms"], st["trace_ms"], st["shade_ms"], st["trace_ms"] + st["shade_ms"] - st["render_ms"],
             n / st["render_ms"] / 1e3, st["last_rays"] / st["render_ms"] / 1e3,
             st["last_node_visits"] / st["last_rays"], st["last_leaf_visits"] / st["last_rays"], crc))
