@@ -22,7 +22,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 PATH = os.path.join(HERE, "reference_shaders", "outputs.npz")  # apart from the scene fixtures of test_golden.py
 N_SAMPLE = 64
 
-_store = None
+_stores = {}
 
 
 def canonical(a):
@@ -52,12 +52,12 @@ def record(out, key, a):
     out[key + ":val"] = a.reshape(-1)[idx]
 
 
-def check(key, got):
-    """Asserts that `got` has the bits the reference's shaders computed for `key`."""
-    global _store
-    if _store is None:
-        with np.load(PATH) as z:
-            _store = {k: z[k] for k in z.files}
+def check(key, got, path=PATH):
+    """Asserts that `got` has the bits the reference's shaders computed for `key` (stored in `path`)."""
+    if path not in _stores:
+        with np.load(path) as z:
+            _stores[path] = {k: z[k] for k in z.files}
+    _store = _stores[path]
     got = np.ascontiguousarray(got)
     shape = tuple(int(x) for x in _store[key + ":shape"])
     assert got.shape == shape, "%s: shape %s, the reference's is %s" % (key, got.shape, shape)
