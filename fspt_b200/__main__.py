@@ -11,7 +11,11 @@ def main():
     ap = argparse.ArgumentParser(prog="python -m fspt_b200")
     ap.add_argument("scene", help="path to a scene JSON, or one of the built-in procedural scenes: bunny, soup, pbr")
     ap.add_argument("--res", default="1280x720")
-    ap.add_argument("--spp", type=int, default=None, help="samples per pixel (default: scene.samples + 1, like the reference)")
+    ap.add_argument("--spp", type=int, default=None, help="samples per pixel (default: scene.samples + 1, like the reference); "
+                    "with --max-rel-error, the most any pixel gets")
+    ap.add_argument("--max-rel-error", type=float, default=None,
+                    help="adaptive sampling: stop a pixel once the relative standard error of its mean luminance is below this")
+    ap.add_argument("--min-spp", type=int, default=16, help="adaptive sampling: samples every pixel gets first (>= 2)")
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--seed", type=int, default=1)
     ap.add_argument("--denoise", action="store_true")
@@ -43,12 +47,16 @@ def main():
         return
     spp = a.spp if a.spp is not None else pt.maxSamples + 1
     t0 = time.time()
-    pt.tick(spp)
+    if a.max_rel_error is not None:
+        pt.converge(a.max_rel_error, max_samples=spp, min_samples=a.min_spp)
+    else:
+        pt.tick(spp)
     img = pt.image()
     dt = time.time() - t0
     st = pt.stats()
     Image.fromarray(np.ascontiguousarray(img)).save(a.output)
-    print("%d spp in %.2f s: %.1f Mpath-samples/s, %.1f Mrays/s -> %s" % (spp, dt, W * H * spp / dt / 1e6, st["rays"] / dt / 1e6, a.output))
+    print("%d spp in %.2f s: %.1f Mpath-samples/s, %.1f Mrays/s, %.1f samples per pixel on average -> %s"
+          % (spp, dt, st["samples"] / dt / 1e6, st["rays"] / dt / 1e6, st["samples"] / (W * H), a.output))
 
 
 if __name__ == "__main__":

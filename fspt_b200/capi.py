@@ -56,6 +56,7 @@ EXPORTS = [
     "fspt_env_bins", "fspt_pack_layer", "fspt_set_param", "fspt_set_tile", "fspt_comm_unique_id", "fspt_comm_init",
     "fspt_comm_destroy", "fspt_reduce_accum", "fspt_scene_broadcast", "fspt_scene_upload_async", "fspt_scene_upload_wait",
     "fspt_host_register", "fspt_host_unregister", "fspt_debug_pack_scene", "fspt_bvh_build_device", "fspt_device_check",
+    "fspt_set_adaptive", "fspt_active_pixels", "fspt_read_moment", "fspt_write_moment",
 ]
 PARAM_ANYHIT, PARAM_MAX_REFRACTIONS, PARAM_SANITIZE_NAN = 1, 2, 3
 
@@ -347,6 +348,29 @@ class Context:
         s = C.c_uint64(0)
         self._ck(self.lib.fspt_accum_device_ptr(self.h, C.byref(p), C.byref(n), C.byref(s)))
         return p.value, int(n.value), int(s.value)
+
+    def set_adaptive(self, max_rel_error, min_samples=16):
+        """fspt_set_adaptive: max_rel_error > 0 renders, before each wave, only the pixels whose relative standard error
+        of the mean luminance is still above it (or that have fewer than min_samples samples); 0 turns it off.  Sum mode
+        only (set_accum_mode(1))."""
+        self._ck(self.lib.fspt_set_adaptive(self.h, C.c_float(max_rel_error), C.c_int32(min_samples)))
+
+    def active_pixels(self):
+        """fspt_active_pixels: how many pixels of the rectangle the next wave would render (synchronises)."""
+        n = C.c_uint64(0)
+        self._ck(self.lib.fspt_active_pixels(self.h, C.byref(n)))
+        return int(n.value)
+
+    def read_moment(self):
+        """fspt_read_moment: per pixel, the f32 sum of the squared luminances of its samples (height, width)."""
+        out = np.empty((self.height, self.width), np.float32)
+        self._ck(self.lib.fspt_read_moment(self.h, ptr(out)))
+        return out
+
+    def write_moment(self, m2):
+        m2 = f32(m2)
+        assert m2.size == self.width * self.height
+        self._ck(self.lib.fspt_write_moment(self.h, ptr(m2)))
 
     def set_tile(self, x0, y0, w, h):
         """The pixel rectangle of the frame this context renders (GL row order); default = whole frame."""

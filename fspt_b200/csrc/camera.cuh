@@ -14,10 +14,12 @@ __device__ __forceinline__ float rnd(float& seed) {
 // camera.fs main, :37-46, for path slot p.  slot = pixel * S + sample: the S samples of one pixel sit in adjacent
 // slots (adjacent lanes), so their primary rays, hit records and texel footprints coincide and are served once per
 // warp instead of once per sample.
+// LIST (adaptive sampling): j indexes `list`, which holds the slots of the pixels this wave renders (adaptive.cuh).
+template <bool LIST = false>
 __device__ __forceinline__ void camera_ray(const FrameParams& f, const float* __restrict__ rb_cam, const FastDiv& div_s, int p,
-                                           v3& o, v3& d, int& x, int& y) {
+                                           v3& o, v3& d, int& x, int& y, const int* __restrict__ list = nullptr) {
   const int j = (int)fast_div((unsigned)p, div_s), s = p - j * (int)div_s.d;  // div_s: by the samples per wave
-  path_to_pixel(f, j, x, y);  // inside the context's rectangle; gl_FragCoord is the frame pixel
+  path_to_pixel(f, LIST ? list[j] : j, x, y);  // inside the context's rectangle; gl_FragCoord is the frame pixel
   const float resx = (float)f.width, resy = (float)f.height;
   const float fx = (float)(x + f.rx0) + 0.5f, fy = (float)(y + f.ry0) + 0.5f;  // gl_FragCoord
   const float uvx = (fx / resx) * 2.0f - 1.0f, uvy = (fy / resy) * 2.0f - 1.0f;  // `uv` varying (camera.vs)

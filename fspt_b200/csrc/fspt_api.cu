@@ -33,6 +33,7 @@
 #include <vector>
 
 #include "../../include/fspt_b200.h"
+#include "adaptive.cuh"
 #include "device_common.cuh"
 #include "host_pool.h"
 #include "scene_pack.h"
@@ -189,6 +190,12 @@ struct Ctx {
   int sanitize = 1;
   int max_refractions = 64;
   int anyhit = 1;
+  // adaptive sampling (fspt_set_adaptive), on while adapt_err > 0
+  float adapt_err = 0.0f;
+  int adapt_min = 2;
+  DevBuf<float> d_m2;         // per frame pixel: sum of the squared luminances of its samples (allocated when first on)
+  DevBuf<int> d_list;         // slots of the pixels a wave renders: band b's segment starts at its first pixel
+  uint64_t adaptive_samples = 0;  // d_stats[8] as last read: path samples of adaptive renders since fspt_clear
 
   // wavefront state
   int wave_samples = 0;       // samples in flight per wave (whole frame)
@@ -199,8 +206,9 @@ struct Ctx {
   DevBuf<float4> d_rec[2];    // what ps2[k] points to
   DevBuf<unsigned char> d_sh[2];
   DevBuf<float4> d_shadow;    // shadow rays of the current bounce, dense: origin | record position, direction | -
-  // per band b, from b * BAND_INTS: set k at [2k, 2k+1] = (#continuation, #shadow), [32] traversal fetch cursor, [64]
-  // shading tile cursor -- each cursor on a 128-byte line of its own: every warp's (block's) atomicAdd hits it
+  // per band b, from b * BAND_INTS: set k at [2k, 2k+1] = (#continuation, #shadow), [8] active pixels of the wave
+  // (adaptive sampling), [32] traversal fetch cursor, [64] shading tile cursor -- each cursor on a 128-byte line of its
+  // own: every warp's (block's) atomicAdd hits it
   static constexpr int BAND_INTS = 96;
   DevBuf<int> d_counts;
   DevBuf<int> d_count_out;    // per-slot visit count (debug)
@@ -230,6 +238,7 @@ struct Ctx {
   cudaEvent_t ev_bcast = nullptr;  // end of phase 1 on the context's stream
   int trace_blocks = 0, trace_blocks_cnt = 0, trace_blocks_cam = 0, shade_blocks = 0;
   int trace_blocks_nt = 0, trace_blocks_cnt_nt = 0, trace_blocks_cam_nt = 0;  // NODE_TEX = false instantiations
+  int trace_blocks_cam_list = 0, trace_blocks_cam_list_nt = 0;                // LIST (adaptive sampling) instantiations
 
   fspt_stats stats{};
 };
@@ -346,8 +355,9 @@ int alloc_wave(Ctx* c) {
   CK(cudaMemset(c->d_counts.p, 0, 2 * Ctx::BAND_INTS * sizeof(int)));
   CK(c->d_count_out.fit(W * sizeof(int)));
   CK(c->d_hit_flag.fit(W));
-  CK(c->d_stats.fit(8 * sizeof(unsigned long long)));  // [0..3] live, [4..7] snapshot at render start
-  CK(cudaMemset(c->d_stats.p, 0, 8 * sizeof(unsigned long long)));
+  // [0..3] live, [4..7] snapshot at render start, [8] path samples of adaptive renders since fspt_clear
+  CK(c->d_stats.fit(9 * sizeof(unsigned long long)));
+  CK(cudaMemset(c->d_stats.p, 0, 9 * sizeof(unsigned long long)));
   CK(c->d_sample_color.fit(W * 16));
   c->rb_cap = 64;
   CK(c->d_rb.fit(2 * (size_t)c->rb_cap * sizeof(float)));
@@ -405,8 +415,10 @@ __global__ void __launch_bounds__(256) k_interleave_atlas(cudaSurfaceObject_t su
 
 // counts = band_counts().  The shading tile cursor [64] is zeroed here at the start of every wave; between the shading
 // launches of a wave, k_shade puts it back to 0 itself (the block that draws a launch's last ticket), which holds as long
-// as every launch runs to completion with the grid it was launched with.
-__global__ void k_set_counts(int* counts, int n_cont, int n_shadow) {
+// as every launch runs to completion with the grid it was launched with.  per_active > 0 (adaptive sampling): n_cont is
+// per_active paths for each active pixel k_select_active counted into [8].
+__global__ void k_set_counts(int* counts, int n_cont, int n_shadow, int per_active) {
+  if (per_active) n_cont = per_active * counts[8];
   counts[0] = n_cont; counts[1] = n_shadow; counts[2] = 0; counts[3] = 0; counts[32] = 0; counts[64] = 0;
 }
 
@@ -714,7 +726,8 @@ BandSlice band_slice(const Ctx* c, size_t off) {
 // Traverses the continuation ray of every record of array `which` (counts[2*which] of them) + counts[2*which+1]
 // shadow rays of band `band` (slice `sl`); results go into the records, plus one hit/miss byte per position (for k_shade).
 int launch_trace(Ctx* c, int band, const BandSlice& sl, int which, bool hit_flags, bool write_count,
-                 const FrameParams* cam = nullptr, const float* rb_cam = nullptr, int n_samples = 1) {
+                 const FrameParams* cam = nullptr, const float* rb_cam = nullptr, int n_samples = 1,
+                 const int* list = nullptr) {
   TraceArgs A;
   if (cam) A.f = *cam; else memset(&A.f, 0, sizeof A.f);
   A.rb_cam = rb_cam; A.n_samples = n_samples;
@@ -728,9 +741,13 @@ int launch_trace(Ctx* c, int band, const BandSlice& sl, int which, bool hit_flag
   A.stats = c->d_stats.p;
   A.count_out = write_count ? c->d_count_out.p : nullptr;
   A.hit_flag = hit_flags ? sl.hit_flag : nullptr;
+  A.list = list;
   const cudaStream_t s = band_stream(c, band);
   record_trace_begin(c, s, cam ? 2 : 0);  // tag 2: the camera-fused primary launch of a wave
-  if (A.nodes_tex) {
+  if (list) {  // (adaptive sampling: camera-fused launches only)
+    if (A.nodes_tex) k_trace<false, true, true, true><<<c->trace_blocks_cam_list, TRACE_THREADS, 0, s>>>(A);
+    else k_trace<false, true, false, true><<<c->trace_blocks_cam_list_nt, TRACE_THREADS, 0, s>>>(A);
+  } else if (A.nodes_tex) {
     if (cam) k_trace<false, true, true><<<c->trace_blocks_cam, TRACE_THREADS, 0, s>>>(A);
     else if (write_count) k_trace<true, false, true><<<c->trace_blocks_cnt, TRACE_THREADS, 0, s>>>(A);
     else k_trace<false, false, true><<<c->trace_blocks, TRACE_THREADS, 0, s>>>(A);
@@ -746,8 +763,27 @@ int launch_trace(Ctx* c, int band, const BandSlice& sl, int which, bool hit_flag
 }
 
 int set_counts(Ctx* c, int band, int n_cont, int n_shadow) {  // also zeroes #hit, #miss and both cursors
-  k_set_counts<<<1, 1, 0, band_stream(c, band)>>>(band_counts(c, band), n_cont, n_shadow);
+  k_set_counts<<<1, 1, 0, band_stream(c, band)>>>(band_counts(c, band), n_cont, n_shadow, 0);
   CK(cudaGetLastError());
+  return FSPT_OK;
+}
+
+// Adaptive sampling: the slots of the active pixels of rectangle f -> list, their number -> band_counts(band)[8], on the
+// band's stream.  samples_per_pixel > 0: the wave's path count (S per active pixel) is set as set_counts does, and the
+// samples are counted into d_stats[8].
+int select_active(Ctx* c, int band, const FrameParams& f, int* list, int samples_per_pixel) {
+  const cudaStream_t s = band_stream(c, band);
+  int* counts = band_counts(c, band);
+  const int P = f.rw * f.rh;
+  CK(cudaMemsetAsync(counts + 8, 0, sizeof(int), s));
+  k_select_active<<<(P + 255) / 256, 256, 0, s>>>(f, c->d_fb.p, c->d_m2.p, c->adapt_err, c->adapt_min, list, counts + 8,
+                                                  samples_per_pixel ? c->d_stats.p + 8 : nullptr, samples_per_pixel);
+  c->stats.kernel_launches++;
+  CK(cudaGetLastError());
+  if (samples_per_pixel) {
+    k_set_counts<<<1, 1, 0, s>>>(counts, 0, 0, samples_per_pixel);
+    CK(cudaGetLastError());
+  }
   return FSPT_OK;
 }
 
@@ -823,19 +859,31 @@ int split_bands(const FrameParams& fp, int S, FrameParams band[2]) {
 // One wave.  Path records are dense arrays that ping-pong: set k = (array ps[k], counts band_counts()[2k .. 2k+1] =
 // #records, #shadow rays); the shadow list holds record positions.  The bands' launches are enqueued interleaved, so
 // that each stream always has its next launch queued behind the running one.
+// Adaptive sampling: each band first lists its active pixels (k_select_active); the wave renders S samples of each,
+// and its path count is known on the device only.  A wave with no active pixel still runs, with zero paths.
 int render_wave(Ctx* c, const FrameParams& fp, uint32_t first_tick, int S, const float* rb_cam, const float* rb_trace) {
   FrameParams bfp[2];
   const int nb = split_bands(fp, S, bfp);
   BandSlice sl[2];
+  int* list[2] = {nullptr, nullptr};
   int cur[2] = {0, 0};
   bool live[2] = {true, nb > 1};
-  for (int b = 0, off = 0; b < nb; ++b) {
+  const bool adaptive = c->adapt_err > 0.0f;
+  for (int b = 0, off = 0, px = 0; b < nb; ++b) {
     sl[b] = band_slice(c, (size_t)off);
     const int n_paths = S * bfp[b].rw * bfp[b].rh;
     off += n_paths;
-    int rc = set_counts(c, b, n_paths, 0);
+    int rc;
+    if (adaptive) {
+      list[b] = c->d_list.p + px;
+      px += bfp[b].rw * bfp[b].rh;
+      rc = select_active(c, b, bfp[b], list[b], S);
+    } else {
+      rc = set_counts(c, b, n_paths, 0);
+    }
     if (rc) return rc;
-    rc = launch_trace(c, b, sl[b], 0, true, false, &bfp[b], rb_cam, S);  // camera.fs + primary rays (tracer.fs:440), fused
+    // camera.fs + primary rays (tracer.fs:440), fused
+    rc = launch_trace(c, b, sl[b], 0, true, false, &bfp[b], rb_cam, S, list[b]);
     if (rc) return rc;
   }
   int rc;
@@ -873,9 +921,16 @@ int render_wave(Ctx* c, const FrameParams& fp, uint32_t first_tick, int S, const
       A.counts_in = counts + 2 * cur[b];
       A.counts_out = counts + 2 * nxt;
       A.tile_next = counts + 64;
+      A.list = list[b];
       record_trace_begin(c, s, 1);
-      if (c->sc.mat_tex) k_shade<true><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
-      else k_shade<false><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
+      if (adaptive) {
+        if (c->sc.mat_tex) k_shade<true, true><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
+        else k_shade<false, true><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
+      } else if (c->sc.mat_tex) {
+        k_shade<true><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
+      } else {
+        k_shade<false><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
+      }
       record_trace_end(c, s);
       c->stats.kernel_launches++;
       CK(cudaGetLastError());
@@ -910,9 +965,14 @@ int render_wave(Ctx* c, const FrameParams& fp, uint32_t first_tick, int S, const
   for (int b = 0; b < nb; ++b) {
     const FrameParams& f = bfp[b];
     const int P = f.rw * f.rh;
-    k_accumulate<<<(P + 255) / 256, 256, 0, band_stream(c, b)>>>(sl[b].sample_color, c->d_fb.p, c->d_last_color.p, f.rx0,
-                                                                 f.ry0, f.rw, f.rh, f.width, S, first_tick,
-                                                                 c->accum_mode, c->sanitize);
+    if (adaptive)
+      k_accumulate_active<<<(P + 255) / 256, 256, 0, band_stream(c, b)>>>(f, list[b], band_counts(c, b) + 8,
+                                                                          sl[b].sample_color, c->d_fb.p,
+                                                                          c->d_last_color.p, c->d_m2.p, S, c->sanitize);
+    else
+      k_accumulate<<<(P + 255) / 256, 256, 0, band_stream(c, b)>>>(sl[b].sample_color, c->d_fb.p, c->d_last_color.p,
+                                                                   f.rx0, f.ry0, f.rw, f.rh, f.width, S, first_tick,
+                                                                   c->accum_mode, c->sanitize);
     c->stats.kernel_launches++;
     CK(cudaGetLastError());
   }
@@ -1065,9 +1125,10 @@ int broadcast_phase2(Ctx* c) {
 }
 
 int pull_stats(Ctx* c) {
-  unsigned long long h[8];
+  unsigned long long h[9];
   CK(cudaMemcpy(h, c->d_stats.p, sizeof h, cudaMemcpyDeviceToHost));
   c->stats.rays = h[0]; c->stats.node_visits = h[1]; c->stats.leaf_visits = h[2]; c->stats.capped_paths = h[3];
+  c->adaptive_samples = h[8];
   c->stats.last_rays = h[0] - h[4]; c->stats.last_node_visits = h[1] - h[5]; c->stats.last_leaf_visits = h[2] - h[6];
   return FSPT_OK;
 }
@@ -1144,6 +1205,8 @@ int fspt_create(fspt_ctx** out, int32_t width, int32_t height, int32_t device) {
   c->trace_blocks_nt = persistent(k_trace<false, false, false>);
   c->trace_blocks_cnt_nt = persistent(k_trace<true, false, false>);
   c->trace_blocks_cam_nt = persistent(k_trace<false, true, false>);
+  c->trace_blocks_cam_list = persistent(k_trace<false, true, true, true>);
+  c->trace_blocks_cam_list_nt = persistent(k_trace<false, true, false, true>);
   int per_sm = 0;
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shade<true>, SHADE_THREADS, 1024);
   c->shade_blocks = std::max(1, per_sm) * c->sm_count;
@@ -1474,6 +1537,11 @@ int fspt_clear(fspt_ctx* ctx) {
   if (!c) return FSPT_E_INVALID;
   CK(cudaSetDevice(c->device));
   CK(cudaMemsetAsync(c->d_fb.p, 0, (size_t)c->n_pixels * 16, c->stream));
+  if (c->d_m2.p) {  // adaptive sampling has been on: its moment and sample count start again too
+    CK(cudaMemsetAsync(c->d_m2.p, 0, (size_t)c->n_pixels * sizeof(float), c->stream));
+    CK(cudaMemsetAsync(c->d_stats.p + 8, 0, sizeof(unsigned long long), c->stream));
+    c->adaptive_samples = 0;
+  }
   c->next_tick = 0;
   c->accum_samples = 0;
   c->stats.samples = 0;
@@ -1487,6 +1555,9 @@ int fspt_render(fspt_ctx* ctx, const fspt_frame_params* frame, uint32_t first_ti
   if (!frame || n_samples < 0 || (n_samples > 0 && (!rand_base_camera || !rand_base_tracer)))
     return fail(c, FSPT_E_INVALID, "fspt_render: bad arguments");
   if (!c->has_scene) return fail(c, FSPT_E_STATE, "fspt_render before fspt_scene_upload");
+  const bool adaptive = c->adapt_err > 0.0f;
+  if (adaptive && c->accum_mode != 1)
+    return fail(c, FSPT_E_STATE, "fspt_render: adaptive sampling needs the sum accumulation mode (fspt_set_accum_mode(ctx, 1))");
   CK(cudaSetDevice(c->device));
   const FrameParams fp = make_frame(c, frame);
   c->ev_trace_used = 0;
@@ -1526,7 +1597,7 @@ int fspt_render(fspt_ctx* ctx, const fspt_frame_params* frame, uint32_t first_ti
   c->render_timed = true;
   c->next_tick = first_tick + (uint32_t)n_samples;
   c->accum_samples += (uint64_t)n_samples;
-  c->stats.samples += (uint64_t)n_samples * (uint64_t)fp.rw * (uint64_t)fp.rh;
+  if (!adaptive) c->stats.samples += (uint64_t)n_samples * (uint64_t)fp.rw * (uint64_t)fp.rh;  // (adaptive: d_stats[8])
   return FSPT_OK;
 }
 
@@ -1599,6 +1670,62 @@ int fspt_set_accum_samples(fspt_ctx* ctx, uint64_t n) {
   Ctx* c = reinterpret_cast<Ctx*>(ctx);
   if (!c) return FSPT_E_INVALID;
   c->accum_samples = n;
+  return FSPT_OK;
+}
+
+int fspt_set_adaptive(fspt_ctx* ctx, float max_rel_error, int32_t min_samples) {
+  Ctx* c = reinterpret_cast<Ctx*>(ctx);
+  if (!c) return FSPT_E_INVALID;
+  if (!(max_rel_error >= 0.0f) || min_samples < 2)  // (NaN fails the comparison; a variance needs two samples)
+    return fail(c, FSPT_E_INVALID, "fspt_set_adaptive: max_rel_error %g must be >= 0 and min_samples %d >= 2",
+                (double)max_rel_error, min_samples);
+  if (max_rel_error > 0.0f && !c->d_list.p) {
+    CK(cudaSetDevice(c->device));
+    if (!c->d_m2.p) {
+      CK(c->d_m2.fit((size_t)c->n_pixels * sizeof(float)));
+      CK(cudaMemsetAsync(c->d_m2.p, 0, (size_t)c->n_pixels * sizeof(float), c->stream));
+    }
+    CK(c->d_list.fit((size_t)c->n_pixels * sizeof(int)));
+  }
+  c->adapt_err = max_rel_error;
+  c->adapt_min = min_samples;
+  return FSPT_OK;
+}
+
+int fspt_active_pixels(fspt_ctx* ctx, uint64_t* n_out) {
+  Ctx* c = reinterpret_cast<Ctx*>(ctx);
+  if (!c || !n_out) return FSPT_E_INVALID;
+  if (!(c->adapt_err > 0.0f)) return fail(c, FSPT_E_STATE, "fspt_active_pixels: adaptive sampling is off (fspt_set_adaptive)");
+  CK(cudaSetDevice(c->device));
+  FrameParams f;
+  memset(&f, 0, sizeof f);
+  f.width = c->width; f.height = c->height;
+  set_rect(f, c->rx0, c->ry0, c->rw, c->rh);
+  if (int rc = select_active(c, 0, f, nullptr, 0)) return rc;
+  int n = 0;
+  CK(cudaMemcpyAsync(&n, band_counts(c, 0) + 8, sizeof n, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  *n_out = (uint64_t)n;
+  return FSPT_OK;
+}
+
+int fspt_read_moment(fspt_ctx* ctx, float* out) {
+  Ctx* c = reinterpret_cast<Ctx*>(ctx);
+  if (!c || !out) return FSPT_E_INVALID;
+  if (!c->d_m2.p) return fail(c, FSPT_E_STATE, "fspt_read_moment: adaptive sampling has never been on (fspt_set_adaptive)");
+  CK(cudaSetDevice(c->device));
+  CK(cudaMemcpyAsync(out, c->d_m2.p, (size_t)c->n_pixels * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  return FSPT_OK;
+}
+
+int fspt_write_moment(fspt_ctx* ctx, const float* in) {
+  Ctx* c = reinterpret_cast<Ctx*>(ctx);
+  if (!c || !in) return FSPT_E_INVALID;
+  if (!c->d_m2.p) return fail(c, FSPT_E_STATE, "fspt_write_moment: adaptive sampling has never been on (fspt_set_adaptive)");
+  CK(cudaSetDevice(c->device));
+  CK(cudaMemcpyAsync(c->d_m2.p, in, (size_t)c->n_pixels * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
   return FSPT_OK;
 }
 
@@ -1904,6 +2031,7 @@ int fspt_get_stats(fspt_ctx* ctx, fspt_stats* out) {
   (void)cudaGetLastError();  // event queries must not leave a sticky status for the next launch check
   c->stats.trace_ms = tr;
   *out = c->stats;
+  out->samples += c->adaptive_samples;
   out->kernel_launches += c->atlas_launches.load();
   return FSPT_OK;
 }

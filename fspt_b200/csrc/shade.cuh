@@ -244,6 +244,8 @@ struct ShadeArgs {
                                   // together with the path record -- shade +2.4 %: wider reads and queues cost more than
                                   // the shorter dependent chain saves at 32 warps/SM.  Also measured and dropped: requesting
                                   // the NEXT tile's bytes before this tile's groups are shaded, +0.5 %.)
+  const int* list;            // LIST: the slots of the pixels this wave renders (adaptive.cuh); last, so that the other
+                              // instantiations keep their parameter offsets and instructions
 };
 
 // Warp-aggregated append: one atomicAdd per warp per list (ballot + popc prefix); call with all 32 lanes
@@ -270,16 +272,18 @@ __device__ __forceinline__ int append_pos(bool want, int* counter) {
   return base + __popc(m & ((1u << lane) - 1u));
 }
 
+template <bool LIST>
 __device__ __forceinline__ void write_sample(const ShadeArgs& A, int slot, v3 color) {
   const int j = (int)fast_div((unsigned)slot, A.div_s), s = slot - j * A.n_samples;
   int x, y;
-  path_to_pixel(A.f, j, x, y);
+  path_to_pixel(A.f, LIST ? A.list[j] : j, x, y);
   // [pixel][sample]: the samples of a pixel finish in adjacent lanes and land in adjacent 16-byte entries
   A.sample_color[((size_t)y * A.f.rw + x) * A.n_samples + s] = make_float4(color.x, color.y, color.z, 1.0f);
 }
 
 // The tail of the previous loop iteration for a path whose ray MISSED: tracer.fs:442-443 (primary) or
 // :502-504 + :508-512 (bounce).  Ends the path.
+template <bool LIST>
 __device__ __forceinline__ void shade_miss(const ShadeArgs& A, int pos) {
   const int slot_in = pos;  // record position in A.ps
   int slot = pos;           // path identity (pixel * S + sample); equals the position only in the first pass
@@ -300,7 +304,7 @@ __device__ __forceinline__ void shade_miss(const ShadeArgs& A, int pos) {
     const v3 reflectance = mk3(t4.x, t4.y, t4.z);                 // accumulatedReflectance *= bsdfThroughput (:508) was
     color = add(color, mul(mul(reflectance, env), t4.w));         // folded into the stored value; :510
   }
-  write_sample(A, slot, color);
+  write_sample<LIST>(A, slot, color);
 }
 
 // One loop iteration of tracer.fs main (:446-513) for a path whose ray HIT, split at the intersectScene calls.
@@ -312,7 +316,7 @@ __device__ __forceinline__ void store_record(const PathState& ps, int pos, const
   dst[0] = rec.w[0]; dst[1] = rec.w[1]; dst[2] = rec.w[3]; dst[3] = rec.w[4]; dst[4] = rec.w[5];
   ps.sh[pos] = shadow ? 1 : 0;  // (every record: a stale 2 of an earlier bounce must not survive at this position)
 }
-template <bool MAT_TEX>
+template <bool MAT_TEX, bool LIST>
 __device__ __forceinline__ bool shade_hit(const ShadeArgs& A, int pos, bool& shadow, PathRecord& out) {
   const DeviceScene& sc = A.sc;
   int slot = pos;  // path identity; equals the record position only in the first pass
@@ -340,7 +344,7 @@ __device__ __forceinline__ bool shade_hit(const ShadeArgs& A, int pos, bool& sha
     if (shadow_state == 2) color = add(color, mk3(p4.x, p4.y, p4.z));  // shadow.index == -1, :502-504
     ++i;                                                    // for (...; ++i), :446
     if (!(i < FSPT_NUM_BOUNCES)) {
-      write_sample(A, slot, color);
+      write_sample<LIST>(A, slot, color);
       return false;
     }
   }
@@ -519,7 +523,8 @@ __device__ __forceinline__ bool shade_hit(const ShadeArgs& A, int pos, bool& sha
 // queues and work starts only on full groups of one kind, so hit shading and miss shading never share a warp.
 // MAT_TEX: the atlas is the material-interleaved one (false = plain RGBA8 layers, the fallback of fspt_scene_upload);
 // a template parameter so that only one of the two sampling routines is in the kernel's instruction footprint.
-template <bool MAT_TEX>
+// LIST (adaptive sampling): path j * S + s belongs to the pixel of slot A.list[j].
+template <bool MAT_TEX, bool LIST = false>
 __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS) k_shade(const ShadeArgs A) {
   init_unorm8_lut();
   // block-local queues: every tile pushes its hits and misses, and work is only started on FULL groups of
@@ -570,7 +575,7 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS) k_shade(const
       const int take = nh < SHADE_THREADS ? nh : SHADE_THREADS;
       bool cont = false, shadow = false;
       PathRecord rec;
-      if ((int)threadIdx.x < take) cont = shade_hit<MAT_TEX>(A, q_hit[nh - take + threadIdx.x], shadow, rec);
+      if ((int)threadIdx.x < take) cont = shade_hit<MAT_TEX, LIST>(A, q_hit[nh - take + threadIdx.x], shadow, rec);
       // stream compaction of the surviving paths: the new record goes to the next free position of ps_out
       const int pos_out = append_pos(cont, A.counts_out + 0);
       if (cont) store_record(A.ps_out, pos_out, rec, shadow);
@@ -587,7 +592,7 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS) k_shade(const
     }
     while (nm >= SHADE_THREADS || (last && nm > 0)) {
       const int take = nm < SHADE_THREADS ? nm : SHADE_THREADS;
-      if ((int)threadIdx.x < take) shade_miss(A, q_miss[nm - take + threadIdx.x]);
+      if ((int)threadIdx.x < take) shade_miss<LIST>(A, q_miss[nm - take + threadIdx.x]);
       nm -= take;
       __syncthreads();
     }
@@ -599,13 +604,13 @@ __global__ void __launch_bounds__(SHADE_THREADS, SHADE_MIN_BLOCKS) k_shade(const
 // tracer.fs:515-517: clamp, then running mean over ticks (mode 0) or plain sum (mode 1), per pixel in tick
 // order so that the f32 result equals the reference's sequence of passes.
 // sample_color is indexed by the pixel inside the context's rectangle (rw x rh at rx0, ry0), fb by the frame pixel.
-__global__ void __launch_bounds__(256) k_accumulate(const float4* __restrict__ sample_color, float4* fb, float4* last_color,
-                                                    int rx0, int ry0, int rw, int rh, int width, int n_samples,
-                                                    unsigned first_tick, int mode, int sanitize) {
-  const int q = blockIdx.x * blockDim.x + threadIdx.x;
-  if (q >= rw * rh) return;
-  const size_t p = (size_t)(ry0 + q / rw) * width + (size_t)(rx0 + q % rw);
+// MOMENT (adaptive sampling, adaptive.cuh): the luminance l of every clamped sample adds l*l to *m2, in tick order.
+template <bool MOMENT>
+__device__ __forceinline__ void accumulate_pixel(const float4* __restrict__ sample_color, float4* fb, float4* last_color,
+                                                 int q, size_t p, int n_samples, unsigned first_tick, int mode,
+                                                 int sanitize, float* m2) {
   float4 acc = fb[p];
+  float m = MOMENT ? m2[p] : 0.0f;
   v3 c = mk3(0.0f, 0.0f, 0.0f);
   for (int s = 0; s < n_samples; ++s) {
     const float4 c4 = sample_color[(size_t)q * n_samples + s];
@@ -616,6 +621,10 @@ __global__ void __launch_bounds__(256) k_accumulate(const float4* __restrict__ s
       if (c.z != c.z) c.z = 0.0f;
     }
     c = clamp3(c, 0.0f, 1024.0f);  // :515
+    if (MOMENT) {
+      const float l = (c.x * 0.2126f + c.y * 0.7152f) + c.z * 0.0722f;
+      m += l * l;
+    }
     if (mode == 0) {
       const float ft = (float)(first_tick + (unsigned)s);
       const v3 t = mk3(acc.x, acc.y, acc.z);
@@ -626,7 +635,16 @@ __global__ void __launch_bounds__(256) k_accumulate(const float4* __restrict__ s
     }
   }
   fb[p] = acc;
+  if (MOMENT) m2[p] = m;
   if (last_color) last_color[p] = make_float4(c.x, c.y, c.z, 1.0f);
+}
+__global__ void __launch_bounds__(256) k_accumulate(const float4* __restrict__ sample_color, float4* fb, float4* last_color,
+                                                    int rx0, int ry0, int rw, int rh, int width, int n_samples,
+                                                    unsigned first_tick, int mode, int sanitize) {
+  const int q = blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= rw * rh) return;
+  const size_t p = (size_t)(ry0 + q / rw) * width + (size_t)(rx0 + q % rw);
+  accumulate_pixel<false>(sample_color, fb, last_color, q, p, n_samples, first_tick, mode, sanitize, nullptr);
 }
 
 // ---------------------------------------------------------------------------------------------------------

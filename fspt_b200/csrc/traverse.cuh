@@ -47,6 +47,8 @@ struct TraceArgs {
   int n_samples;
   FastDiv div_s;          // by n_samples
   int anyhit;             // 1: hit-or-miss rays (shadow rays, marked last-bounce rays) stop at their first intersection
+  const int* list;        // LIST: the slots of the pixels this wave renders (adaptive.cuh); last, so that the other
+                          // instantiations keep their parameter offsets and instructions
 };
 
 #ifndef TRACE_THREADS
@@ -126,7 +128,8 @@ __device__ __forceinline__ float tri_test(const float4 q0, const float4 q1, cons
 // ray + hit record is written at retirement, so the camera pass, its 32 B/path of writes and this launch's
 // record reads disappear.
 // NODE_TEX = false: the node array is too large for a linear texture (2^27 texels), everything goes through the LSU.
-template <bool WRITE_COUNT, bool CAMERA, bool NODE_TEX>
+// LIST (CAMERA only, adaptive sampling): path j * S + s renders the pixel of slot A.list[j].
+template <bool WRITE_COUNT, bool CAMERA, bool NODE_TEX, bool LIST = false>
 __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const TraceArgs A) {
   const unsigned lane = threadIdx.x & 31u;
   const unsigned FULL = 0xffffffffu;
@@ -240,7 +243,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
             kind = false;
             v3 o, d;
             int px, py;
-            camera_ray(A.f, A.rb_cam, A.div_s, my, o, d, px, py);
+            camera_ray<LIST>(A.f, A.rb_cam, A.div_s, my, o, d, px, py, A.list);
             start_ray(make_float4(o.x, o.y, o.z, 0.0f), make_float4(d.x, d.y, d.z, 0.0f), my);
           } else {
             // continuation rays: words 0 / 1 of record `my`; shadow rays: their own dense array written by k_shade

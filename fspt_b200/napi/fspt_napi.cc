@@ -11,6 +11,8 @@
 //   const rgba8 = fspt.resolve(ctx, {exposure, saturation, maxSigma, scale, denoise});
 // Multi-GPU (one process per GPU, see main_multi.mjs): fspt.commUniqueId() / commInit(ctx, id, rank, world) /
 //   sceneBroadcast(ctx, root) / setTile(ctx, x0, y0, w, h) / setAccumMode(ctx, 1) / reduceAccum(ctx, root).
+// Adaptive sampling (sum mode): setAdaptive(ctx, maxRelError, minSamples) / activePixels(ctx) / readMoment(ctx, w, h) /
+//   writeMoment(ctx, Float32Array, w, h).
 #include <node_api.h>
 
 #include <cstring>
@@ -348,13 +350,74 @@ napi_value SceneBroadcast(napi_env env, napi_callback_info info) {  // sceneBroa
   return nullptr;
 }
 
+// ---- adaptive sampling (fspt_set_adaptive): render until the pixels' means have converged ----------------------------
+napi_value SetAdaptive(napi_env env, napi_callback_info info) {  // setAdaptive(ctx, maxRelError, minSamples)
+  size_t argc = 3;
+  napi_value argv[3];
+  NAPI_OK(napi_get_cb_info(env, info, &argc, argv, nullptr, nullptr));
+  fspt_ctx* ctx = Unwrap(env, argv[0]);
+  double err = 0;
+  napi_get_value_double(env, argv[1], &err);
+  int r = fspt_set_adaptive(ctx, (float)err, argc > 2 ? Int32Arg(env, argv[2]) : 16);
+  if (r) return Throw(env, ctx, r);
+  return nullptr;
+}
+
+napi_value ActivePixels(napi_env env, napi_callback_info info) {  // activePixels(ctx) -> pixels the next wave renders
+  size_t argc = 1;
+  napi_value argv[1];
+  NAPI_OK(napi_get_cb_info(env, info, &argc, argv, nullptr, nullptr));
+  fspt_ctx* ctx = Unwrap(env, argv[0]);
+  uint64_t n = 0;
+  int r = fspt_active_pixels(ctx, &n);
+  if (r) return Throw(env, ctx, r);
+  napi_value out;
+  NAPI_OK(napi_create_int32(env, (int32_t)n, &out));  // (fspt_create bounds a frame by 2^27 pixels)
+  return out;
+}
+
+napi_value ReadMoment(napi_env env, napi_callback_info info) {  // readMoment(ctx, w, h) -> Float32Array(w * h)
+  size_t argc = 3;
+  napi_value argv[3];
+  NAPI_OK(napi_get_cb_info(env, info, &argc, argv, nullptr, nullptr));
+  fspt_ctx* ctx = Unwrap(env, argv[0]);
+  const size_t n = (size_t)Int32Arg(env, argv[1]) * (size_t)Int32Arg(env, argv[2]);
+  void* data = nullptr;
+  napi_value ab, out;
+  NAPI_OK(napi_create_arraybuffer(env, n * 4, &data, &ab));
+  int r = fspt_read_moment(ctx, static_cast<float*>(data));
+  if (r) return Throw(env, ctx, r);
+  NAPI_OK(napi_create_typedarray(env, napi_float32_array, n, ab, 0, &out));
+  return out;
+}
+
+napi_value WriteMoment(napi_env env, napi_callback_info info) {  // writeMoment(ctx, Float32Array(w * h), w, h)
+  size_t argc = 4;
+  napi_value argv[4];
+  NAPI_OK(napi_get_cb_info(env, info, &argc, argv, nullptr, nullptr));
+  fspt_ctx* ctx = Unwrap(env, argv[0]);
+  napi_typedarray_type t;
+  size_t n = 0, off;
+  void* data = nullptr;
+  napi_value ab;
+  NAPI_OK(napi_get_typedarray_info(env, argv[1], &t, &n, &data, &ab, &off));
+  if (t != napi_float32_array || n < (size_t)Int32Arg(env, argv[2]) * (size_t)Int32Arg(env, argv[3])) {
+    napi_throw_error(env, nullptr, "writeMoment: needs a Float32Array of w * h values");
+    return nullptr;
+  }
+  int r = fspt_write_moment(ctx, static_cast<const float*>(data));
+  if (r) return Throw(env, ctx, r);
+  return nullptr;
+}
+
 napi_value Init(napi_env env, napi_value exports) {
   const struct { const char* name; napi_callback fn; } fns[] = {
       {"create", Create}, {"sceneUpload", SceneUpload}, {"sceneUploadWait", SceneUploadWait},
       {"hostRegister", HostRegister}, {"hostUnregister", HostUnregister}, {"render", Render}, {"clear", Clear},
       {"resolve", Resolve}, {"readAccum", ReadAccum}, {"bvhBuild", BvhBuild},
       {"setTile", SetTile}, {"setAccumMode", SetAccumMode}, {"commUniqueId", CommUniqueId}, {"commInit", CommInit},
-      {"reduceAccum", ReduceAccum}, {"sceneBroadcast", SceneBroadcast}};
+      {"reduceAccum", ReduceAccum}, {"sceneBroadcast", SceneBroadcast}, {"setAdaptive", SetAdaptive},
+      {"activePixels", ActivePixels}, {"readMoment", ReadMoment}, {"writeMoment", WriteMoment}};
   for (auto& f : fns) {
     napi_value fn;
     napi_create_function(env, f.name, NAPI_AUTO_LENGTH, f.fn, nullptr, &fn);

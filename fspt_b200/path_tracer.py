@@ -77,6 +77,19 @@ class PathTracer:
             self.tick(samples - self.pingpong)
         return self.drawQuad()
 
+    def converge(self, max_rel_error, max_samples=None, min_samples=16, batch=16):
+        """Render until every pixel's mean has converged (adaptive sampling, fspt_set_adaptive) or the sample budget is
+        spent (default maxSamples + 1, as in render()), in calls of `batch` ticks; no reference counterpart.  Clears
+        first and leaves the context in sum mode with adaptive sampling on, so later tick() calls go on refining the
+        pixels that are still active.  Returns drawQuad()."""
+        budget = self.maxSamples + 1 if max_samples is None else int(max_samples)
+        self.clear()
+        self.ctx.set_accum_mode(1)
+        self.ctx.set_adaptive(max_rel_error, min_samples)
+        while self.pingpong < budget and self.ctx.active_pixels() > 0:
+            self.tick(min(batch, budget - self.pingpong))
+        return self.drawQuad()
+
     # -- shootAutoFocusRay (main.js:447-546): one ray along the camera axis -> lensFeatures[0] = 1 - 1/dist.
     # The reference walks its JS tree in float64 with maxT = 1e6; here the same query is one GPU ray (f32,
     # MAX_T = 1e5), which differs from the JS value by f32 rounding of the distance.

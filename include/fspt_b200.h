@@ -82,7 +82,8 @@ typedef struct fspt_post_params {
 } fspt_post_params;
 
 typedef struct fspt_stats {
-  uint64_t samples;       /* path samples rendered since fspt_clear (pixels * ticks)                 */
+  uint64_t samples;       /* path samples rendered since fspt_clear (pixels * ticks; with adaptive sampling,
+                             the samples of the active pixels, counted on the device)                 */
   uint64_t rays;          /* intersectScene-equivalent calls: primary + shadow + continuation        */
   uint64_t node_visits;   /* V: loop iterations of intersectScene (tracer.fs:373)                    */
   uint64_t leaf_visits;   /* L: processLeaf calls (tracer.fs:380)                                    */
@@ -154,6 +155,35 @@ int fspt_set_accum_mode(fspt_ctx* ctx, int32_t mode);
  * into it, for torch.distributed / NCCL reduction by the host.  The pointer stays valid until destroy. */
 int fspt_accum_device_ptr(fspt_ctx* ctx, void** dptr, uint64_t* n_floats, uint64_t* n_samples);
 int fspt_set_accum_samples(fspt_ctx* ctx, uint64_t n_samples);
+
+/* ---- adaptive sampling (sum mode only; no reference counterpart) -------------------------------------------------
+ * max_rel_error > 0 turns it on for later fspt_render calls, 0 turns it off (the default).  FSPT_E_INVALID for a NaN or
+ * negative max_rel_error or for min_samples < 2 (a variance needs two samples).  While it is on, fspt_render in
+ * accumulation mode 0 returns FSPT_E_STATE: the running mean keeps no per-pixel count.
+ * Before each wave of a render, every pixel of the context's rectangle is tested; an ACTIVE pixel gets all samples of
+ * the wave, the others none.  With n = the pixel's count (alpha), m2 = its moment (below), every step in f32, in order:
+ *   mean   = ((r*0.2126 + g*0.7152) + b*0.0722) / n                          (draw.fs lumaCoefs)
+ *   var    = (m2/n - mean*mean) * (n / (n - 1))
+ *   active = n < min_samples  ||  sqrt(max(var, 0) / n) > max_rel_error * max(mean, 1e-3)
+ * A pixel that is not rendered keeps its sum, count and moment, so under a fixed threshold it never becomes active
+ * again: the ticks a pixel received are always a prefix of the render's ticks, and it equals, bit for bit, the uniform
+ * sum-mode render after that many ticks.  The moment m2 is a frame-sized f32 buffer, allocated (zeroed) when adaptive
+ * sampling is first turned on and zeroed by fspt_clear; while adaptive sampling is on, every sample adds l*l, l =
+ * (c.r*0.2126 + c.g*0.7152) + c.b*0.0722 of its colour after the NaN sanitising and the clamp (tracer.fs:515), in tick
+ * order.  Renders with adaptive sampling off do not update it.
+ * Counters: fspt_stats.samples counts the path samples actually rendered (counted on the device);
+ * fspt_accum_device_ptr's n_samples stays the number of ticks; fspt_debug_last_color keeps the older value for the
+ * pixels a wave did not render.
+ * Multi-GPU: tile sharding composes (each rank decides for its own pixels; reduce and resolve are unchanged).
+ * Sample-set sharding does not: one pixel's samples are split across ranks, and no rank sees its whole history. */
+int fspt_set_adaptive(fspt_ctx* ctx, float max_rel_error, int32_t min_samples);
+/* The number of pixels of the rectangle the next wave would render (the rule above on the current state); synchronises
+ * the context's stream.  A host loop stops when it returns 0.  FSPT_E_STATE while adaptive sampling is off. */
+int fspt_active_pixels(fspt_ctx* ctx, uint64_t* n_out);
+/* The moment buffer, width*height f32 in GL order (next to fspt_read_accum / fspt_write_accum: a resumed adaptive render
+ * writes back both).  FSPT_E_STATE before adaptive sampling has been turned on for the first time. */
+int fspt_read_moment(fspt_ctx* ctx, float* out);
+int fspt_write_moment(fspt_ctx* ctx, const float* in);
 
 /* ---- multi-GPU: one context per GPU (one process per GPU, or several contexts in one process) ------------------
  * The reference renders one image on one GPU, one sample per requestAnimationFrame (main.js:838-857); every (pixel,
