@@ -24,6 +24,7 @@
 #include <array>
 #include <atomic>
 #include <map>
+#include <memory>
 #include <chrono>
 #include <condition_variable>
 #include <functional>
@@ -118,6 +119,36 @@ struct TexArray {
   }
 };
 
+cudaError_t create_handle(cudaStream_t* h, unsigned flags) { return cudaStreamCreateWithFlags(h, flags); }
+cudaError_t create_handle(cudaEvent_t* h, unsigned flags) { return cudaEventCreateWithFlags(h, flags); }
+void destroy_handle(cudaStream_t h) { cudaStreamDestroy(h); }
+void destroy_handle(cudaEvent_t h) { cudaEventDestroy(h); }
+void destroy_handle(cudaTextureObject_t h) { cudaDestroyTextureObject(h); }
+
+// A stream, an event (create) or a texture object (created by the caller into `h`), destroyed on destruction or reset.
+// Movable, so that a growing std::vector can hold it; converts to the raw handle.
+template <class H>
+struct Handle {
+  H h{};
+  Handle() = default;
+  Handle(Handle&& o) noexcept : h(o.h) { o.h = H{}; }
+  ~Handle() { reset(); }
+  cudaError_t create(unsigned flags) {
+    reset();
+    const cudaError_t e = create_handle(&h, flags);
+    if (e != cudaSuccess) h = H{};
+    return e;
+  }
+  void reset() {
+    if (h) destroy_handle(h);
+    h = H{};
+  }
+  operator H() const { return h; }
+};
+using Stream = Handle<cudaStream_t>;
+using Event = Handle<cudaEvent_t>;
+using TexObject = Handle<cudaTextureObject_t>;
+
 // A resident scene apart from its atlas: what fspt_scene_upload derived from the host buffers and what
 // fspt_scene_broadcast sends to the other ranks.  Both size the buffers by it (fit_scene) and make it the scene the
 // kernels read (publish_scene).
@@ -133,15 +164,38 @@ struct AtlasInfo {
   int32_t res, layers;
 };
 
+// The launch variants of k_trace: plain, with per-slot visit counts (debug), camera-fused (the primary launch of a wave)
+// and camera-fused over the listed pixels (adaptive sampling).
+enum TraceMode { TRACE_PLAIN, TRACE_COUNT, TRACE_CAMERA, TRACE_CAMERA_LIST, TRACE_MODES };
+struct TraceKernel {
+  void (*fn)(TraceArgs);
+  int blocks = 0;  // persistent grid (fspt_create)
+};
+
+// Members are destroyed in reverse order of declaration: the host workers first, a texture object before the buffer it
+// reads, the events and streams last.
 struct Ctx {
   int device = 0, sm_count = 0;
   int width = 0, height = 0, n_pixels = 0;
   int rx0 = 0, ry0 = 0, rw = 0, rh = 0;  // the pixel rectangle this context renders (fspt_set_tile); default = frame
-  cudaStream_t stream = nullptr;
-  cudaStream_t stream2 = nullptr;     // the second row band of a render (render_wave); forked from and joined to `stream`
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  cudaEvent_t ev_begin = nullptr, ev_end = nullptr;
-  std::vector<cudaEvent_t> ev_trace;  // pairs around traversal (tag 0) / shading (tag 1) launches of the last render
+  static constexpr int RB_SLOTS = 8;    // rand-base staging slots (h_rb)
+  static constexpr int POLL_SLOTS = 8;  // refraction poll slots per band (h_poll)
+
+  // streams and events
+  Stream stream;
+  Stream stream2;      // the second row band of a render (render_wave); forked from and joined to `stream`
+  Stream copy_stream;  // atlas DMA, overlaps the primary traversal
+  Event ev_fork, ev_join;
+  Event ev_begin, ev_end;
+  std::vector<Event> ev_trace;  // pairs around traversal (tag 0) / shading (tag 1) launches of the last render
+  Event ev_atlas;               // behind the atlas copies (copy_stream) the first shading launch waits for
+  Event ev_env;                 // behind the environment copies on the context's stream (recorded when env_in_place)
+  std::vector<Event> ev_ring;   // per ring slot (h_ring): the copies that read it have completed
+  Event ev_rb[RB_SLOTS];        // per rand-base slot: the copy that read it has completed
+  Event ev_poll[2][POLL_SLOTS]; // per band and poll slot (h_poll): the count has landed
+  Event ev_red0, ev_red1;       // around the last fspt_reduce_accum
+  Event ev_bcast;               // end of phase 1 of fspt_scene_broadcast on the context's stream
+
   std::vector<int> ev_tag;
   size_t ev_trace_used = 0;
   bool render_timed = false;
@@ -153,28 +207,23 @@ struct Ctx {
   AtlasInfo atlas_info{};
   DeviceScene sc{};  // the kernels' view, set by publish_scene / publish_atlas
   DevBuf<uint8_t> d_nodes, d_tris, d_shade, d_bins;
+  TexObject nodes_tex;                // the node array again as a linear texture (second L1 data pipe)
   DevBuf<uint2> d_layer_info;
   DevBuf<int4> d_mat_info;
   TexArray env, mat, atlas;           // mat: the material-interleaved atlas; atlas: the plain RGBA8 one (one of the two)
   DevBuf<uint8_t> d_raw;              // distinct varying atlas layers as uploaded (RGBA8), source of the GPU interleave
   DevBuf<uint8_t> d_mat_src;          // MatSrc per textured material
-  cudaTextureObject_t nodes_tex = 0;  // the node array again as a linear texture (second L1 data pipe)
   PinnedBuf<uint8_t> h_stage;         // pinned staging for the atlas (one slot per layer)
-  cudaStream_t copy_stream = nullptr;                       // atlas DMA, overlaps the primary traversal
-  cudaEvent_t ev_atlas = nullptr;
   // fspt_scene_upload_async: the atlas part of the upload (constant-layer scan, host interleave into pinned memory,
   // band-wise DMA) runs on this thread after the call has returned; joined before the first shading launch and by
   // everything that touches scene state
   std::thread atlas_thread;
   // page-locked sources are DMA'd in place: they stay borrowed until the copies have completed, not just been enqueued
   bool env_in_place = false, atlas_in_place = false;
-  cudaEvent_t ev_env = nullptr;  // behind the environment copies on the context's stream (recorded when env_in_place)
   std::atomic<uint64_t> atlas_launches{0};  // kernels launched by the atlas part (folded into stats.kernel_launches)
   int atlas_rc = 0;            // outcome of the atlas part (written by the atlas thread, read after joining it)
   std::string atlas_error;
-  HostPool* pool = nullptr;    // host workers of fspt_scene_upload (created at the first upload)
   PinnedBuf<uint8_t> h_ring;   // pinned ring the geometry records are staged through, chunk by chunk
-  std::vector<cudaEvent_t> ev_ring;  // per ring slot: the copies that read it have completed
   PinnedBuf<uint8_t> h_geo;    // pinned block of the small tables (bins, layer / material tables) + env
 
   // frame state
@@ -216,31 +265,33 @@ struct Ctx {
   DevBuf<unsigned long long> d_stats;  // rays, nodes, leaves, capped
   DevBuf<float> d_rb;         // rand bases of one render call: [0,cap) camera, [cap,2cap) tracer
   // pinned staging, a ring of RB_SLOTS blocks of 2*rb_cap floats: a slot is rewritten only after the copy that last
-  // read it has completed (its event), so fspt_render never waits for the GPU to drain
-  static constexpr int RB_SLOTS = 8;
+  // read it has completed (ev_rb), so fspt_render never waits for the GPU to drain
   PinnedBuf<float> h_rb;
-  cudaEvent_t ev_rb[RB_SLOTS] = {};
   int rb_slot = 0;
   int rb_cap = 0;
   // refraction bounces beyond NUM_BOUNCES (tracer.fs:488): path counts polled two iterations behind the enqueue
-  static constexpr int POLL_SLOTS = 8;
-  PinnedBuf<int> h_poll;                   // [band * POLL_SLOTS + slot]
-  cudaEvent_t ev_poll[2][POLL_SLOTS] = {};
+  PinnedBuf<int> h_poll;                   // [band * POLL_SLOTS + slot], each behind its event ev_poll[band][slot]
   // collectives (fspt_comm_init): NCCL communicator over NVLink / NVSwitch
   ncclComm_t comm = nullptr;
   int comm_rank = 0, comm_world = 1;
-  cudaEvent_t ev_red0 = nullptr, ev_red1 = nullptr;  // around the last fspt_reduce_accum
   bool reduce_timed = false;
   DevBuf<uint8_t> d_lin;      // linear staging of the atlas array for fspt_scene_broadcast (phase 2)
   DevBuf<uint8_t> d_hdr;      // broadcast headers
   DevBuf<uint8_t> d_lin_env;  // linear staging of the environment array (phase 1 of the broadcast)
   int bcast_pending_root = -1;  // >= 0: phase 2 of fspt_scene_broadcast (the atlas) has not been issued yet
-  cudaEvent_t ev_bcast = nullptr;  // end of phase 1 on the context's stream
-  int trace_blocks = 0, trace_blocks_cnt = 0, trace_blocks_cam = 0, shade_blocks = 0;
-  int trace_blocks_nt = 0, trace_blocks_cnt_nt = 0, trace_blocks_cam_nt = 0;  // NODE_TEX = false instantiations
-  int trace_blocks_cam_list = 0, trace_blocks_cam_list_nt = 0;                // LIST (adaptive sampling) instantiations
+  // the kernel variants: k_trace by [TraceMode][node texture; 0: the node array is beyond the linear-texture limit],
+  // each with its persistent grid, and k_shade by [mat_tex][list], all with the grid of k_shade<true>
+  TraceKernel trace_kernels[TRACE_MODES][2] = {
+      {{k_trace<false, false, false>}, {k_trace<false, false, true>}},
+      {{k_trace<true, false, false>}, {k_trace<true, false, true>}},
+      {{k_trace<false, true, false>}, {k_trace<false, true, true>}},
+      {{k_trace<false, true, false, true>}, {k_trace<false, true, true, true>}},
+  };
+  void (*shade_kernels[2][2])(ShadeArgs) = {{k_shade<false>, k_shade<false, true>}, {k_shade<true>, k_shade<true, true>}};
+  int shade_blocks = 0;
 
   fspt_stats stats{};
+  std::unique_ptr<HostPool> pool;  // host workers of fspt_scene_upload (created at the first upload)
 };
 
 void comm_free(Ctx* c);
@@ -270,9 +321,8 @@ int fail(Ctx* c, int code, const char* fmt, ...) {
 
 // A device array of 16-byte words as a linear texture (tex1Dfetch): the second L1 data path next to the LSU.  Arrays
 // beyond the 2^27-texel limit get no texture (0) and are read with plain loads.
-int linear_tex(Ctx* c, cudaTextureObject_t* tex, void* ptr, size_t bytes, bool allowed = true) {
-  if (*tex) cudaDestroyTextureObject(*tex);
-  *tex = 0;
+int linear_tex(Ctx* c, TexObject* tex, void* ptr, size_t bytes, bool allowed) {
+  tex->reset();
   if (!allowed || bytes / 16 > ((size_t)1 << 27) || bytes == 0) return FSPT_OK;
   cudaResourceDesc r = {};
   r.resType = cudaResourceTypeLinear;
@@ -281,7 +331,7 @@ int linear_tex(Ctx* c, cudaTextureObject_t* tex, void* ptr, size_t bytes, bool a
   r.res.linear.sizeInBytes = bytes;
   cudaTextureDesc t = {};
   t.readMode = cudaReadModeElementType;
-  CK(cudaCreateTextureObject(tex, &r, &t, nullptr));
+  CK(cudaCreateTextureObject(&tex->h, &r, &t, nullptr));
   return FSPT_OK;
 }
 
@@ -362,10 +412,10 @@ int alloc_wave(Ctx* c) {
   c->rb_cap = 64;
   CK(c->d_rb.fit(2 * (size_t)c->rb_cap * sizeof(float)));
   CK(c->h_rb.fit(Ctx::RB_SLOTS * 2 * (size_t)c->rb_cap * sizeof(float)));
-  for (auto& e : c->ev_rb) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  for (Event& e : c->ev_rb) CK(e.create(cudaEventDisableTiming));
   CK(c->h_poll.fit(2 * Ctx::POLL_SLOTS * sizeof(int)));
   for (auto& band : c->ev_poll)
-    for (auto& e : band) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    for (Event& e : band) CK(e.create(cudaEventDisableTiming));
   return FSPT_OK;
 }
 
@@ -375,13 +425,16 @@ int alloc_wave(Ctx* c) {
 cudaStream_t band_stream(const Ctx* c, int band) { return band ? c->stream2 : c->stream; }
 int* band_counts(const Ctx* c, int band) { return c->d_counts.p + Ctx::BAND_INTS * band; }
 
-void record_trace_begin(Ctx* c, cudaStream_t s, int tag = 0) {
-  if (c->ev_trace_used + 2 > c->ev_trace.size()) {
-    for (int i = 0; i < 2; ++i) { cudaEvent_t e; cudaEventCreate(&e); c->ev_trace.push_back(e); }
+int record_trace_begin(Ctx* c, cudaStream_t s, int tag) {
+  while (c->ev_trace_used + 2 > c->ev_trace.size()) {
+    Event e;
+    CK(e.create(cudaEventDefault));
+    c->ev_trace.push_back(std::move(e));
   }
   if (c->ev_tag.size() < c->ev_trace.size() / 2) c->ev_tag.resize(c->ev_trace.size() / 2);
   c->ev_tag[c->ev_trace_used / 2] = tag;
   cudaEventRecord(c->ev_trace[c->ev_trace_used], s);
+  return FSPT_OK;
 }
 void record_trace_end(Ctx* c, cudaStream_t s) {
   cudaEventRecord(c->ev_trace[c->ev_trace_used + 1], s);
@@ -743,19 +796,11 @@ int launch_trace(Ctx* c, int band, const BandSlice& sl, int which, bool hit_flag
   A.hit_flag = hit_flags ? sl.hit_flag : nullptr;
   A.list = list;
   const cudaStream_t s = band_stream(c, band);
-  record_trace_begin(c, s, cam ? 2 : 0);  // tag 2: the camera-fused primary launch of a wave
-  if (list) {  // (adaptive sampling: camera-fused launches only)
-    if (A.nodes_tex) k_trace<false, true, true, true><<<c->trace_blocks_cam_list, TRACE_THREADS, 0, s>>>(A);
-    else k_trace<false, true, false, true><<<c->trace_blocks_cam_list_nt, TRACE_THREADS, 0, s>>>(A);
-  } else if (A.nodes_tex) {
-    if (cam) k_trace<false, true, true><<<c->trace_blocks_cam, TRACE_THREADS, 0, s>>>(A);
-    else if (write_count) k_trace<true, false, true><<<c->trace_blocks_cnt, TRACE_THREADS, 0, s>>>(A);
-    else k_trace<false, false, true><<<c->trace_blocks, TRACE_THREADS, 0, s>>>(A);
-  } else {  // node array beyond the linear-texture limit
-    if (cam) k_trace<false, true, false><<<c->trace_blocks_cam_nt, TRACE_THREADS, 0, s>>>(A);
-    else if (write_count) k_trace<true, false, false><<<c->trace_blocks_cnt_nt, TRACE_THREADS, 0, s>>>(A);
-    else k_trace<false, false, false><<<c->trace_blocks_nt, TRACE_THREADS, 0, s>>>(A);
-  }
+  // (a pixel list comes with camera-fused launches only)
+  const int mode = list ? TRACE_CAMERA_LIST : cam ? TRACE_CAMERA : write_count ? TRACE_COUNT : TRACE_PLAIN;
+  const TraceKernel& k = c->trace_kernels[mode][A.nodes_tex != 0];
+  if (int rc = record_trace_begin(c, s, cam ? 2 : 0)) return rc;  // tag 2: the camera-fused primary launch of a wave
+  k.fn<<<k.blocks, TRACE_THREADS, 0, s>>>(A);
   record_trace_end(c, s);
   c->stats.kernel_launches++;
   CK(cudaGetLastError());
@@ -922,15 +967,8 @@ int render_wave(Ctx* c, const FrameParams& fp, uint32_t first_tick, int S, const
       A.counts_out = counts + 2 * nxt;
       A.tile_next = counts + 64;
       A.list = list[b];
-      record_trace_begin(c, s, 1);
-      if (adaptive) {
-        if (c->sc.mat_tex) k_shade<true, true><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
-        else k_shade<false, true><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
-      } else if (c->sc.mat_tex) {
-        k_shade<true><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
-      } else {
-        k_shade<false><<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
-      }
+      if ((rc = record_trace_begin(c, s, 1))) return rc;
+      c->shade_kernels[c->sc.mat_tex != 0][adaptive]<<<c->shade_blocks, SHADE_THREADS, 1024, s>>>(A);
       record_trace_end(c, s);
       c->stats.kernel_launches++;
       CK(cudaGetLastError());
@@ -1148,29 +1186,18 @@ int fspt_create(fspt_ctx** out, int32_t width, int32_t height, int32_t device) {
   Ctx* c = nullptr;
   if (!out || width <= 0 || height <= 0 || (int64_t)width * height > (1 << 27))
     return fail(c, FSPT_E_INVALID, "fspt_create: bad arguments (%d x %d)", width, height);
-  int n_dev = 0;
-  cudaError_t e = cudaGetDeviceCount(&n_dev);
-  if (e != cudaSuccess || n_dev <= 0)
-    return fail(c, FSPT_E_CUDA, "no CUDA device: %s (this library has no CPU fallback)", cudaGetErrorString(e));
-  if (device < 0 || device >= n_dev) return fail(c, FSPT_E_INVALID, "device %d out of range (%d present)", device, n_dev);
-  cudaDeviceProp prop;
-  if (cudaGetDeviceProperties(&prop, device) != cudaSuccess || prop.major != 10)
-    return fail(c, FSPT_E_CUDA, "device %d is sm_%d%d; kernels are built for sm_100a only", device, prop.major, prop.minor);
+  if (int rc = fspt_device_check(device)) return rc;
   c = new Ctx();
-  c->device = device; c->sm_count = prop.multiProcessorCount;
+  c->device = device;
   c->width = width; c->height = height; c->n_pixels = width * height;
   c->rx0 = c->ry0 = 0; c->rw = width; c->rh = height;
   auto init = [c]() -> int {
     const size_t px16 = (size_t)c->n_pixels * 16;
     CK(cudaSetDevice(c->device));
-    CK(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-    CK(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-    CK(cudaStreamCreateWithFlags(&c->stream2, cudaStreamNonBlocking));
-    CK(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
-    CK(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
-    CK(cudaEventCreateWithFlags(&c->ev_atlas, cudaEventDisableTiming));
-    CK(cudaEventCreate(&c->ev_begin));
-    CK(cudaEventCreate(&c->ev_end));
+    CK(cudaDeviceGetAttribute(&c->sm_count, cudaDevAttrMultiProcessorCount, c->device));
+    for (Stream* s : {&c->stream, &c->copy_stream, &c->stream2}) CK(s->create(cudaStreamNonBlocking));
+    for (Event* e : {&c->ev_fork, &c->ev_join, &c->ev_atlas, &c->ev_env, &c->ev_bcast}) CK(e->create(cudaEventDisableTiming));
+    for (Event* e : {&c->ev_begin, &c->ev_end, &c->ev_red0, &c->ev_red1}) CK(e->create(cudaEventDefault));
     CK(c->d_fb.fit(px16));
     CK(cudaMemset(c->d_fb.p, 0, px16));
     CK(c->d_last_color.fit(px16));
@@ -1199,14 +1226,8 @@ int fspt_create(fspt_ctx** out, int32_t width, int32_t height, int32_t device) {
     }
     return per_sm * c->sm_count;
   };
-  c->trace_blocks = persistent(k_trace<false, false, true>);
-  c->trace_blocks_cnt = persistent(k_trace<true, false, true>);
-  c->trace_blocks_cam = persistent(k_trace<false, true, true>);
-  c->trace_blocks_nt = persistent(k_trace<false, false, false>);
-  c->trace_blocks_cnt_nt = persistent(k_trace<true, false, false>);
-  c->trace_blocks_cam_nt = persistent(k_trace<false, true, false>);
-  c->trace_blocks_cam_list = persistent(k_trace<false, true, true, true>);
-  c->trace_blocks_cam_list_nt = persistent(k_trace<false, true, false, true>);
+  for (auto& row : c->trace_kernels)
+    for (TraceKernel& k : row) k.blocks = persistent(k.fn);
   int per_sm = 0;
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shade<true>, SHADE_THREADS, 1024);
   c->shade_blocks = std::max(1, per_sm) * c->sm_count;
@@ -1220,30 +1241,10 @@ void fspt_destroy(fspt_ctx* ctx) {
   cudaSetDevice(c->device);
   if (c->atlas_thread.joinable()) c->atlas_thread.join();
   c->bcast_pending_root = -1;  // (no collective in a destructor)
-  if (c->stream) cudaStreamSynchronize(c->stream);
-  if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
-  if (c->stream2) cudaStreamSynchronize(c->stream2);
-  delete c->pool;
-  linear_tex(c, &c->nodes_tex, nullptr, 0);  // (destroys it)
-  for (auto e : c->ev_ring) cudaEventDestroy(e);
-  for (auto e : c->ev_rb) if (e) cudaEventDestroy(e);
-  for (auto& band : c->ev_poll)
-    for (auto e : band) if (e) cudaEventDestroy(e);
+  for (const Stream* s : {&c->stream, &c->copy_stream, &c->stream2})
+    if (*s) cudaStreamSynchronize(*s);
   comm_free(c);
-  if (c->ev_red0) cudaEventDestroy(c->ev_red0);
-  if (c->ev_red1) cudaEventDestroy(c->ev_red1);
-  if (c->ev_bcast) cudaEventDestroy(c->ev_bcast);
-  if (c->ev_env) cudaEventDestroy(c->ev_env);
-  for (auto e : c->ev_trace) cudaEventDestroy(e);
-  if (c->ev_begin) cudaEventDestroy(c->ev_begin);
-  if (c->ev_end) cudaEventDestroy(c->ev_end);
-  if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-  if (c->stream2) cudaStreamDestroy(c->stream2);
-  if (c->ev_fork) cudaEventDestroy(c->ev_fork);
-  if (c->ev_join) cudaEventDestroy(c->ev_join);
-  if (c->ev_atlas) cudaEventDestroy(c->ev_atlas);
-  if (c->stream) cudaStreamDestroy(c->stream);
-  delete c;  // frees the buffers and arrays
+  delete c;  // frees the host workers, texture objects, buffers, arrays, events and streams (Ctx's member order)
 }
 
 // fspt_scene_upload / fspt_scene_upload_async.
@@ -1286,7 +1287,7 @@ static int scene_upload_impl(fspt_ctx* ctx, const fspt_scene_desc* s, bool async
   // (dist.share_host_threads sets FSPT_UPLOAD_THREADS = cores / processes on this node)
   int hw = (int)std::max(4u, std::min(32u, std::thread::hardware_concurrency()));
   if (const char* e = getenv("FSPT_UPLOAD_THREADS")) hw = std::max(4, std::min(64, atoi(e)));
-  if (!c->pool) { const int device = c->device; c->pool = new HostPool([device]() { cudaSetDevice(device); }); }
+  if (!c->pool) { const int device = c->device; c->pool = std::make_unique<HostPool>([device]() { cudaSetDevice(device); }); }
   HostPool& pool = *c->pool;
   // ---- pre-passes (scene_pack.h): interior-record numbering, material ids, depth / tree check
   ScenePrepass pre;
@@ -1349,9 +1350,9 @@ static int scene_upload_impl(fspt_ctx* ctx, const fspt_scene_desc* s, bool async
   const bool ring_wraps = n_geo_items > n_slots;  // otherwise every chunk has a slot of its own and no event is needed
   CK(c->h_ring.fit(slot_bytes * (size_t)n_slots));
   while ((int)c->ev_ring.size() < n_slots) {
-    cudaEvent_t e;
-    CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    c->ev_ring.push_back(e);
+    Event e;
+    CK(e.create(cudaEventDisableTiming));
+    c->ev_ring.push_back(std::move(e));
   }
   lap("buffers + pinned ring");
   struct GeoStatus { int code = FSPT_OK; char msg[192] = {0}; } geo;
@@ -1417,10 +1418,7 @@ static int scene_upload_impl(fspt_ctx* ctx, const fspt_scene_desc* s, bool async
   });
   if (dma_err.load()) return fail(c, FSPT_E_CUDA, "geometry upload failed: %s", cudaGetErrorString((cudaError_t)dma_err.load()));
   c->env_in_place = src_env_pinned;
-  if (src_env_pinned) {
-    if (!c->ev_env) CK(cudaEventCreateWithFlags(&c->ev_env, cudaEventDisableTiming));
-    CK(cudaEventRecord(c->ev_env, c->stream));
-  }
+  if (src_env_pinned) CK(cudaEventRecord(c->ev_env, c->stream));
   lap("geometry + env + layer scan");
   if ((rc_ = publish_scene(c, si))) return rc_;
   // ---- the atlas part: here, or on the context's atlas thread (the caller's atlas stays borrowed until it is joined).
@@ -1847,24 +1845,22 @@ int fspt_debug_read_bandwidth(fspt_ctx* ctx, uint64_t bytes, int32_t iters, doub
   Ctx* c = reinterpret_cast<Ctx*>(ctx);
   if (!c || !gb_per_s_out || bytes < 4096 || iters < 1) return FSPT_E_INVALID;
   CK(cudaSetDevice(c->device));
-  uint4* buf = nullptr;
-  unsigned* sink = nullptr;
+  DevBuf<uint4> buf;
+  DevBuf<unsigned> sink;
   const size_t n16 = (size_t)bytes / 16;
-  CK(cudaMalloc(&buf, n16 * 16));
-  CK(cudaMalloc(&sink, 4));
-  CK(cudaMemsetAsync(buf, 1, n16 * 16, c->stream));
-  cudaEvent_t e0, e1;
-  CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
+  CK(buf.fit(n16 * 16));
+  CK(sink.fit(4));
+  CK(cudaMemsetAsync(buf.p, 1, n16 * 16, c->stream));
+  Event e0, e1;
+  CK(e0.create(cudaEventDefault)); CK(e1.create(cudaEventDefault));
   const int blocks = c->sm_count * 8;
-  k_read_bw<<<blocks, 256, 0, c->stream>>>(buf, n16, 1, sink);  // warm-up: brings the buffer into L2 when it fits
+  k_read_bw<<<blocks, 256, 0, c->stream>>>(buf.p, n16, 1, sink.p);  // warm-up: brings the buffer into L2 when it fits
   CK(cudaEventRecord(e0, c->stream));
-  k_read_bw<<<blocks, 256, 0, c->stream>>>(buf, n16, iters, sink);
+  k_read_bw<<<blocks, 256, 0, c->stream>>>(buf.p, n16, iters, sink.p);
   CK(cudaEventRecord(e1, c->stream));
   CK(cudaStreamSynchronize(c->stream));
   float ms = 0.0f;
   CK(cudaEventElapsedTime(&ms, e0, e1));
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
-  cudaFree(buf); cudaFree(sink);
   *gb_per_s_out = (double)n16 * 16.0 * iters / (ms * 1e-3) / 1e9;
   return FSPT_OK;
 }
@@ -1926,7 +1922,6 @@ int fspt_reduce_accum(fspt_ctx* ctx, int32_t root) {
   CK(cudaSetDevice(c->device));
   if (int rc = broadcast_phase2(c)) return rc;  // (a rank that rendered nothing since the broadcast)
   NcclApi* N = nccl_api();
-  if (!c->ev_red0) { CK(cudaEventCreate(&c->ev_red0)); CK(cudaEventCreate(&c->ev_red1)); }
   CK(cudaEventRecord(c->ev_red0, c->stream));
   NK(N->Reduce(c->d_fb.p, c->d_fb.p, (size_t)c->n_pixels * 4, ncclFloat32, ncclSum, root, c->comm, c->stream));
   CK(cudaEventRecord(c->ev_red1, c->stream));
@@ -1950,7 +1945,6 @@ int fspt_scene_broadcast(fspt_ctx* ctx, int32_t root) {
   SceneHeader h;
   memset(&h, 0, sizeof h);
   static_assert(sizeof(SceneHeader) <= 256, "header buffer");
-  if (!c->ev_bcast) CK(cudaEventCreateWithFlags(&c->ev_bcast, cudaEventDisableTiming));
   if (is_root) {
     h.scene = c->info;
     h.magic = 0x46535054;
