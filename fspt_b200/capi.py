@@ -127,6 +127,12 @@ def f32(a):
     return np.ascontiguousarray(a, dtype=np.float32)
 
 
+# fspt_debug_math's probe codes (fspt_b200.h); oracle.dm_eval answers the same names
+DEBUG_MATH = {"sin": 0, "cos": 1, "atan2": 2, "asin": 3, "exp2": 4, "pow": 5, "sincos_s": 6, "sincos_c": 7, "log2": 8,
+              "rnd": 9, "min": 10, "max": 11, "clamp": 12, "div": 13, "div_shared": 14, "div_z": 15, "coord_to_i32": 16,
+              "quant8": 17}
+
+
 def bvh_build(verts, max_tris=4, n_threads=0, box_verts=None):
     """fspt_bvh_build(2): bvh.js + serializeTree + flatten.  Returns (nodes[N,9] f32 masked, order[T] i32, depth).
     box_verts: vertices the stale Triangle.boundingBox was computed from (scene.normalize), default = verts."""
@@ -424,11 +430,12 @@ class Context:
         return out.value
 
     def debug_math(self, fn, x, y=None):
-        names = {"sin": 0, "cos": 1, "atan2": 2, "asin": 3, "exp2": 4, "pow": 5, "sincos_s": 6, "sincos_c": 7}
+        """FSPT-DM2 probe `fn` on the device, elementwise over x (and y); the names are DEBUG_MATH's (fspt_b200.h)."""
         x = f32(x).ravel()
         y = f32(y).ravel() if y is not None else None
         out = np.empty_like(x)
-        self._ck(self.lib.fspt_debug_math(self.h, C.c_int32(names[fn]), ptr(x), ptr(y), ptr(out), C.c_int32(x.size)))
+        code = DEBUG_MATH[fn] if isinstance(fn, str) else int(fn)
+        self._ck(self.lib.fspt_debug_math(self.h, C.c_int32(code), ptr(x), ptr(y), ptr(out), C.c_int32(x.size)))
         return out
 
     def stats(self):

@@ -710,7 +710,8 @@ __global__ void __launch_bounds__(256) k_post(const float4* __restrict__ fb, uch
   out[(size_t)y * W + x] = make_uchar4(quant8(mapped.x), quant8(mapped.y), quant8(mapped.z), 255);
 }
 
-// FSPT-DM2 probes (fspt_debug_math)
+// FSPT-DM2 probes (fspt_debug_math): each code calls the kernels' own helper; the codes are listed in fspt_b200.h
+#define FSPT_DEBUG_MATH_CODES 18
 __global__ void k_debug_math(int fn, const float* x, const float* y, float* out, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -724,6 +725,16 @@ __global__ void k_debug_math(int fn, const float* x, const float* y, float* out,
     case 5: r = dm::powf_(x[i], y[i]); break;
     case 6: { float s, c; dm::sincosf_(x[i], s, c); r = s; break; }
     case 7: { float s, c; dm::sincosf_(x[i], s, c); r = c; break; }
+    case 8: r = dm::log2f_(x[i]); break;
+    case 9: r = sin_hash(x[i]); break;
+    case 10: r = fminf(x[i], y[i]); break;
+    case 11: r = fmaxf(x[i], y[i]); break;
+    case 12: r = clampf(x[i], 0.0f, 1024.0f); break;  // the per-sample colour clamp (tracer.fs:515)
+    case 13: r = x[i] / y[i]; break;
+    case 14: r = div_shared(mk3(x[i], 0.0f, 0.0f), y[i]).x; break;
+    case 15: r = div_z(x[i], y[i]); break;
+    case 16: r = __int_as_float(coord_to_i32(x[i])); break;  // the int's bits
+    case 17: r = (float)quant8(x[i]); break;
   }
   out[i] = r;
 }

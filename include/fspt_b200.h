@@ -227,8 +227,14 @@ int fspt_debug_trace(fspt_ctx* ctx, const float* pos4, const float* dir4, int32_
  * tracer.fs:515), RGBA32F; parity aid. */
 int fspt_debug_last_color(fspt_ctx* ctx, float* rgba32f_out);
 
-/* FSPT-DM2 arithmetic probes evaluated ON THE DEVICE (fn: 0 sin, 1 cos, 2 atan2(y,x), 3 asin, 4 exp2,
- * 5 pow(x,y)); parity aid for the platform built-ins the shaders rely on (tracer.fs:181,412,417). */
+/* FSPT-DM2 arithmetic probes evaluated ON THE DEVICE by the kernels' own helpers, out[i] = f(x[i], y[i]) (y == NULL
+ * reads as zeros); parity aid for the platform built-ins the shaders rely on (tracer.fs:181,412,417,515).  fn:
+ *   0 sin, 1 cos, 2 atan2(y, x), 3 asin, 4 exp2, 5 pow(x, y), 6 / 7 sin / cos of one sincos call, 8 log2,
+ *   9 rnd's hash fract(sin(x) * 43758.5453123), 10 min(x, y), 11 max(x, y), 12 clamp(x, 0, 1024), 13 x / y,
+ *   14 x / y through the camera's shared-reciprocal division, 15 x / y through the zero-dividend select,
+ *   16 the NaN/huge-guarded float->int32 conversion of texel coordinates (out holds the int's bits),
+ *   17 the RGBA8 colour-buffer quantisation (0..255 as a float).
+ * Any other fn: FSPT_E_INVALID. */
 int fspt_debug_math(fspt_ctx* ctx, int32_t fn, const float* x, const float* y, float* out, int32_t n);
 
 /* The host half of fspt_scene_upload without a GPU: pre-passes (interior-record numbering, material ids, depth / tree

@@ -131,11 +131,17 @@ def draw(fb, exposure=1.0, saturation=1.0, denoise=False, max_sigma=2.0, scale=1
     return out
 
 
+# the probe codes of fspt_debug_math (include/fspt_b200.h), answered with the model's plain operations
+DM_CODES = {"sin": 0, "cos": 1, "atan2": 2, "asin": 3, "exp2": 4, "pow": 5, "sincos_s": 6, "sincos_c": 7, "log2": 8,
+            "rnd": 9, "min": 10, "max": 11, "clamp": 12, "div": 13, "div_shared": 14, "div_z": 15, "coord_to_i32": 16,
+            "quant8": 17}
+
+
 def dm_eval(fn, x, y=None):
-    names = {"sin": 0, "cos": 1, "atan2": 2, "asin": 3, "exp2": 4, "pow": 5}
     x = _f32(x).ravel(); y = _f32(y).ravel() if y is not None else np.zeros_like(x)
     out = np.empty_like(x)
-    lib().oracle_dm_eval(C.c_int(names[fn]), _p(x), _p(y), _p(out), C.c_int(x.size))
+    if lib().oracle_dm_eval(C.c_int(DM_CODES[fn]), _p(x), _p(y), _p(out), C.c_int(x.size)) != 0:
+        raise ValueError("oracle_dm_eval: unknown probe %r" % (fn,))
     return out
 
 

@@ -469,19 +469,30 @@ extern "C" {
 
 int oracle_abi_version() { return 1; }
 
-/* ---- det-math probes (so tests can pin FSPT-DM2 against libm and the GPU) ---- */
-void oracle_dm_eval(int fn, const float* x, const float* y, float* out, int n) {
+/* ---- det-math probes (so tests can pin FSPT-DM2 against libm and the GPU) ----
+ * The codes are fspt_debug_math's (include/fspt_b200.h); each answers with the model's plain operation: the device's
+ * division shortcuts (13-15) all answer x / y, sincos (6, 7) answers sin / cos.  Returns -1 for an unknown code. */
+int oracle_dm_eval(int fn, const float* x, const float* y, float* out, int n) {
+  if (fn < 0 || fn > 17) return -1;
   for (int i = 0; i < n; ++i) {
     switch (fn) {
-      case 0: out[i] = dm_sin(x[i]); break;
-      case 1: out[i] = dm_cos(x[i]); break;
+      case 0: case 6: out[i] = dm_sin(x[i]); break;
+      case 1: case 7: out[i] = dm_cos(x[i]); break;
       case 2: out[i] = dm_atan2(y[i], x[i]); break;
       case 3: out[i] = dm_asin(x[i]); break;
       case 4: out[i] = dm_exp2(x[i]); break;
       case 5: out[i] = dm_pow(x[i], y[i]); break;
-      default: out[i] = 0.0f;
+      case 8: out[i] = dm_log2(x[i]); break;
+      case 9: out[i] = fractf(dm_sin(x[i]) * 43758.5453123f); break;
+      case 10: out[i] = fminN(x[i], y[i]); break;
+      case 11: out[i] = fmaxN(x[i], y[i]); break;
+      case 12: out[i] = clampf(x[i], 0.0f, 1024.0f); break;
+      case 13: case 14: case 15: out[i] = x[i] / y[i]; break;
+      case 16: { const int32_t v = (int32_t)tu_coord_to_int(x[i]); memcpy(&out[i], &v, 4); break; }
+      case 17: out[i] = (float)tu_quant8(x[i]); break;
     }
   }
+  return 0;
 }
 
 /* camera.fs main(), :37-46.  Outputs RGBA32F pos/dir, index = y*W + x, y up (gl_FragCoord). */

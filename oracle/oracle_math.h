@@ -13,8 +13,8 @@
  *     sequences below (+ - * / sqrt rint and single-rounded fmaf), i.e. what a GPU
  *     does natively (DM1, the first version, used binary64: 46 % of the shading
  *     kernel's instructions, and FP64 is vestigial on some Blackwell parts);
- *   - min/max are IEEE-754 minNum/maxNum (what GPU FMNMX does; GLSL leaves the
- *     NaN case undefined);
+ *   - min/max are IEEE-754-2019 minimumNumber/maximumNumber: a NaN operand
+ *     loses, -0 < +0 (what GPU FMNMX does; GLSL leaves both cases undefined);
  *   - vector built-ins follow the formulas printed in the GLSL ES 3.00 spec
  *     section 8 (normalize = x/length(x), reflect, refract, mix, clamp, fract).
  *
@@ -31,14 +31,19 @@
 namespace om {
 
 /* ---- scalar helpers --------------------------------------------------- */
-static inline float fminN(float a, float b) { /* IEEE minNum */
+/* min/max are IEEE 754-2019 minimumNumber/maximumNumber, what sm_100a's FMNMX computes (measured over every pair of
+ * tests/test_gpu_dm_exhaustive.py's edge set): a NaN operand loses to a number, and -0 orders below +0 whichever
+ * operand it is, so min(+0, -0) = -0, max(-0, +0) = +0 and clamp(-0, 0, hi) = +0. */
+static inline float fminN(float a, float b) {
   if (a != a) return b;
   if (b != b) return a;
+  if (a == b) return signbit(a) ? a : b; /* equal: the zero with the sign bit, if either has it */
   return b < a ? b : a;
 }
-static inline float fmaxN(float a, float b) { /* IEEE maxNum */
+static inline float fmaxN(float a, float b) {
   if (a != a) return b;
   if (b != b) return a;
+  if (a == b) return signbit(a) ? b : a;
   return a < b ? b : a;
 }
 static inline float clampf(float x, float lo, float hi) { return fminN(fmaxN(x, lo), hi); }
@@ -49,8 +54,11 @@ static inline float mixf(float x, float y, float a) { return x * (1.0f - a) + y 
  * All binary32.  fmaf() is a single-rounded fused multiply-add (x86 FMA3 / glibc fmaf; GPU FFMA.RN via
  * __fmaf_rn); every other operation is a separately rounded IEEE operation.  The operation sequences below ARE
  * the specification; the CUDA side (fspt_b200/csrc/dm_math.cuh) restates them with explicit intrinsics.
- * Accuracy against libm (tests/test_oracle_cpu.py): sin/cos <= 2 ulp for |x| <= 64 and an absolute error below
- * 4e-7 up to |x| = 1e7 (the sin-hash RNG range); atan2/asin/exp2 <= 3 ulp. */
+ * Accuracy against float64 libm, maxima over every f32 input of each range (tools/dm_accuracy.py, DESIGN.md section 2;
+ * checked at the worst arguments by tests/test_oracle_cpu.py): sin/cos <= 1.554 ulp for |x| <= 64, absolute error
+ * <= 1.085e-7 (sin) / 1.020e-7 (cos) up to |x| = 1e7 (the sin-hash RNG range); asin <= 3.671 ulp; exp2 <= 1.136 ulp on
+ * [-126, 127]; log2 <= 3.010 ulp for finite x > 0; pow(x, 0.454545) within 2.321e-5 of an 8-bit step on [0, 1];
+ * atan2 <= 2.901 ulp (sampled). */
 static inline float dm_fma(float a, float b, float c) { return __builtin_fmaf(a, b, c); }
 
 static const float DM_TWO_OVER_PI = 0x1.45f306p-1f;
