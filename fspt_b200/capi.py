@@ -131,6 +131,8 @@ def f32(a):
 DEBUG_MATH = {"sin": 0, "cos": 1, "atan2": 2, "asin": 3, "exp2": 4, "pow": 5, "sincos_s": 6, "sincos_c": 7, "log2": 8,
               "rnd": 9, "min": 10, "max": 11, "clamp": 12, "div": 13, "div_shared": 14, "div_z": 15, "coord_to_i32": 16,
               "quant8": 17}
+# fspt_debug_math's probes of the slab test's packed f32x2 lanes (fspt_b200.h); oracle.DM_PACKED_CODES answers them
+DEBUG_MATH_PACKED = {"sub2_lo": 32, "sub2_hi": 33, "mul2_lo": 34, "mul2_hi": 35}
 
 
 def bvh_build(verts, max_tris=4, n_threads=0, box_verts=None):
@@ -430,11 +432,12 @@ class Context:
         return out.value
 
     def debug_math(self, fn, x, y=None):
-        """FSPT-DM2 probe `fn` on the device, elementwise over x (and y); the names are DEBUG_MATH's (fspt_b200.h)."""
+        """FSPT-DM2 probe `fn` on the device, elementwise over x (and y); the names are DEBUG_MATH's and
+        DEBUG_MATH_PACKED's (fspt_b200.h)."""
         x = f32(x).ravel()
         y = f32(y).ravel() if y is not None else None
         out = np.empty_like(x)
-        code = DEBUG_MATH[fn] if isinstance(fn, str) else int(fn)
+        code = ({**DEBUG_MATH, **DEBUG_MATH_PACKED}[fn]) if isinstance(fn, str) else int(fn)
         self._ck(self.lib.fspt_debug_math(self.h, C.c_int32(code), ptr(x), ptr(y), ptr(out), C.c_int32(x.size)))
         return out
 

@@ -1813,7 +1813,8 @@ int fspt_debug_last_color(fspt_ctx* ctx, float* out) {
 
 int fspt_debug_math(fspt_ctx* ctx, int32_t fn, const float* x, const float* y, float* out, int32_t n) {
   Ctx* c = reinterpret_cast<Ctx*>(ctx);
-  if (!c || !x || !out || n < 0 || fn < 0 || fn >= FSPT_DEBUG_MATH_CODES) return FSPT_E_INVALID;
+  const bool known = (fn >= 0 && fn < FSPT_DEBUG_MATH_CODES) || (fn >= FSPT_DEBUG_MATH_PACKED && fn < FSPT_DEBUG_MATH_PACKED + 4);
+  if (!c || !x || !out || n < 0 || !known) return FSPT_E_INVALID;
   CK(cudaSetDevice(c->device));
   DevBuf<float> buf;  // one allocation (x | y | out), released on every path
   const size_t stride = (size_t)n + 1;

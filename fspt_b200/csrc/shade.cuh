@@ -11,6 +11,7 @@
 #include "dm_math.cuh"
 
 #include "camera.cuh"
+#include "traverse.cuh"  // the slab test's packed f32x2 operations, probed by k_debug_math
 
 // ---------------------------------------------------------------------------------------------------------
 // camera.fs main as a stand-alone pass (mode=test / fspt_debug_primary; the render loop fuses ray generation into
@@ -712,6 +713,7 @@ __global__ void __launch_bounds__(256) k_post(const float4* __restrict__ fb, uch
 
 // FSPT-DM2 probes (fspt_debug_math): each code calls the kernels' own helper; the codes are listed in fspt_b200.h
 #define FSPT_DEBUG_MATH_CODES 18
+#define FSPT_DEBUG_MATH_PACKED 32  // codes 32..35: the slab test's packed f32x2 lanes
 __global__ void k_debug_math(int fn, const float* x, const float* y, float* out, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -735,6 +737,13 @@ __global__ void k_debug_math(int fn, const float* x, const float* y, float* out,
     case 15: r = div_z(x[i], y[i]); break;
     case 16: r = __int_as_float(coord_to_i32(x[i])); break;  // the int's bits
     case 17: r = (float)quant8(x[i]); break;
+    case 32: case 33: case 34: case 35: {  // slab_pair's packed operations: two lanes against one broadcast scalar
+      const f32x2 a = pack2(x[i], -x[i]);
+      float lo, hi;
+      unpack2(fn < 34 ? sub2(a, bc2(y[i])) : mul2(a, bc2(y[i])), lo, hi);
+      r = (fn & 1) ? hi : lo;
+      break;
+    }
   }
   out[i] = r;
 }

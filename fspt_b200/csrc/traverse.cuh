@@ -175,9 +175,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
   } while (0)
   int cur = FSPT_SENTINEL;
   unsigned sp = SP0;
-  unsigned cnt = 0;  // visits of the current ray: low 16 bits all nodes, high 16 bits leaves (statistics; the bvh_test
-                     // count of the WRITE_COUNT variant is kept separately and exact)
-  int cnt_exact = 0;
+  int cnt_exact = 0;  // visits of the current ray (the bvh_test count of the WRITE_COUNT variant)
   bool kind = false, have = false;
   enum { R_DX = 0, R_DY = 1, R_DZ = 2, R_IX = 3, R_IY = 4, R_IZ = 5, R_SLOT = 6 };
 #define RAY_GET(row) ([&] { int v_; LANE_LD(v_, (row) * ROW); return v_; }())
@@ -187,7 +185,10 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
   float ox = 0, oy = 0, oz = 0;
   float tbest = FSPT_MAX_T;
   int ibest = -1;
-  unsigned n_nodes = 0, n_leaves = 0;  // per thread and launch: far below 2^32 (touched at retirement only)
+  // interior / leaf visits of all rays this thread traces in one launch, one increment per step (one ray alone can pass
+  // 2^16: a flat fan or a sliver soup gives 10^5).  The sums are exact while visits per ray times rays per thread per
+  // launch stays below 2^32.
+  unsigned n_interior = 0, n_leaves = 0;
   bool drained = false;
   bool boolean_ray = false;  // only hit-or-miss is consumed (tracer.fs:502, :509 at the last bounce)
 
@@ -200,7 +201,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
     const float ix = 1.0f / dx, iy = 1.0f / dy, iz = 1.0f / dz;  // `vec3 inverse = 1.0 / ray.dir`, tracer.fs:318
     RAY_SETF(R_IX, ix); RAY_SETF(R_IY, iy); RAY_SETF(R_IZ, iz);
     have = true;
-    tbest = FSPT_MAX_T; ibest = -1; cnt = 0; cnt_exact = 0;
+    tbest = FSPT_MAX_T; ibest = -1; cnt_exact = 0;
     sp = SP0;
     STACK_PUSH(FSPT_SENTINEL);
     cur = A.root_ref;
@@ -222,8 +223,6 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
       }
       if (WRITE_COUNT) A.count_out[slot] = cnt_exact;
       if (A.hit_flag && !kind) A.hit_flag[slot] = (ibest != -1);  // continuation rays: slot = queue position
-      n_nodes += cnt & 0xffffu;
-      n_leaves += cnt >> 16;
       have = false;
     }
     if (!drained) {
@@ -273,7 +272,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
         // ---- interior node: both child boxes from one 64-byte record --------------------------------
         if (is_int) {
           if (WRITE_COUNT) cnt_exact++;
-          cnt++;
+          n_interior++;
           // The record's four words are split between the two L1 data pipes (texture fetch / LSU load): the
           // kernel is bound by L1 wavefronts (ncu: l1tex data-pipe ~60 % busy), not by issue slots.  Measured with
           // 36 warps/SM: words 0,1 via TLD + words 2,3 via LDG is 0.5 % / 2.5 % faster than all four via TLD on the
@@ -301,7 +300,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
         // ---- leaf: 4 consecutive triangles ----------------------------------------------------------
         if (is_leaf) {
           if (WRITE_COUNT) cnt_exact++;
-          cnt += 0x10001u;
+          n_leaves++;
           const float dx = RAY_GETF(R_DX), dy = RAY_GETF(R_DY), dz = RAY_GETF(R_DZ);
           const int first = ~cur;
           const float4* tp = A.tris + 3 * (size_t)first;
@@ -319,7 +318,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(const
     }
   }
   // per-warp statistics -> 3 atomics per warp
-  unsigned long long s_nodes = n_nodes, s_leaves = n_leaves;
+  unsigned long long s_nodes = (unsigned long long)n_interior + n_leaves, s_leaves = n_leaves;
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     s_nodes += __shfl_xor_sync(FULL, s_nodes, o);

@@ -219,7 +219,10 @@ int fspt_scene_broadcast(fspt_ctx* ctx, int32_t root);
 int fspt_debug_primary(fspt_ctx* ctx, const fspt_frame_params* frame, float rand_base_camera,
                        int32_t* index_out, float* t_out, int32_t* count_out, float* pos4_out, float* dir4_out);
 
-/* intersectScene (tracer.fs:366-404) on caller-supplied rays (RGBA32F pos/dir like the camera targets). */
+/* intersectScene (tracer.fs:366-404) on caller-supplied rays (RGBA32F pos/dir like the camera targets).  A ray whose
+ * dir4.w holds the int32 bits -2 (the path record's last-bounce marker) is traced hit-or-miss when FSPT_PARAM_ANYHIT is
+ * 1: it stops after the first leaf in which it hits a triangle, and index / t / count are those of that leaf's closest
+ * hit and of the visits up to it.  Any other dir4.w, or ANYHIT 0: the full closest-hit traversal. */
 int fspt_debug_trace(fspt_ctx* ctx, const float* pos4, const float* dir4, int32_t n_rays,
                      int32_t* index_out, float* t_out, int32_t* count_out);
 
@@ -233,7 +236,10 @@ int fspt_debug_last_color(fspt_ctx* ctx, float* rgba32f_out);
  *   9 rnd's hash fract(sin(x) * 43758.5453123), 10 min(x, y), 11 max(x, y), 12 clamp(x, 0, 1024), 13 x / y,
  *   14 x / y through the camera's shared-reciprocal division, 15 x / y through the zero-dividend select,
  *   16 the NaN/huge-guarded float->int32 conversion of texel coordinates (out holds the int's bits),
- *   17 the RGBA8 colour-buffer quantisation (0..255 as a float).
+ *   17 the RGBA8 colour-buffer quantisation (0..255 as a float);
+ * and, for the slab test's packed f32x2 pipe:
+ *   32 / 33 the low / high lane of its packed subtraction sub.rn.f32x2 of (x, -x) and the broadcast y (x - y, -x - y),
+ *   34 / 35 the same two lanes of its packed multiplication mul.rn.f32x2 (x * y, -x * y).
  * Any other fn: FSPT_E_INVALID. */
 int fspt_debug_math(fspt_ctx* ctx, int32_t fn, const float* x, const float* y, float* out, int32_t n);
 

@@ -84,13 +84,15 @@ class Oracle:
         s.n_bins, s.leaf_size = self.bins.shape[0], leaf_size
         self.s = s
 
-    def bvh_test(self, pos4, dir4, nthreads=0):
+    def bvh_test(self, pos4, dir4, nthreads=0, anyhit=False):
+        """(index, t, count, stats) of intersectScene per ray; anyhit: stop after the first leaf that yields a hit, as the
+        product's hit-or-miss rays do (FSPT_PARAM_ANYHIT)"""
         pos4, dir4 = _f32(pos4).reshape(-1, 4), _f32(dir4).reshape(-1, 4)
         n = pos4.shape[0]
         idx = np.empty(n, np.int32); t = np.empty(n, np.float32); cnt = np.empty(n, np.int32)
         st = OStats()
         lib().oracle_bvh_test(C.byref(self.s), _p(pos4), _p(dir4), C.c_int(n), _p(idx), _p(t), _p(cnt), C.byref(st),
-                              C.c_int(nthreads))
+                              C.c_int(nthreads), C.c_int(1 if anyhit else 0))
         return idx, t, cnt, st.as_dict()
 
     def brute_force(self, pos4, dir4, nthreads=0):
@@ -135,12 +137,15 @@ def draw(fb, exposure=1.0, saturation=1.0, denoise=False, max_sigma=2.0, scale=1
 DM_CODES = {"sin": 0, "cos": 1, "atan2": 2, "asin": 3, "exp2": 4, "pow": 5, "sincos_s": 6, "sincos_c": 7, "log2": 8,
             "rnd": 9, "min": 10, "max": 11, "clamp": 12, "div": 13, "div_shared": 14, "div_z": 15, "coord_to_i32": 16,
             "quant8": 17}
+# the packed f32x2 lanes of the slab test, answered with the scalar IEEE operation
+DM_PACKED_CODES = {"sub2_lo": 32, "sub2_hi": 33, "mul2_lo": 34, "mul2_hi": 35}
 
 
 def dm_eval(fn, x, y=None):
     x = _f32(x).ravel(); y = _f32(y).ravel() if y is not None else np.zeros_like(x)
     out = np.empty_like(x)
-    if lib().oracle_dm_eval(C.c_int(DM_CODES[fn]), _p(x), _p(y), _p(out), C.c_int(x.size)) != 0:
+    code = DM_CODES[fn] if fn in DM_CODES else DM_PACKED_CODES[fn]
+    if lib().oracle_dm_eval(C.c_int(code), _p(x), _p(y), _p(out), C.c_int(x.size)) != 0:
         raise ValueError("oracle_dm_eval: unknown probe %r" % (fn,))
     return out
 

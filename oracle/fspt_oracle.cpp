@@ -116,8 +116,10 @@ inline float rayBoxIntersect(const OScene& s, int index, v3 ro, v3 rd) {
   return (tMax >= tMin && tMax > 0.0f) ? tMin : MAX_T;
 }
 
-/* intersectScene with the visit counter: bvh_test.fs:173-221 (== tracer.fs:366-404) */
-Hit intersectScene(const OScene& s, v3 ro, v3 rd, Counters& c, int* countOut) {
+/* intersectScene with the visit counter: bvh_test.fs:173-221 (== tracer.fs:366-404).
+ * anyhit: the product's hit-or-miss traversal (FSPT_PARAM_ANYHIT), which finishes the leaf of the first hit and stops
+ * there; the reference has no such exit. */
+Hit intersectScene(const OScene& s, v3 ro, v3 rd, Counters& c, int* countOut, bool anyhit = false) {
   int stack[256]; /* reference: int stack[64] (tracer.fs:368); overflow is flagged */
   int ptr = 0;
   stack[ptr++] = -1;
@@ -145,6 +147,7 @@ Hit intersectScene(const OScene& s, v3 ro, v3 rd, Counters& c, int* countOut) {
           result.t = res;
         }
       }
+      if (anyhit && result.index != -1) break;
     } else {
       if (leftHit < result.t && rightHit < result.t) {
         int deferred;
@@ -471,9 +474,10 @@ int oracle_abi_version() { return 1; }
 
 /* ---- det-math probes (so tests can pin FSPT-DM2 against libm and the GPU) ----
  * The codes are fspt_debug_math's (include/fspt_b200.h); each answers with the model's plain operation: the device's
- * division shortcuts (13-15) all answer x / y, sincos (6, 7) answers sin / cos.  Returns -1 for an unknown code. */
+ * division shortcuts (13-15) all answer x / y, sincos (6, 7) answers sin / cos, the packed slab-test lanes (32-35) the
+ * scalar subtraction / multiplication of their operands.  Returns -1 for an unknown code. */
 int oracle_dm_eval(int fn, const float* x, const float* y, float* out, int n) {
-  if (fn < 0 || fn > 17) return -1;
+  if (fn < 0 || (fn > 17 && (fn < 32 || fn > 35))) return -1;
   for (int i = 0; i < n; ++i) {
     switch (fn) {
       case 0: case 6: out[i] = dm_sin(x[i]); break;
@@ -490,6 +494,10 @@ int oracle_dm_eval(int fn, const float* x, const float* y, float* out, int n) {
       case 13: case 14: case 15: out[i] = x[i] / y[i]; break;
       case 16: { const int32_t v = (int32_t)tu_coord_to_int(x[i]); memcpy(&out[i], &v, 4); break; }
       case 17: out[i] = (float)tu_quant8(x[i]); break;
+      case 32: out[i] = x[i] - y[i]; break;
+      case 33: out[i] = -x[i] - y[i]; break;
+      case 34: out[i] = x[i] * y[i]; break;
+      case 35: out[i] = -x[i] * y[i]; break;
     }
   }
   return 0;
@@ -531,9 +539,10 @@ void oracle_camera(int W, int H, const float* P, const float* I, float fovScale,
   });
 }
 
-/* bvh_test.fs main(), :224-232, exporting (result.index, result.t, count) instead of the heat-map */
+/* bvh_test.fs main(), :224-232, exporting (result.index, result.t, count) instead of the heat-map; anyhit != 0 traces
+ * every ray hit-or-miss (see intersectScene) */
 void oracle_bvh_test(const OScene* s, const float* pos4, const float* dir4, int n, int32_t* index, float* t,
-                     int32_t* count, OStats* stats, int nthreads) {
+                     int32_t* count, OStats* stats, int nthreads, int anyhit) {
   int chunk = 4096;
   int rows = (n + chunk - 1) / chunk;
   std::vector<Counters> cs(256);
@@ -545,7 +554,7 @@ void oracle_bvh_test(const OScene* s, const float* pos4, const float* dir4, int 
       v3 o = mk3(pos4[4 * (size_t)i], pos4[4 * (size_t)i + 1], pos4[4 * (size_t)i + 2]);
       v3 d = mk3(dir4[4 * (size_t)i], dir4[4 * (size_t)i + 1], dir4[4 * (size_t)i + 2]);
       int cnt = 0;
-      Hit h = intersectScene(*s, o, d, cs[tid], &cnt);
+      Hit h = intersectScene(*s, o, d, cs[tid], &cnt, anyhit != 0);
       index[i] = h.index;
       t[i] = h.t;
       count[i] = cnt;

@@ -4,7 +4,10 @@ Every bit-exact render test rests on dm_math.cuh / device_common.cuh computing w
 compute for every input, not only for the arguments the scenes happen to produce.  Unary probes run on all 2^32 bit
 patterns; binary probes on V x V, V being oracle/dm_edges.py's structured set (every exponent, every branch edge of the
 model +-2 ulp, the shared-reciprocal division's window).  A NaN matches any NaN (the model does not fix payloads); the
-int-valued probe is compared bit for bit.  The file takes about 4 minutes on a B200 host."""
+int-valued probe is compared bit for bit.  The slab test's packed f32x2 subtraction and multiplication (FADD2 / FMUL2
+with a broadcast scalar operand) are compared on both lanes with numpy's float32 arithmetic, which is correctly rounded
+IEEE: a packed pipe that flushed subnormals or treated inf / NaN differently would change box order and visit counts.
+The file takes about 4 minutes on a B200 host."""
 import os
 import time
 from concurrent.futures import ThreadPoolExecutor
@@ -20,6 +23,9 @@ THREADS = max(1, min(32, os.cpu_count() or 1))
 UNARY = {"sin": ("sin",), "cos": ("cos",), "sincos": ("sincos_s", "sincos_c"), "asin": ("asin",), "exp2": ("exp2",),
          "log2": ("log2",), "rnd": ("rnd",), "clamp": ("clamp",), "coord_to_i32": ("coord_to_i32",), "quant8": ("quant8",)}
 BINARY = ("atan2", "pow", "min", "max", "div", "div_shared", "div_z")
+# slab_pair's packed lanes: (x, -x) against the broadcast y
+PACKED = {"sub2_lo": lambda x, y: x - y, "sub2_hi": lambda x, y: -x - y, "mul2_lo": lambda x, y: x * y,
+          "mul2_hi": lambda x, y: -x * y}
 INT_BITS = {"coord_to_i32"}  # the output holds an int's bits, some of which read as NaN: compare bits exactly
 
 
@@ -90,6 +96,30 @@ def test_binary_edges(ctx, oracle_mod, pool, fn):
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("fn", list(PACKED))
+def test_packed_slab_arithmetic_edges(ctx, oracle_mod, fn):
+    V = dm_edges.values()
+    x, y = np.repeat(V, V.size), np.tile(V, V.size)
+    with np.errstate(all="ignore"):
+        ref = PACKED[fn](x, y)
+    for who, got in (("device", ctx.debug_math(fn, x, y)), ("oracle", oracle_mod.dm_eval(fn, x, y))):
+        idx = _mismatch(got, ref, False)
+        assert idx.size == 0, who + " " + _report(fn, idx, got, ref, x, y)
+
+
+def test_packed_probe_operands_reach_every_class():
+    """V x V gives the packed lanes subnormal and overflowing results and every inf / NaN operand pairing"""
+    V = dm_edges.values()
+    x, y = np.repeat(V, V.size), np.tile(V, V.size)
+    tiny = np.finfo(np.float32).tiny
+    with np.errstate(all="ignore"):
+        for f in PACKED.values():
+            r = f(x, y)
+            fin = np.isfinite(x) & np.isfinite(y)
+            assert ((r != 0) & (np.abs(r) < tiny)).sum() > 1000 and np.isinf(r[fin]).sum() > 1000 and np.isnan(r).any()
+
+
+@pytest.mark.gpu
 def test_debug_math_rejects_unknown_code(ctx):
     from fspt_b200 import capi
     for code in (-1, len(capi.DEBUG_MATH), 1 << 20):
@@ -103,6 +133,27 @@ def test_probe_names_agree(oracle_mod):
     assert oracle_mod.DM_CODES == capi.DEBUG_MATH
     assert {name for names in UNARY.values() for name in names} | set(BINARY) == set(capi.DEBUG_MATH)  # each one tested
     assert oracle_mod.lib().oracle_dm_eval(len(capi.DEBUG_MATH), None, None, None, 0) == -1
+
+
+def test_packed_probe_names_agree(oracle_mod):
+    """Both sides answer the packed-lane probes with the same codes, apart from the scalar ones; each one is tested and
+    the oracle refuses the codes around their block."""
+    from fspt_b200 import capi
+    assert oracle_mod.DM_PACKED_CODES == capi.DEBUG_MATH_PACKED and set(PACKED) == set(capi.DEBUG_MATH_PACKED)
+    assert not set(capi.DEBUG_MATH_PACKED.values()) & set(capi.DEBUG_MATH.values())
+    lo, hi = min(capi.DEBUG_MATH_PACKED.values()), max(capi.DEBUG_MATH_PACKED.values())
+    assert hi - lo + 1 == len(capi.DEBUG_MATH_PACKED)
+    for code in (len(capi.DEBUG_MATH), lo - 1, hi + 1):
+        assert oracle_mod.lib().oracle_dm_eval(code, None, None, None, 0) == -1
+
+
+@pytest.mark.gpu
+def test_debug_math_rejects_codes_around_the_packed_block(ctx):
+    from fspt_b200 import capi
+    lo, hi = min(capi.DEBUG_MATH_PACKED.values()), max(capi.DEBUG_MATH_PACKED.values())
+    for code in (len(capi.DEBUG_MATH), lo - 1, hi + 1):
+        with pytest.raises(capi.FsptError):
+            ctx.debug_math(code, [1.0])
 
 
 def test_edge_set_holds_every_edge():
